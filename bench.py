@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's config, on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--dump-outputs DIR]
 
 Workload at N=1 (configs[1]): batch stylisation, 64 synthetic 512x512 images per step, c=64 / 3-block
 EnhancedGenerator, 3 styles (3 state dicts, seeds 0..2) blended in output space with weights
@@ -15,8 +15,16 @@ embeds `train` (configs[3]: EnhancedCycleGAN.train_step, batch 8 per GPU, NCCL a
 (configs[2]), `highres` (configs[4]), `cpu_baseline` and `parity` (GPU fp32 / bf16 vs the oracle at 512x512, c=64).
 
 --impl reference: the reference's own CPU implementation of the path (its PyTorch modules restated in
-oracle/restate.py -- /root/reference is not on the GPU box) on the host cores, on a bounded sample
+oracle/restate.py -- the reference is not part of this repository) on the host cores, on a bounded sample
 (1 image x 3 styles per step).
+
+--dump-outputs DIR: after the timed steps, writes what the timed call returned in its last step as DIR/<name>.npy
+(float32 images, float64 losses), so that two builds run with the same arguments -- hence the same seeded inputs and
+weights -- can be compared output for output.  An output larger than DUMP_MAX_ELEMS is cut to a fixed, seeded sample of its
+elements (dump_sample).  With N > 1 every rank writes its own shard as <name>_rank<r>.npy, sampled to DUMP_MAX_ELEMS / N.
+
+--steps K sets the timed steps of every measurement of the run: the headline, the end-to-end pass, its per-launch
+breakdown, and the embedded train, gram, highres and cpu_baseline measurements.
 """
 import argparse
 import json
@@ -42,6 +50,30 @@ IN_BYTES_512_BF16 = 520e6    # InstanceNorm algorithmic bytes per image (1 read 
 def synth_images(B, H, W, seed=1234):
     g = torch.Generator().manual_seed(seed)
     return torch.rand(B, 3, H, W, generator=g) * 2 - 1
+
+
+DUMP_MAX_ELEMS = 1 << 23           # 32 MB of float32 over all ranks: the dumps of one run stay under 64 MB
+
+
+def dump_sample(t, max_elems=DUMP_MAX_ELEMS):
+    """t as a host float32 array or, beyond max_elems, a fixed sample of it: the elements at max_elems flat indices drawn
+    without replacement by a generator seeded with 0, in increasing order (the same indices for the same shape)."""
+    t = t.detach().float()
+    if t.numel() > max_elems:
+        idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:max_elems].sort().values
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.cpu().numpy()
+
+
+def write_outputs(out_dir, arrays, rank=0, world=1):
+    """arrays: {name: numpy float32 / float64 array} -> out_dir/<name>.npy (<name>_rank<r>.npy when world > 1).  Every rank
+    writes at most this rank's share of 64 MB, so the dump of the whole run stays under 64 MB."""
+    import numpy as np
+    assert sum(a.nbytes for a in arrays.values()) * world <= 64e6, "output dump over 64 MB over all ranks"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + (f"_rank{rank}" if world > 1 else "") + ".npy"), a)
 
 
 def peaks():
@@ -136,14 +168,16 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    v, per_step, cores, _ = cpu_reference_images_per_sec(args.steps, args.warmup)
+    v, per_step, cores, y = cpu_reference_images_per_sec(args.steps, args.warmup)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"stylised": dump_sample(y)})
     line = {"metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": per_step * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "impl": "reference",
             "config": {"workload": "batch stylisation 512x512, c=64/3-block generator, 3 styles blended [0.2,0.3,0.5]",
                        "sample": "1 image x 3 styles per step (of the 64-image batch)",
-                       "note": "the reference is 100 % Python (stock torch.nn modules); /root/reference does not travel to the GPU "
-                               "box, so this arm runs its restatement oracle/restate.py (kind 'port'), which is pinned to the "
+                       "note": "the reference is 100 % Python (stock torch.nn modules) and not part of this repository, "
+                               "so this arm runs its restatement oracle/restate.py (kind 'port'), which is pinned to the "
                                "unmodified reference by tests/golden/ (bit-identical init, <= 1e-4 outputs)"},
             "cpu_baseline": {"value": v, "unit": UNIT, "cores": cores, "kind": "port",
                              "sample": "1 image x 3 generator forwards + blend per step, fp32, torch CPU (oracle/restate.py)"},
@@ -236,8 +270,9 @@ class Ctx:
         return self.max_over_ranks(ms) / steps, _lib.launches - l0, breakdown
 
 
-def bench_stylise(cx, args, gens, B_rank, seed_off=0, want_breakdown=True, want_e2e=True):
-    """One stylisation measurement with B_rank images on this rank.  Returns a dict of per-step times (max over ranks)."""
+def bench_stylise(cx, args, gens, B_rank, seed_off=0, want_breakdown=True, want_e2e=True, want_output=False):
+    """One stylisation measurement with B_rank images on this rank.  Returns a dict of per-step times (max over ranks) and,
+    with want_output, the (sampled) images of the last timed step under "output"."""
     from multi_style_transfer_gan_b200.stylize import MultiStyleStylizer
     H = W = args.size
     sty = MultiStyleStylizer(gens, precision=args.precision, micro_batch=args.micro_batch)
@@ -249,6 +284,8 @@ def bench_stylise(cx, args, gens, B_rank, seed_off=0, want_breakdown=True, want_
     # 126 MB L2, so nothing is L2-resident between timed iterations (no explicit flush needed).
     r = {"sty": sty, "x_host": x_host, "out_host": out_host}
     r["ms_dev"], r["launches"], _ = cx.timed(lambda: sty(x_dev, STYLE_W, out=out_dev), args.steps, args.warmup)
+    if want_output:                        # before the passes below overwrite out_dev
+        r["output"] = dump_sample(out_dev, DUMP_MAX_ELEMS // cx.world)
     if want_breakdown:
         # per-launch CUDA-event breakdown (roofline): the same step with one stream and no graph replay, because launches
         # inside a replayed graph cannot be bracketed by events and concurrent kernels of different styles share the SMs
@@ -258,7 +295,7 @@ def bench_stylise(cx, args, gens, B_rank, seed_off=0, want_breakdown=True, want_
     if want_e2e:
         # the public API with HOST buffers: pinned fp32 in -> uint8 out, both copies inside the timed region (the call
         # returns when the last D2H copy has landed)
-        r["ms_e2e"], _, _ = cx.timed(lambda: sty(x_host, STYLE_W, out_uint8=True, out=out_host), max(2, args.steps), 1)
+        r["ms_e2e"], _, _ = cx.timed(lambda: sty(x_host, STYLE_W, out_uint8=True, out=out_host), args.steps, 1)
     return r
 
 
@@ -414,7 +451,7 @@ def bench_train(cx, args, steps, warmup):
     return out
 
 
-def bench_gram(cx):
+def bench_gram(cx, args):
     """BASELINE.json configs[2]: Gram-matrix style loss forward + backward on the five VGG-19 tap shapes, batch 16 at 256x256
     (kernel-only, bf16 features = relu(randn)), and the same with the VGG-19 trunk forward + backward to the image."""
     from multi_style_transfer_gan_b200 import ops
@@ -431,7 +468,7 @@ def bench_gram(cx):
             _, g = ops.gram_loss_fwd(f, t, 1.0, loss)
             ops.gram_loss_bwd(f, g, t, 1.0)
 
-    ms, _, _ = cx.timed(gram_fb, 10, 3)
+    ms, _, _ = cx.timed(gram_fb, args.steps, 3)
     fl = 2 * sum(2.0 * c * c * s * s * 16 for c, s in shapes)            # fwd + bwd, 2*C^2*HW each
     by = sum(f.numel() * 2 * 3 for f in feats)                           # features read twice (fwd, bwd) + dF written
     pk = peaks()
@@ -443,7 +480,7 @@ def bench_gram(cx):
         y.grad = None
         sl(y).backward()
 
-    ms_full, _, _ = cx.timed(full, 5, 3)
+    ms_full, _, _ = cx.timed(full, args.steps, 3)
     return {"config": "Gram + style-loss forward + backward, VGG-19 relu1_1..relu5_1 shapes, batch 16 at 256x256, bf16",
             "ms": ms, "tflops_algorithmic": fl / ms / 1e9, "feature_gbs": by / ms / 1e6,
             "hbm_frac": by / ms / 1e6 / pk["hbm_gbs"], "parity": "unpinned (not in the reference; trunk pinned to torchvision, "
@@ -465,15 +502,15 @@ def bench_highres(cx, args):
     st = MultiStyleStylizer(gens, precision=args.precision, micro_batch=4)
     x = synth_images(8, 1024, 1024, seed=5).to(cx.dev)
     torch.cuda.reset_peak_memory_stats()
-    ms, _, _ = cx.timed(lambda: st(x, w4), 3, 2)
+    ms, _, _ = cx.timed(lambda: st(x, w4), args.steps, 2)
     peak_gib = torch.cuda.max_memory_allocated() / 2 ** 30
     ser = MultiStyleStylizer(gens, precision=args.precision, micro_batch=4, style_streams=False, use_graph=False)
-    _, _, bd = cx.timed(lambda: ser(x, w4), 1, 1, prof=True)
+    _, _, bd = cx.timed(lambda: ser(x, w4), args.steps, 1, prof=True)
     pk = peaks()
     out = {"config": "1024x1024, batch 8, 4 styles blended [0.4,0.3,0.2,0.1], c=64/3-block, bf16, micro-batch 4",
            "ms_per_batch": ms, "images_per_sec": 8e3 / ms, "peak_memory_gib": peak_gib}
-    in_ms = bd.get("msg_instnorm_apply", {}).get("ms", 0.0)
-    n = bd.get("msg_instnorm_apply", {}).get("launches", 0)
+    in_ms = bd.get("msg_instnorm_apply", {}).get("ms", 0.0) / args.steps
+    n = bd.get("msg_instnorm_apply", {}).get("launches", 0) // args.steps
     if in_ms > 0:
         per_fwd = n // (4 * 2)
         H = W = 1024
@@ -522,7 +559,9 @@ def run_ours(args):
     sampler = ClockSampler(cx.local)
     if rank == 0:
         sampler.start()
-    main = bench_stylise(cx, args, gens, hi - lo, seed_off=rank)
+    main = bench_stylise(cx, args, gens, hi - lo, seed_off=rank, want_output=bool(args.dump_outputs))
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"stylised": main.pop("output")}, rank, world)
     weak = None
     if world > 1:                         # the weak-scaling point of round 1 (64 images per GPU), kept as an extra key
         w = bench_stylise(cx, args, gens, B, seed_off=rank, want_breakdown=False, want_e2e=False)
@@ -557,14 +596,14 @@ def run_ours(args):
     if not args.no_extras:
         # BASELINE.json configs[3] (train step, every N: the only data-path collective of the repo), configs[2] and configs[4] (N = 1)
         try:
-            t = bench_train(cx, args, steps=max(3, args.steps), warmup=3)
+            t = bench_train(cx, args, steps=args.steps, warmup=3)
             if rank == 0:
                 line["train"] = t
         except Exception as e:           # the headline must survive a failure of a secondary workload -- but loudly
             if rank == 0:
                 line["train"] = {"error": repr(e)}
         if world == 1:
-            for key, fn in (("gram", lambda: bench_gram(cx)), ("highres", lambda: bench_highres(cx, args))):
+            for key, fn in (("gram", lambda: bench_gram(cx, args)), ("highres", lambda: bench_highres(cx, args))):
                 try:
                     line[key] = fn()
                 except Exception as e:
@@ -572,10 +611,10 @@ def run_ours(args):
     if rank == 0:
         if world == 1 and not args.no_cpu_baseline:
             x0 = synth_images(B, H, W, seed=1234)[0:1].contiguous()
-            v, per_step, cores, y_ref = cpu_reference_images_per_sec(5, 2, H, W, c, nb, x=x0, median=True)
+            v, per_step, cores, y_ref = cpu_reference_images_per_sec(args.steps, 2, H, W, c, nb, x=x0, median=True)
             line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": cores, "kind": "port",
                                     "sample": "1 image x 3 generator forwards + blend, fp32, torch CPU restatement of the "
-                                              "reference modules (oracle/restate.py), 2 warm-ups + median of 5"}
+                                              f"reference modules (oracle/restate.py), 2 warm-ups + median of {args.steps}"}
             try:
                 line["parity"] = bench_parity(cx, args, gens, x0, y_ref)
             except Exception as e:
@@ -589,6 +628,10 @@ def run_train(args):
     """Secondary workload on its own (BASELINE.json configs[3]); the default run embeds the same measurement as `train`."""
     cx = Ctx()
     t = bench_train(cx, args, steps=args.steps, warmup=args.warmup)
+    if args.dump_outputs:                  # the five losses train_step returned in the last timed step
+        import numpy as np
+        write_outputs(args.dump_outputs, {f"train_{k}": np.array(v, dtype=np.float64) for k, v in t["losses"].items()},
+                      cx.rank, cx.world)
     if cx.rank == 0:
         line = {"n_gpus": cx.world, "higher_is_better": True, "vs_baseline": None, "data": "synthetic"}
         line.update(t)
@@ -600,7 +643,7 @@ def run_train(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every measurement of the run (see the module docstring)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--size", type=int, default=512)
@@ -616,7 +659,11 @@ def main():
     ap.add_argument("--train-size", type=int, default=256)
     ap.add_argument("--lambda-style", type=float, default=0.0,
                     help="train workload: weight of the VGG-19 Gram style term (0 = the reference's train_step)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed call returned in its last step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.pt from the UNMODIFIED reference.
 
-Run in the build container (where /root/reference exists):  python oracle/make_golden.py
+Run with a checkout of the reference at oracle/_ref/ (or $MSG_REFERENCE_ROOT):  python oracle/make_golden.py
 The reference has no tests, fixtures or checkpoints of its own (SURVEY.md section 4), so the golden
 vectors are outputs of the reference classes themselves: seeded random init
 (torch.manual_seed(seed) before the constructor), seeded synthetic input

@@ -1,4 +1,5 @@
-"""TEST INFRASTRUCTURE ONLY -- imports the *real* reference (read-only, /root/reference).
+"""TEST INFRASTRUCTURE ONLY -- imports the *real* reference (read-only) from a checkout of it at
+``oracle/_ref/`` (kept out of git) or at ``$MSG_REFERENCE_ROOT``.
 
 The reference cannot be imported as shipped: ``enhanced_generator.py:4`` imports
 ``StructuralTransformerBlock`` from a module ``structural_transformer`` that is not in the
@@ -7,17 +8,17 @@ repository (SURVEY.md F2).  This shim registers an identity stub under that name
 (ctor ``StructuralTransformerBlock(dim=...)``, call ``block(x, style, orig) -> x``,
 enhanced_generator.py:114-117, :222-223).
 
-/root/reference exists only in the build container -- never on the GPU box -- so this file is
-used solely by ``oracle/make_golden.py`` and by the container-only ``-m "not gpu"`` tests that
-pin ``oracle/restate.py`` against the reference.  Nothing under ``multi_style_transfer_gan_b200/``
-may import it.
+The reference is not part of this repository, so this file is used solely by
+``oracle/make_golden.py`` and by the tests marked ``reference``, which skip without a checkout.
+Everything else is pinned to the reference by the vectors in ``tests/golden/``.  Nothing under
+``multi_style_transfer_gan_b200/`` may import it.
 """
 import os
 import sys
 import types
 import warnings
 
-REFERENCE_ROOT = os.environ.get("MSG_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("MSG_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def available() -> bool:

@@ -11,7 +11,7 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200, sm_100a)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs a checkout of the reference (oracle/ref_import.py)")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -23,7 +23,7 @@ def pytest_collection_modifyitems(config, items):
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
         if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
+            item.add_marker(pytest.mark.skip(reason=f"no checkout of the reference at {ref_import.REFERENCE_ROOT}"))
 
 
 @pytest.fixture(scope="session")

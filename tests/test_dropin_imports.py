@@ -73,12 +73,12 @@ print('load_models ok')
 def test_reference_load_models_runs_against_dropin():
     """batch_process_images.load_models of the UNMODIFIED reference (batch_process_images.py:60-120), imported with dropin/ first
     on sys.path: it builds OUR classes, loads both checkpoint layouts the reference writes, and the model call refuses a CPU
-    tensor loudly.  Needs /root/reference (build container only)."""
+    tensor loudly.  Needs a checkout of the reference (oracle/ref_import.py)."""
     import pytest
     from oracle import ref_import
     if not ref_import.available():
-        pytest.skip("/root/reference not present")
-    r = subprocess.run([sys.executable, "-c", LOAD_MODELS_SCRIPT, ROOT, os.path.join(ROOT, "dropin"), "/root/reference"],
+        pytest.skip(f"no checkout of the reference at {ref_import.REFERENCE_ROOT}")
+    r = subprocess.run([sys.executable, "-c", LOAD_MODELS_SCRIPT, ROOT, os.path.join(ROOT, "dropin"), ref_import.REFERENCE_ROOT],
                        capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stdout + r.stderr
     assert "load_models ok" in r.stdout

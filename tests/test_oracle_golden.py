@@ -139,9 +139,9 @@ def test_pretrain_generator(golden):
     loss = R.pretrain_masked_l1(y, g["real"], g["mask"])
     assert abs(float(loss) - float(g["loss"])) <= 1e-6
     loss.backward()
-    assert_parity(x.grad, g["dx"], 1e-4, "pretrain dx")
-    for k, ref in g["grads"].items():
-        assert_parity(params[k].grad, ref, 1e-4, f"pretrain grad {k}")
+    # the conv biases in front of each BatchNorm have an analytically-zero gradient (~1e-10 of rounding noise in the
+    # reference, which the summation order of the host's CPU changes): check_generator_grads tests them for ~0
+    check_generator_grads(g, x.grad, {k: p.grad for k, p in params.items()}, rel=1e-4)
     for k, ref in g["running_after"].items():
         assert torch.allclose(new[k].double(), ref.double(), rtol=1e-6, atol=1e-7), k
     sd2 = {k: v.detach() for k, v in sd.items()}
