@@ -1,5 +1,6 @@
 // ConvTranspose2d(k = 4, stride 2, pad 1) of the decoder (enhanced_generator.py:116-123, up2: 128 -> 64 channels) as a ROW RING of
-// tensor-memory accumulators (sm_100a, bf16 operands, fp32 accumulate) -- the transposed-conv sibling of msb_ring.cu.
+// tensor-memory accumulators (sm_100a, bf16 operands, fp32 accumulate) -- the transposed-conv sibling of msb_ring.cu; the shared
+// mechanics are in ring.cuh.
 //
 // out[o, u] = sum in[i, j] w[ky, kx] with o = 2 i - 1 + ky, u = 2 j - 1 + kx.  The four sub-pixel phase launches of the row-slab
 // path (conv_slab.cu) each re-read two input rows per output row and issue one N = 64 MMA per tap; here a CTA walks DOWN a
@@ -10,38 +11,29 @@
 //     eight-slot ring (slot = output row mod 8): for each of the two horizontal taps of the phase (a shifted view of the slab) ALL
 //     FOUR vertical taps are one tcgen05.mma of N = 256 over the weight stack [ky = 0 | 1 | 2 | 3] -- 2 to 4 MMAs per K step and
 //     input row instead of 16 (the ring wraps once every four rows: two N = 128 MMAs there);
-//   * input row r completes output rows 2r-1 and 2r: eight epilogue warps (lane quarter x channel half) drain both, zero the slots
-//     with tcgen05.st (every MMA accumulates), add the bias, accumulate the IN statistics, and hand their [32 px x 32 ch] pieces to
-//     the TMA store through a tensor map whose pixel stride is 2 (the other phase's pixels lie in between).
+//   * input row r completes output rows 2r-1 and 2r: eight epilogue warps (lane quarter x channel half) drain both and hand their
+//     [32 px x 32 ch] pieces to the TMA store through a tensor map whose pixel stride is 2 (the other phase's pixels lie in between).
 // A slot is touched again three input rows after its row completed, so the issuer may run LEAD = 3 rows ahead of the epilogue.
+// A piece [y0, y1) of input rows owns the output rows [2 y0, 2 y1) and reads the input rows y0 - 1 .. y1.
 // The schedule is stated and run on tensors in slab.py (convt_ring_row_mmas) / tests/test_convt_ring_cpu.py.
 //
 //   warp 0      TMA producer: the phase's weight stacks once, then one slab per input row
 //   warp 1      MMA issuer (also allocates TMEM)
 //   warps 4-11  epilogue
-#include <cuda.h>
-
-#include "common.cuh"
-#include "tcgen05.cuh"
+#include "ring.cuh"
 
 namespace msg {
 namespace {
-using namespace tc;
+using namespace ring;
 
-constexpr int BM = 128;                 // strip width (input pixels = output pixels of one phase)
-constexpr int HALO = 4;                 // slab pixels left of the strip (1 needed; 4 keeps the 64-channel blocks 1024-byte multiples)
-constexpr int SLAB_PX = BM + 2 * HALO;  // 136
-constexpr int SLAB_BYTES = SLAB_PX * 128;
-constexpr int EPI0 = 4;                 // first epilogue warp
 constexpr int NEW = 8;                  // epilogue warps
 constexpr int NC = 64;                  // output channels per launch = columns per row accumulator
-constexpr int NBAR = 8;
 constexpr uint32_t LEAD = 3;
-#ifndef CT_PREFETCH
-#define CT_PREFETCH 0                   // input rows pulled into L2 ahead of the slab ring: 0 / 4 / 8 measured 0.271 / 0.276 / 0.283 ms
-                                        // (16 x 256 x 256, 128 -> 64): the kernel is bound by the tensor pipe, not by load latency
-#endif
 constexpr int W_ROWS = 2 * 4 * NC;      // weight rows per 64-channel block of the input: [2 horizontal taps][4 ky][64 co]
+constexpr int OUT_B = 2048;             // per-warp scratch: [16 ch][32 px] fp32 for the statistics, then the [32 px][32 ch] bf16 piece
+
+template <int KB>
+__host__ __device__ constexpr Shape ct_shape() { return Shape{KB * W_ROWS * 128, KB * SLAB_BYTES, NC, NEW * OUT_B, 2}; }
 
 struct CtParams {
   int N, H, W, Co_total, co_off;        // input plane H x W; output 2H x 2W
@@ -58,161 +50,50 @@ template <int KB>
 __global__ void __launch_bounds__(32 * (EPI0 + NEW), 1)
 convt_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                   const __grid_constant__ CUtensorMap mapY, const CtParams p) {
-  constexpr int W_BYTES = KB * W_ROWS * 128;
-  constexpr int STAGE = KB * SLAB_BYTES;
-  constexpr int OUT_B = 2048;           // per-warp scratch: [16 ch][32 px] fp32 for the statistics, then the [32 px][32 ch] bf16 piece
+  constexpr Shape SH = ct_shape<KB>();
+  using Walk = Pieces<1, 1>;
   extern __shared__ uint8_t smem_raw[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int S = p.stages;
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t sB = base;                               // weight stacks [KB][W_ROWS][128 B], SW128
-  const uint32_t sA = sB + W_BYTES;                       // slab ring
-  const uint32_t sBias = sA + S * STAGE;                  // bias [64]
-  const uint32_t sOut = (sBias + NC * 4 + 127u) & ~127u;  // per-warp scratch [NEW][OUT_B]
-  const uint32_t sBar = (sOut + NEW * OUT_B + 7u) & ~7u;
-  float* sbias = reinterpret_cast<float*>(gen + (sBias - base));
-  auto full_bar = [&](int s) { return sBar + 8u * s; };
-  auto empty_bar = [&](int s) { return sBar + 8u * (S + s); };
-  const uint32_t wres_bar = sBar + 8u * (2 * S);
-  auto rowdone_bar = [&](uint32_t k) { return sBar + 8u * (2 * S + 1 + (k & (NBAR - 1))); };
-  auto drained_bar = [&](uint32_t k) { return sBar + 8u * (2 * S + 1 + NBAR + (k & (NBAR - 1))); };
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(gen + (sBar - base) + 8 * (2 * S + 1 + 2 * NBAR));
+  const Smem sm(smem_raw, SH, p.stages);
+  const Bars& bars = sm.b;
+  float* sbias = sm.bias();
 
   if (tid < NC) sbias[tid] = p.bias ? p.bias[tid] : 0.f;
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < S; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-      mbar_init(wres_bar, 1);
-      for (int k = 0; k < NBAR; ++k) { mbar_init(rowdone_bar(k), 1); mbar_init(drained_bar(k), NEW); }
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  } else if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapB)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapY)) : "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  if (warp >= EPI0 && warp < EPI0 + 4) {  // every accumulator starts at zero: each MMA of the kernel accumulates
-    const uint32_t lane_addr = (uint32_t)((warp & 3) * 32) << 16;
-    uint32_t z[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) z[i] = 0u;
-    for (int c = 0; c < 512; c += 32) tmem_st32(tmem_base + lane_addr + (uint32_t)c, z);
-    tmem_st_wait();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-
-  // Work = the INPUT rows of all column strips laid end to end, an equal share per CTA (msb_ring.cu): a piece [y0, y1) of input rows
-  // owns the output rows [2 y0, 2 y1) and reads the input rows y0 - 1 .. y1.
-  const long long g_lo = (long long)blockIdx.x * p.total_rows / gridDim.x, g_hi = (long long)(blockIdx.x + 1) * p.total_rows / gridDim.x;
-  auto item = [&](long long g, int& img, int& seg, int& y0, int& y1) {
-    const int strip = (int)(g / p.H);
-    y0 = (int)(g - (long long)strip * p.H);
-    const long long left = g_hi - g;
-    y1 = (long long)(p.H - y0) < left ? p.H : y0 + (int)left;
-    img = strip / p.segs;
-    seg = strip - img * p.segs;
-  };
+  const uint32_t tmem_base = prologue(sm, warp, lane, 1, NEW, 0, &mapA, &mapB, &mapY);
+  const Walk pieces(p.total_rows, p.H, p.segs);
 
   if (warp == 0) {
-    // ===================================== TMA producer =====================================
-    if (lane == 0) {
-      mbar_expect_tx(wres_bar, (uint32_t)W_BYTES);
-      for (int r = 0; r < KB * W_ROWS; r += 64) tma_load_2d(sB + r * 128, &mapB, wres_bar, 0, p.w_row0 + r);
-      int s = 0;
-      uint32_t n = 0;                      // slabs issued
-      for (long long g = g_lo; g < g_hi;) {
-        int img, seg, y0, y1;
-        item(g, img, seg, y0, y1);
-        g += y1 - y0;
-        const int r_lo = y0 - 1 < 0 ? 0 : y0 - 1, r_hi = y1 + 1 > p.H ? p.H : y1 + 1;
-        for (int r = r_lo; r < r_hi; ++r, ++n) {
-#if CT_PREFETCH > 0
-          // the slab ring is only two deep at Cin = 128 (the weights take 128 KB): rows further ahead are pulled into L2, so the
-          // load that fills a freed stage pays L2 latency, not DRAM latency
-          if (r == r_lo)
-            for (int a = 1; a < CT_PREFETCH && r + a < r_hi; ++a)
+    if (lane == 0)
+      producer(sm, pieces, p.H, &mapB, SH.w_bytes, p.w_row0, SH.stage_bytes, [&](const Walk& pc, int r, uint32_t dst, uint32_t bar) {
 #pragma unroll
-              for (int kb = 0; kb < KB; ++kb) tma_prefetch_4d(&mapA, kb * 64, seg * BM - HALO, r + a, img);
-          if (r + CT_PREFETCH < r_hi)
-#pragma unroll
-            for (int kb = 0; kb < KB; ++kb) tma_prefetch_4d(&mapA, kb * 64, seg * BM - HALO, r + CT_PREFETCH, img);
-#endif
-          if (n >= (uint32_t)S) mbar_wait(empty_bar(s), ((n / S) - 1) & 1);
-          mbar_expect_tx(full_bar(s), (uint32_t)STAGE);
-#pragma unroll
-          for (int kb = 0; kb < KB; ++kb)
-            tma_load_4d(sA + s * STAGE + kb * SLAB_BYTES, &mapA, full_bar(s), kb * 64, seg * BM - HALO, r, img);
-          if (++s == S) s = 0;
-        }
-      }
-    }
+        for (int kb = 0; kb < KB; ++kb) tma_load_4d(dst + kb * SLAB_BYTES, &mapA, bar, kb * 64, pc.seg * BM - HALO, r, pc.img);
+      });
   } else if (warp == 1) {
-    // ===================================== MMA issuer =====================================
     const bool leader = elect_one();
     const uint32_t hi = (uint32_t)(make_sw128_desc(0) >> 32);
-    const uint32_t idesc0 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BM >> 4) << 24);      // + N
-    const uint32_t b_base = sB >> 4;
+    const uint32_t b_base = sm.sB() >> 4;
     const int dx1 = p.px == 0 ? -1 : 1;    // the phase's second horizontal tap reads the neighbour pixel on this side
-    int s = 0;
-    uint32_t n = 0, k = 0;                 // slabs consumed, global step count
-    mbar_wait(wres_bar, 0);
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      for (int r = y0 - 1; r < y1 + 1; ++r, ++k) {
-        if (k >= LEAD) mbar_wait(drained_bar(k - LEAD), ((k - LEAD) / NBAR) & 1);
-        // a new piece maps its rows onto the slots afresh: everything of the previous piece must have been drained
-        if (r == y0 - 1 && k > 0) mbar_wait(drained_bar(k - 1), ((k - 1) / NBAR) & 1);
-        if (r >= 0 && r < p.H) {
-          mbar_wait(full_bar(s), (n / S) & 1);
-          tc_fence_after();
-          if (leader) {
-            const uint32_t a0 = (sA + s * STAGE) >> 4;
-            // entries e = ky = 0..3 = output rows 2r-1 .. 2r+2; those of this piece are an interval whose ring slots are adjacent
-            // except where the ring wraps: one or two runs, found by arithmetic (no run table in local memory)
-            auto issue_run = [&](int e, int nrun, int slot) {
-              const uint32_t idesc = idesc0 | ((uint32_t)((NC * nrun) >> 3) << 17);
-              const uint32_t dcol = tmem_base + (uint32_t)(slot * NC);
+    issuer<LEAD, false>(bars, pieces, p.H, leader, [&](const Walk& pc, int r, int s) {
+      const uint32_t a0 = sm.sA(s, SH.stage_bytes) >> 4;
+      // entries e = ky = 0..3 = output rows 2r-1 .. 2r+2; those of this piece are an interval of adjacent ring slots
+      const int o_lo = 2 * r - 1 > 2 * pc.y0 ? 2 * r - 1 : 2 * pc.y0, o_hi = 2 * r + 2 < 2 * pc.y1 - 1 ? 2 * r + 2 : 2 * pc.y1 - 1;   // inclusive
+      if (o_lo <= o_hi)
+        runs(o_hi - o_lo + 1, o_lo & 7, 8, [&](int e, int nrun, int slot) {
+          const uint32_t idesc = idesc_bf16(NC * nrun);
+          const uint32_t dcol = tmem_base + (uint32_t)(slot * NC);
 #pragma unroll
-              for (int t = 0; t < 2; ++t) {
-                const uint32_t wrow = (uint32_t)(t * 4 * NC + NC * e);
-                const uint32_t av = a0 + (uint32_t)((HALO + (t == 0 ? 0 : dx1)) * 8);
+          for (int t = 0; t < 2; ++t) {
+            const uint32_t wrow = (uint32_t)(t * 4 * NC + NC * (o_lo - (2 * r - 1) + e));
+            const uint32_t av = a0 + (uint32_t)((HALO + (t == 0 ? 0 : dx1)) * 8);
 #pragma unroll
-                for (int kb = 0; kb < KB; ++kb)
+            for (int kb = 0; kb < KB; ++kb)
 #pragma unroll
-                  for (int ks = 0; ks < 4; ++ks)
-                    umma_bf16_lo(dcol, av + (uint32_t)(kb * (SLAB_BYTES >> 4) + 2 * ks),
-                                 b_base + (uint32_t)(kb * W_ROWS * 8) + wrow * 8u + (uint32_t)(2 * ks), hi, idesc, true);
-              }
-            };
-            const int o_lo = 2 * r - 1 > 2 * y0 ? 2 * r - 1 : 2 * y0, o_hi = 2 * r + 2 < 2 * y1 - 1 ? 2 * r + 2 : 2 * y1 - 1;      // inclusive
-            if (o_lo <= o_hi) {
-              const int cnt = o_hi - o_lo + 1, slot = o_lo & 7;
-              const int n1 = cnt < 8 - slot ? cnt : 8 - slot;
-              issue_run(o_lo - (2 * r - 1), n1, slot);
-              if (cnt > n1) issue_run(o_lo - (2 * r - 1) + n1, cnt - n1, 0);
-            }
-            umma_commit(empty_bar(s));
+              for (int ks = 0; ks < 4; ++ks)
+                umma_bf16_lo(dcol, av + (uint32_t)(kb * (SLAB_BYTES >> 4) + 2 * ks),
+                             b_base + (uint32_t)(kb * W_ROWS * 8) + wrow * 8u + (uint32_t)(2 * ks), hi, idesc, true);
           }
-          __syncwarp();
-          if (++s == S) s = 0;
-          ++n;
-        }
-        if (leader) umma_commit(rowdone_bar(k));     // arrives when every MMA issued so far has completed
-        __syncwarp();
-      }
-    }
+        });
+    });
   } else if (warp >= EPI0) {
     // ===================================== epilogue: warp = (lane quarter q, channel half h) =====================================
     const int q = warp & 3;
@@ -220,34 +101,19 @@ convt_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
     const int h = ew >> 2;                            // channels [32 h, 32 h + 32) of the launch's 64
     const int row = q * 32 + lane;                    // strip pixel = TMEM lane
     const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-    uint8_t* buf = gen + (sOut - base) + ew * OUT_B;
-    float2 ws = make_float2(0.f, 0.f), wq = make_float2(0.f, 0.f);     // lane l: running sum / sum of squares of channel 32 h + l
+    uint8_t* buf = sm.scratch(ew, OUT_B);
+    Stats stats;                                      // lane l: channel 32 h + l
     const bool do_stats = p.stats != nullptr;
-    int stat_img = -1;
-    auto flush_stats = [&]() {
-      if (stat_img >= 0) {
-        double* st = p.stats + ((size_t)stat_img * p.Co_total + p.co_off + 32 * h + lane) * 2;
-        atomicAdd(st, f2sum_value(ws));
-        atomicAdd(st + 1, f2sum_value(wq));
-      }
-      ws = make_float2(0.f, 0.f); wq = make_float2(0.f, 0.f);
-    };
-    uint32_t zero32[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) zero32[i] = 0u;
     uint32_t k = 0;
     bool stored = false;                   // a TMA store of this warp may still be reading buf
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      const bool valid = seg * BM + row < p.W;
-      if (do_stats && img != stat_img) { flush_stats(); stat_img = img; }
-      for (int r = y0 - 1; r < y1 + 1; ++r, ++k) {
-        mbar_wait(rowdone_bar(k), (k / NBAR) & 1);
+    for (Walk pc = pieces; pc.next();) {
+      const bool valid = pc.seg * BM + row < p.W;
+      if (do_stats && pc.img != stats.img) { stats.flush<32>(p.stats, p.Co_total, p.co_off + 32 * h, lane); stats.img = pc.img; }
+      for (int r = pc.r0; r < pc.r1; ++r, ++k) {
+        bars.wait_rowdone(k);
         // input row r completed the output rows 2r - 1 and 2r (those of this piece)
         const int oA = 2 * r - 1, oB = 2 * r;
-        const bool okA = oA >= 2 * y0 && oA < 2 * y1, okB = oB >= 2 * y0 && oB < 2 * y1;        // (warp-uniform)
+        const bool okA = oA >= 2 * pc.y0 && oA < 2 * pc.y1, okB = oB >= 2 * pc.y0 && oB < 2 * pc.y1;        // (warp-uniform)
         float vA[32], vB[32];
         if (okA | okB) {
           tc_fence_after();
@@ -256,116 +122,30 @@ convt_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
           if (okA) tmem_ld32(tA, vA);
           if (okB) tmem_ld32(tB, vB);
           tmem_ld_wait();
-          if (okA) tmem_st32(tA, zero32);              // the slots are free for the rows that wrap onto them
-          if (okB) tmem_st32(tB, zero32);
+          if (okA) tmem_zero<32>(tA);
+          if (okB) tmem_zero<32>(tB);
           tmem_st_wait();
           tc_fence_before();
         }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(drained_bar(k));    // handed back before anything else: the issuer waits on this
+        arrive_drained(bars, k, lane);
 #pragma unroll
         for (int half = 0; half < 2; ++half) {
           if (!(half == 0 ? okA : okB)) continue;
           float (&v)[32] = half == 0 ? vA : vB;
-          const int o = half == 0 ? oA : oB;
 #pragma unroll
           for (int c = 0; c < 32; ++c) v[c] += sbias[32 * h + c];
-          if (stored) {                                // the previous piece's store has read buf
-            if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            __syncwarp();
-          }
-          if (do_stats) {
-            // per-channel sums over the warp's 32 pixels, 16 channels at a time through buf as [16 ch][32 px] fp32 (pixel index XOR
-            // channel: conflict-free both ways); lane (c, half) sums 16 pixels of channel c in a fixed order, one shuffle joins the
-            // halves; lane l accumulates channel l (msb_ring.cu)
-            float* sc = reinterpret_cast<float*>(buf);
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-#pragma unroll
-              for (int c = 0; c < 16; ++c) sc[c * 32 + (lane ^ c)] = valid ? v[16 * hh + c] : 0.f;
-              __syncwarp();
-              const int c = lane & 15, r0 = lane & 16;
-              float cs0 = 0.f, cs1 = 0.f, q0 = 0.f, q1 = 0.f;
-#pragma unroll
-              for (int j = 0; j < 16; j += 2) {
-                const float x0 = sc[c * 32 + ((r0 + j) ^ c)], x1 = sc[c * 32 + ((r0 + j + 1) ^ c)];
-                cs0 += x0; cs1 += x1;
-                q0 = fmaf(x0, x0, q0); q1 = fmaf(x1, x1, q1);
-              }
-              float cs = cs0 + cs1, qs = q0 + q1;
-              const float cs_o = __shfl_xor_sync(0xffffffffu, cs, 16), qs_o = __shfl_xor_sync(0xffffffffu, qs, 16);
-              cs = r0 ? cs_o + cs : cs + cs_o;         // pixels 0-15 first on both halves: the same bits
-              qs = r0 ? qs_o + qs : qs + qs_o;
-              if ((lane >> 4) == hh) { f2sum_add(ws, cs); f2sum_add(wq, qs); }
-              __syncwarp();
-            }
-          }
-          // the warp's [32 pixels x 32 channels] piece into buf (rows of 64 bytes, dense; the 16-byte chunk a lane writes at step j is
-          // rotated by the lane so that the eight lanes of a store phase cover all 32 banks), then ONE TMA store: the tensor map's
-          // pixel stride is 2 (this phase's pixels of the output row) and it clips pixels beyond the plane
-          uint4 pk[4];
-#pragma unroll
-          for (int c8 = 0; c8 < 4; ++c8) {
-            float o8[8];
-#pragma unroll
-            for (int c = 0; c < 8; ++c) o8[c] = v[c8 * 8 + c];
-            pk[c8] = pack8(o8);
-          }
-          const int rot = (lane >> 1) & 3;
-#pragma unroll
-          for (int bit = 1; bit < 4; bit <<= 1) {
-            const bool sw = (rot & bit) != 0;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              if (j & bit) continue;
-              const uint4 a = pk[j], c2 = pk[j | bit];
-              pk[j] = sw ? c2 : a;
-              pk[j | bit] = sw ? a : c2;
-            }
-          }
-#pragma unroll
-          for (int j = 0; j < 4; ++j) *reinterpret_cast<uint4*>(buf + lane * 64 + (j ^ rot) * 16) = pk[j];
-          fence_proxy_async();
-          __syncwarp();
-          if (lane == 0) {
-            tma_store_4d(&mapY, smem_u32(buf), p.co_off + 32 * h, seg * BM + q * 32, o, img);
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-          }
+          if (stored) wait_store_read<0>(lane);      // the previous piece's store has read buf
+          if (do_stats) piece_stats<32>(reinterpret_cast<float*>(buf), v, valid, lane, stats);
+          // this phase's pixels of the output row: the tensor map's pixel stride is 2
+          store_piece_bf16<32>(buf, v, lane, &mapY, p.co_off + 32 * h, pc.seg * BM + q * 32, half == 0 ? oA : oB, pc.img);
           stored = true;
         }
       }
     }
-    if (do_stats) flush_stats();
+    if (do_stats) stats.flush<32>(p.stats, p.Co_total, p.co_off + 32 * h, lane);
     if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-  }
-}
-
-template <int KB>
-int launch_phase(const CUtensorMap& mapA, const CUtensorMap& mapB, const CUtensorMap& mapY, CtParams p, cudaStream_t st) {
-  constexpr int W_BYTES = KB * W_ROWS * 128, STAGE = KB * SLAB_BYTES;
-  const int fixed = W_BYTES + NC * 4 + 128 + NEW * 2048 + 8 + 384 + 1024;
-  int stages = (227 * 1024 - fixed) / STAGE;
-  if (stages > 8) stages = 8;
-  MSG_REQUIRE(stages >= 2, MSG_ERR_UNSUPPORTED, "convt_ring: the slab ring does not fit shared memory (Cin = %d)", KB * 64);
-  p.stages = stages;
-  const size_t smem = (size_t)stages * STAGE + fixed;
-  static DeviceOnce attr_set;
-  if (attr_set.needed()) {
-    cudaError_t e = cudaFuncSetAttribute(convt_ring_kernel<KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    MSG_REQUIRE(e == cudaSuccess, MSG_ERR_CUDA, "convt_ring: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    attr_set.done();
-  }
-  const int sms = sm_count();
-  const long long grid_ll = p.total_rows / 4;       // at least 4 input rows per CTA (each piece re-reads 2 halo rows)
-  const int grid = grid_ll < 1 ? 1 : (grid_ll > sms ? sms : (int)grid_ll);
-  convt_ring_kernel<KB><<<grid, 32 * (EPI0 + NEW), smem, st>>>(mapA, mapB, mapY, p);
-  return check_launch("convt_ring_kernel");
+  teardown(warp, tmem_base);
 }
 
 }  // namespace
@@ -385,8 +165,7 @@ extern "C" int msg_convt_ring(const msg_convt_ring_desc* d, const void* x, const
   MSG_REQUIRE((d->Co_total & 7) == 0 && (d->co_off & 7) == 0 && d->co_off + d->Cout <= d->Co_total, MSG_ERR_SHAPE, "convt_ring: output channel layout");
   MSG_REQUIRE((((uintptr_t)x | (uintptr_t)w_stacks | (uintptr_t)y) & 15) == 0, MSG_ERR_ALIGN, "convt_ring: operands must be 16-byte aligned");
   MSG_REQUIRE(!(d->flags & MSG_CONV_STATS) || stats != nullptr, MSG_ERR_SHAPE, "convt_ring: stats buffer missing");
-  EncodeTiledFn enc = get_encode();
-  MSG_REQUIRE(enc != nullptr, MSG_ERR_CUDA, "convt_ring: cuTensorMapEncodeTiled unavailable");
+  MSG_REQUIRE(get_encode() != nullptr, MSG_ERR_CUDA, "convt_ring: cuTensorMapEncodeTiled unavailable");
   const int KB = d->Cin / 64, G = d->Cout / 64;
 
   CtParams p;
@@ -397,43 +176,25 @@ extern "C" int msg_convt_ring(const msg_convt_ring_desc* d, const void* x, const
   MSG_REQUIRE(p.total_rows < (1LL << 40), MSG_ERR_SHAPE, "convt_ring: too many rows");
 
   CUtensorMap mapA, mapB;
-  {
-    cuuint64_t dims[4] = {(cuuint64_t)d->Cin, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-    cuuint64_t strides[3] = {(cuuint64_t)d->Ci_total * 2, (cuuint64_t)d->W * d->Ci_total * 2, (cuuint64_t)d->H * d->W * d->Ci_total * 2};
-    cuuint32_t box[4] = {64, (cuuint32_t)SLAB_PX, 1, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    void* b0 = (void*)((const __nv_bfloat16*)x + d->ci_off);
-    CUresult r = enc(&mapA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, b0, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "convt_ring: cuTensorMapEncodeTiled(x) failed with %d", (int)r);
-  }
-  {
-    cuuint64_t dims[2] = {64, (cuuint64_t)G * 2 * KB * W_ROWS};
-    cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, 64};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = enc(&mapB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)w_stacks, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "convt_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
-  }
+  CUresult r = encode_slab(&mapA, (const __nv_bfloat16*)x + d->ci_off, d->Cin, d->Ci_total, d->W, d->H, d->N);
+  MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "convt_ring: cuTensorMapEncodeTiled(x) failed with %d", (int)r);
+  r = encode_weights(&mapB, w_stacks, (long long)G * 2 * KB * W_ROWS);
+  MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "convt_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
   for (int g = 0; g < G; ++g)
     for (int px = 0; px < 2; ++px) {
       CUtensorMap mapY;
       // this phase's pixels of the output: pixel stride 2, starting at pixel px
-      cuuint64_t dims[4] = {(cuuint64_t)d->Co_total, (cuuint64_t)d->W, (cuuint64_t)2 * d->H, (cuuint64_t)d->N};
-      cuuint64_t strides[3] = {(cuuint64_t)2 * d->Co_total * 2, (cuuint64_t)2 * d->W * d->Co_total * 2,
-                               (cuuint64_t)4 * d->H * d->W * d->Co_total * 2};
-      cuuint32_t box[4] = {32, 32, 1, 1};
-      cuuint32_t es[4] = {1, 1, 1, 1};
-      void* y0 = (void*)((__nv_bfloat16*)y + (size_t)px * d->Co_total);
-      CUresult r = enc(&mapY, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y0, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                       CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+      r = encode_store(&mapY, (__nv_bfloat16*)y + (size_t)px * d->Co_total, d->Co_total, d->W, 2 * d->H, d->N, 32, 2);
       MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "convt_ring: cuTensorMapEncodeTiled(y) failed with %d", (int)r);
       p.px = px;
       p.co_off = d->co_off + 64 * g;
       p.bias = bias ? bias + 64 * g : nullptr;
       p.w_row0 = (g * 2 + px) * KB * W_ROWS;
-      const int rc = KB == 1 ? launch_phase<1>(mapA, mapB, mapY, p, st) : launch_phase<2>(mapA, mapB, mapY, p, st);
+      // at least 4 input rows per CTA (each piece re-reads 2 halo rows)
+      const int rc = KB == 1 ? launch<convt_ring_kernel<1>>("convt_ring_kernel", ct_shape<1>(), 32 * (EPI0 + NEW), p.total_rows, 4, p,
+                                                            mapA, mapB, mapY, st)
+                             : launch<convt_ring_kernel<2>>("convt_ring_kernel", ct_shape<2>(), 32 * (EPI0 + NEW), p.total_rows, 4, p,
+                                                            mapA, mapB, mapY, st);
       if (rc) return rc;
     }
   return MSG_OK;

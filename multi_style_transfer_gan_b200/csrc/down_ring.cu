@@ -1,6 +1,7 @@
 // The first down-sampling conv of the encoder (enhanced_generator.py:99-104: Conv2d(c, 2c, 4, stride 2, padding 1), c = 64) fused with
 // the InstanceNorm + ReLU of the 7x7 input layer in front of it (enhanced_generator.py:93-97), as a ROW RING of tensor-memory
-// accumulators (sm_100a, bf16 operands, fp32 accumulate) -- the stride-2 member of the msb_ring.cu / convt_ring.cu / out7_ring.cu family.
+// accumulators (sm_100a, bf16 operands, fp32 accumulate) -- the stride-2 member of the msb_ring.cu / convt_ring.cu / out7_ring.cu family
+// (shared mechanics in ring.cuh).
 //
 //   a = ReLU(IN(x))              x: raw output of the 7x7 input conv with its plane statistics
 //   y[o, u] = sum a[2o - 1 + ky, 2u - 1 + kx] w[ky, kx] + b      (+ IN statistics of y)
@@ -16,38 +17,29 @@
 //   * input row r feeds two output rows -- (r-1)/2 rounded down and the next one -- whose accumulators are adjacent 64-column slots of
 //     an eight-slot ring: per horizontal tap the two vertical taps are ONE MMA of N = 128 (full rate on the tensor pipe), 16 MMAs per
 //     input row at c = 64;
-//   * every second input row completes an output row: eight epilogue warps (lane quarter x channel half) drain it, zero the slot,
-//     add the bias, accumulate the IN statistics and hand [32 px x 32 ch] pieces to the TMA store.
+//   * every second input row completes an output row: eight epilogue warps (lane quarter x channel half) drain it and hand
+//     [32 px x 32 ch] pieces to the TMA store.
+// A piece [y0, y1) of OUTPUT rows reads the input rows 2 y0 - 1 .. 2 y1, one step each.
 // Schedule stated and run on tensors in slab.py (down_ring_row_mmas) / tests/test_down_ring_cpu.py.
 //
 //   warp 0       TMA producer: the launch's weight stacks once, then the even / odd slabs of one input row per stage
 //   warp 1       MMA issuer (also allocates TMEM)
 //   warps 4-11   epilogue
 //   warps 12-15  transform
-#include <cuda.h>
-
-#include "common.cuh"
-#include "tcgen05.cuh"
+#include "ring.cuh"
 
 namespace msg {
 namespace {
-using namespace tc;
+using namespace ring;
 
-constexpr int BM = 128;                 // strip width in OUTPUT pixels
-constexpr int HALO = 4;                 // slab pixels (of one parity) left of the strip (1 needed)
-constexpr int SLAB_PX = BM + 2 * HALO;  // 136
-constexpr int SLAB_BYTES = SLAB_PX * 128;
-constexpr int STAGE = 2 * SLAB_BYTES;   // even pixels | odd pixels of one input row, 64 channels
 constexpr int NC = 64;                  // output channels per launch = columns per row accumulator
-constexpr int EPI0 = 4, NEW = 8, XF0 = 12;
-constexpr int NBAR = 8;
+constexpr int NEW = 8, XF0 = 12;
 constexpr uint32_t LEAD = 8;            // a slot is touched again 13 steps after its row completed
 constexpr int W_ROWS = 4 * 2 * 2 * NC;  // [kx][input-row parity][entry][64 co] rows of 64 input channels
-constexpr int W_BYTES = W_ROWS * 128;
 constexpr int NTHREADS = 32 * 16;
-#ifndef DN_PREFETCH
-#define DN_PREFETCH 0                   // input rows pulled into L2 ahead of the two-stage slab ring: 0 / 4 measured the same (0.462 / 0.463 ms)
-#endif
+constexpr int OUT_B = 2048;             // per-warp scratch: [16 ch][32 px] fp32 for the statistics, then the [32 px][32 ch] bf16 piece
+// weights | stages of the even | odd pixels of one input row, 64 channels | bias | scratch; full / empty / transformed per stage
+__host__ __device__ constexpr Shape dn_shape() { return Shape{W_ROWS * 128, 2 * SLAB_BYTES, NC, NEW * OUT_B, 3}; }
 
 struct DnParams {
   int N, H, W;                          // input plane (H, W even); output H/2 x W/2
@@ -65,155 +57,49 @@ struct DnParams {
 __global__ void __launch_bounds__(NTHREADS, 1)
 down_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                  const __grid_constant__ CUtensorMap mapY, const DnParams p) {
-  constexpr int OUT_B = 2048;           // per-warp scratch: [16 ch][32 px] fp32 for the statistics, then the [32 px][32 ch] bf16 piece
+  constexpr Shape SH = dn_shape();
+  using Walk = Pieces<2, 1>;
   extern __shared__ uint8_t smem_raw[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int S = p.stages;
   const int Ho = p.H >> 1, Wo = p.W >> 1;
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t sB = base;
-  const uint32_t sA = sB + W_BYTES;
-  const uint32_t sBias = sA + S * STAGE;
-  const uint32_t sOut = (sBias + NC * 4 + 127u) & ~127u;
-  const uint32_t sBar = (sOut + NEW * OUT_B + 7u) & ~7u;
-  float* sbias = reinterpret_cast<float*>(gen + (sBias - base));
-  auto full_bar = [&](int s) { return sBar + 8u * s; };
-  auto empty_bar = [&](int s) { return sBar + 8u * (S + s); };
-  auto xf_bar = [&](int s) { return sBar + 8u * (2 * S + s); };
-  const uint32_t wres_bar = sBar + 8u * (3 * S);
-  auto rowdone_bar = [&](uint32_t k) { return sBar + 8u * (3 * S + 1 + (k & (NBAR - 1))); };
-  auto drained_bar = [&](uint32_t k) { return sBar + 8u * (3 * S + 1 + NBAR + (k & (NBAR - 1))); };
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(gen + (sBar - base) + 8 * (3 * S + 1 + 2 * NBAR));
+  const Smem sm(smem_raw, SH, p.stages);
+  const Bars& bars = sm.b;
+  float* sbias = sm.bias();
 
   if (tid < NC) sbias[tid] = p.bias ? p.bias[tid] : 0.f;
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < S; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); mbar_init(xf_bar(s), 4); }
-      mbar_init(wres_bar, 1);
-      for (int k = 0; k < NBAR; ++k) { mbar_init(rowdone_bar(k), 1); mbar_init(drained_bar(k), NEW); }
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  } else if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapB)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapY)) : "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  if (warp >= EPI0 && warp < EPI0 + 4) {  // every accumulator starts at zero: each MMA of the kernel accumulates
-    const uint32_t lane_addr = (uint32_t)((warp & 3) * 32) << 16;
-    uint32_t z[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) z[i] = 0u;
-    for (int c = 0; c < 512; c += 32) tmem_st32(tmem_base + lane_addr + (uint32_t)c, z);
-    tmem_st_wait();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-
-  // Work = the OUTPUT rows of all column strips laid end to end, an equal share per CTA (msb_ring.cu): a piece [y0, y1) of output
-  // rows reads the input rows 2 y0 - 1 .. 2 y1, one step each.
-  const long long g_lo = (long long)blockIdx.x * p.total_rows / gridDim.x, g_hi = (long long)(blockIdx.x + 1) * p.total_rows / gridDim.x;
-  auto item = [&](long long g, int& img, int& seg, int& y0, int& y1) {
-    const int strip = (int)(g / Ho);
-    y0 = (int)(g - (long long)strip * Ho);
-    const long long left = g_hi - g;
-    y1 = (long long)(Ho - y0) < left ? Ho : y0 + (int)left;
-    img = strip / p.segs;
-    seg = strip - img * p.segs;
-  };
+  const uint32_t tmem_base = prologue(sm, warp, lane, 1, NEW, 4, &mapA, &mapB, &mapY);
+  const Walk pieces(p.total_rows, Ho, p.segs);
 
   if (warp == 0) {
-    // ===================================== TMA producer =====================================
-    if (lane == 0) {
-      mbar_expect_tx(wres_bar, (uint32_t)W_BYTES);
-      for (int r = 0; r < W_ROWS; r += 64) tma_load_2d(sB + r * 128, &mapB, wres_bar, 0, p.w_row0 + r);
-      int s = 0;
-      uint32_t n = 0;
-      for (long long g = g_lo; g < g_hi;) {
-        int img, seg, y0, y1;
-        item(g, img, seg, y0, y1);
-        g += y1 - y0;
-        const int r_lo = 2 * y0 - 1 < 0 ? 0 : 2 * y0 - 1, r_hi = 2 * y1 + 1 > p.H ? p.H : 2 * y1 + 1;
-        for (int r = r_lo; r < r_hi; ++r, ++n) {
-#if DN_PREFETCH > 0
-          // Two stages (the weights take 128 KB) = one load in flight: rows further ahead are pulled into L2, so that the load filling
-          // a freed stage pays L2 latency instead of DRAM latency
-          if (r == r_lo)
-            for (int a = 1; a < DN_PREFETCH && r + a < r_hi; ++a)
-              for (int par = 0; par < 2; ++par) tma_prefetch_5d(&mapA, 0, par, seg * BM - HALO, r + a, img);
-          if (r + DN_PREFETCH < r_hi)
-            for (int par = 0; par < 2; ++par) tma_prefetch_5d(&mapA, 0, par, seg * BM - HALO, r + DN_PREFETCH, img);
-#endif
-          if (n >= (uint32_t)S) mbar_wait(empty_bar(s), ((n / S) - 1) & 1);
-          mbar_expect_tx(full_bar(s), (uint32_t)STAGE);
-          tma_load_5d(sA + s * STAGE, &mapA, full_bar(s), 0, 0, seg * BM - HALO, r, img);                  // even pixels
-          tma_load_5d(sA + s * STAGE + SLAB_BYTES, &mapA, full_bar(s), 0, 1, seg * BM - HALO, r, img);     // odd pixels
-          if (++s == S) s = 0;
-        }
-      }
-    }
+    if (lane == 0)
+      producer(sm, pieces, p.H, &mapB, SH.w_bytes, p.w_row0, SH.stage_bytes, [&](const Walk& pc, int r, uint32_t dst, uint32_t bar) {
+        tma_load_5d(dst, &mapA, bar, 0, 0, pc.seg * BM - HALO, r, pc.img);                  // even pixels
+        tma_load_5d(dst + SLAB_BYTES, &mapA, bar, 0, 1, pc.seg * BM - HALO, r, pc.img);     // odd pixels
+      });
   } else if (warp == 1) {
-    // ===================================== MMA issuer =====================================
     const bool leader = elect_one();
     const uint32_t hi = (uint32_t)(make_sw128_desc(0) >> 32);
-    const uint32_t idesc0 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BM >> 4) << 24);      // + N
-    const uint32_t b_base = sB >> 4;
-    int s = 0;
-    uint32_t n = 0, k = 0;
-    mbar_wait(wres_bar, 0);
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      for (int r = 2 * y0 - 1; r < 2 * y1 + 1; ++r, ++k) {
-        if (k >= LEAD) mbar_wait(drained_bar(k - LEAD), ((k - LEAD) / NBAR) & 1);
-        // a new piece maps its rows onto the slots afresh: everything of the previous piece must have been drained
-        if (r == 2 * y0 - 1 && k > 0) mbar_wait(drained_bar(k - 1), ((k - 1) / NBAR) & 1);
-        if (r >= 0 && r < p.H) {
-          mbar_wait(xf_bar(s), (n / S) & 1);
-          tc_fence_after();
-          if (leader) {
-            const uint32_t a0 = (sA + s * STAGE) >> 4;
-            const int par = r & 1;
-            // entries e = 0, 1 = output rows of = (r - 1) >> 1 and of + 1 (vertical taps ky = 3 - par, 1 - par)
-            auto issue_run = [&](int e, int nrun, int slot) {
-              const uint32_t idesc = idesc0 | ((uint32_t)((NC * nrun) >> 3) << 17);
-              const uint32_t dcol = tmem_base + (uint32_t)(slot * NC);
+    const uint32_t b_base = sm.sB() >> 4;
+    issuer<LEAD, true>(bars, pieces, p.H, leader, [&](const Walk& pc, int r, int s) {
+      const uint32_t a0 = sm.sA(s, SH.stage_bytes) >> 4;
+      const int par = r & 1;
+      // entries e = 0, 1 = output rows of = (r - 1) >> 1 and of + 1 (vertical taps ky = 3 - par, 1 - par)
+      const int of = (r - 1) >> 1;                             // (arithmetic shift: r = 0 -> -1)
+      const int o_lo = of > pc.y0 ? of : pc.y0, o_hi = of + 1 < pc.y1 - 1 ? of + 1 : pc.y1 - 1;      // inclusive
+      if (o_lo <= o_hi)
+        runs(o_hi - o_lo + 1, o_lo & 7, 8, [&](int e, int nrun, int slot) {
+          const uint32_t idesc = idesc_bf16(NC * nrun);
+          const uint32_t dcol = tmem_base + (uint32_t)(slot * NC);
 #pragma unroll
-              for (int kx = 0; kx < 4; ++kx) {
-                // kx = 0: odd pixels at u - 1; 1: even at u; 2: odd at u; 3: even at u + 1
-                const uint32_t av = a0 + (uint32_t)(((kx & 1) ? 0 : (SLAB_BYTES >> 4)) + (HALO + (kx == 0 ? -1 : (kx == 3 ? 1 : 0))) * 8);
-                const uint32_t bv = b_base + (uint32_t)((((kx * 2 + par) * 2 + e) * NC) * 8);
+          for (int kx = 0; kx < 4; ++kx) {
+            // kx = 0: odd pixels at u - 1; 1: even at u; 2: odd at u; 3: even at u + 1
+            const uint32_t av = a0 + (uint32_t)(((kx & 1) ? 0 : (SLAB_BYTES >> 4)) + (HALO + (kx == 0 ? -1 : (kx == 3 ? 1 : 0))) * 8);
+            const uint32_t bv = b_base + (uint32_t)((((kx * 2 + par) * 2 + (o_lo - of + e)) * NC) * 8);
 #pragma unroll
-                for (int ks = 0; ks < 4; ++ks) umma_bf16_lo(dcol, av + (uint32_t)(2 * ks), bv + (uint32_t)(2 * ks), hi, idesc, true);
-              }
-            };
-            const int of = (r - 1) >> 1;                             // (arithmetic shift: r = 0 -> -1)
-            const int o_lo = of > y0 ? of : y0, o_hi = of + 1 < y1 - 1 ? of + 1 : y1 - 1;      // inclusive
-            if (o_lo <= o_hi) {
-              const int cnt = o_hi - o_lo + 1, slot = o_lo & 7;
-              const int n1 = cnt < 8 - slot ? cnt : 8 - slot;
-              issue_run(o_lo - of, n1, slot);
-              if (cnt > n1) issue_run(o_lo - of + n1, cnt - n1, 0);
-            }
-            umma_commit(empty_bar(s));
+            for (int ks = 0; ks < 4; ++ks) umma_bf16_lo(dcol, av + (uint32_t)(2 * ks), bv + (uint32_t)(2 * ks), hi, idesc, true);
           }
-          __syncwarp();
-          if (++s == S) s = 0;
-          ++n;
-        }
-        if (leader) umma_commit(rowdone_bar(k));
-        __syncwarp();
-      }
-    }
+        });
+    });
   } else if (warp >= EPI0 && warp < XF0) {
     // ===================================== epilogue: warp = (lane quarter q, channel half h) =====================================
     const int q = warp & 3;
@@ -221,111 +107,43 @@ down_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     const int h = ew >> 2;
     const int row = q * 32 + lane;
     const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-    uint8_t* buf = gen + (sOut - base) + ew * OUT_B;
-    float2 ws = make_float2(0.f, 0.f), wq = make_float2(0.f, 0.f);
+    uint8_t* buf = sm.scratch(ew, OUT_B);
+    Stats stats;
     const bool do_stats = p.stats != nullptr;
-    int stat_img = -1;
-    auto flush_stats = [&]() {
-      if (stat_img >= 0) {
-        double* st = p.stats + ((size_t)stat_img * p.Co_total + p.co_off + 32 * h + lane) * 2;
-        atomicAdd(st, f2sum_value(ws));
-        atomicAdd(st + 1, f2sum_value(wq));
-      }
-      ws = make_float2(0.f, 0.f); wq = make_float2(0.f, 0.f);
-    };
-    uint32_t zero32[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) zero32[i] = 0u;
     uint32_t k = 0;
     bool stored = false;
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      const bool valid = seg * BM + row < Wo;
-      if (do_stats && img != stat_img) { flush_stats(); stat_img = img; }
-      for (int r = 2 * y0 - 1; r < 2 * y1 + 1; ++r, ++k) {
-        mbar_wait(rowdone_bar(k), (k / NBAR) & 1);
+    for (Walk pc = pieces; pc.next();) {
+      const bool valid = pc.seg * BM + row < Wo;
+      if (do_stats && pc.img != stats.img) { stats.flush<32>(p.stats, p.Co_total, p.co_off + 32 * h, lane); stats.img = pc.img; }
+      for (int r = pc.r0; r < pc.r1; ++r, ++k) {
+        bars.wait_rowdone(k);
         // an even input row r completes the output row r / 2 - 1 (its last tap is ky = 3)
         const int o = (r >> 1) - 1;
-        const bool okr = !(r & 1) && o >= y0 && o < y1;              // (warp-uniform)
+        const bool okr = !(r & 1) && o >= pc.y0 && o < pc.y1;        // (warp-uniform)
         float v[32];
         if (okr) {
           tc_fence_after();
           const uint32_t ta = tmem_base + lane_addr + (uint32_t)((o & 7) * NC + 32 * h);
           tmem_ld32(ta, v);
           tmem_ld_wait();
-          tmem_st32(ta, zero32);
+          tmem_zero<32>(ta);
           tmem_st_wait();
           tc_fence_before();
         }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(drained_bar(k));
+        arrive_drained(bars, k, lane);
         if (!okr) continue;
 #pragma unroll
         for (int c = 0; c < 32; ++c) v[c] += sbias[32 * h + c];
-        if (stored) {
-          if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-          __syncwarp();
-        }
-        if (do_stats) {
-          float* sc = reinterpret_cast<float*>(buf);
-#pragma unroll
-          for (int hh = 0; hh < 2; ++hh) {
-#pragma unroll
-            for (int c = 0; c < 16; ++c) sc[c * 32 + (lane ^ c)] = valid ? v[16 * hh + c] : 0.f;
-            __syncwarp();
-            const int c = lane & 15, r0 = lane & 16;
-            float cs0 = 0.f, cs1 = 0.f, q0 = 0.f, q1 = 0.f;
-#pragma unroll
-            for (int j = 0; j < 16; j += 2) {
-              const float x0 = sc[c * 32 + ((r0 + j) ^ c)], x1 = sc[c * 32 + ((r0 + j + 1) ^ c)];
-              cs0 += x0; cs1 += x1;
-              q0 = fmaf(x0, x0, q0); q1 = fmaf(x1, x1, q1);
-            }
-            float cs = cs0 + cs1, qs = q0 + q1;
-            const float cs_o = __shfl_xor_sync(0xffffffffu, cs, 16), qs_o = __shfl_xor_sync(0xffffffffu, qs, 16);
-            cs = r0 ? cs_o + cs : cs + cs_o;
-            qs = r0 ? qs_o + qs : qs + qs_o;
-            if ((lane >> 4) == hh) { f2sum_add(ws, cs); f2sum_add(wq, qs); }
-            __syncwarp();
-          }
-        }
-        uint4 pk[4];
-#pragma unroll
-        for (int c8 = 0; c8 < 4; ++c8) {
-          float o8[8];
-#pragma unroll
-          for (int c = 0; c < 8; ++c) o8[c] = v[c8 * 8 + c];
-          pk[c8] = pack8(o8);
-        }
-        const int rot = (lane >> 1) & 3;
-#pragma unroll
-        for (int bit = 1; bit < 4; bit <<= 1) {
-          const bool sw = (rot & bit) != 0;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            if (j & bit) continue;
-            const uint4 a = pk[j], c2 = pk[j | bit];
-            pk[j] = sw ? c2 : a;
-            pk[j | bit] = sw ? a : c2;
-          }
-        }
-#pragma unroll
-        for (int j = 0; j < 4; ++j) *reinterpret_cast<uint4*>(buf + lane * 64 + (j ^ rot) * 16) = pk[j];
-        fence_proxy_async();
-        __syncwarp();
-        if (lane == 0) {
-          tma_store_4d(&mapY, smem_u32(buf), p.co_off + 32 * h, seg * BM + q * 32, o, img);
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-        }
+        if (stored) wait_store_read<0>(lane);
+        if (do_stats) piece_stats<32>(reinterpret_cast<float*>(buf), v, valid, lane, stats);
+        store_piece_bf16<32>(buf, v, lane, &mapY, p.co_off + 32 * h, pc.seg * BM + q * 32, o, pc.img);
         stored = true;
       }
     }
-    if (do_stats) flush_stats();
+    if (do_stats) stats.flush<32>(p.stats, p.Co_total, p.co_off + 32 * h, lane);
     if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   } else if (warp >= XF0) {
-    // ===================================== transform: x slabs -> ReLU(IN(x)), in place (out7_ring.cu) =====================================
+    // ===================================== transform: x slabs -> ReLU(IN(x)), in place =====================================
     const int xt = tid - 32 * XF0;                     // 0..127
     const int pchunk = xt & 7, rbase = xt >> 3;
     const int lchunk = pchunk ^ (rbase & 7);
@@ -333,29 +151,18 @@ down_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     const bool xform = p.in_stats != nullptr;
     float sc[8], sh[8];
     int cur_img = -1;
-    int s = 0;
-    uint32_t n = 0;
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      if (xform && img != cur_img) {
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          const double* st = p.in_stats + ((size_t)img * p.Cs_total + p.cs_off + lchunk * 8 + e) * 2;
-          float mean, rstd;
-          finalize_stats(st[0], st[1], inv_hw, mean, rstd);
-          sc[e] = rstd;
-          sh[e] = 0.f - mean * rstd;
-        }
-        cur_img = img;
+    SlabRing ring(bars.S);
+    for (Walk pc = pieces; pc.next();) {
+      if (xform && pc.img != cur_img) {
+        load_scale_shift(p.in_stats, pc.img, p.Cs_total, p.cs_off, lchunk, inv_hw, sc, sh);
+        cur_img = pc.img;
       }
-      const int r_lo = 2 * y0 - 1 < 0 ? 0 : 2 * y0 - 1, r_hi = 2 * y1 + 1 > p.H ? p.H : 2 * y1 + 1;
-      const int j0 = seg * BM - HALO;                  // pixel-pair index of slab pixel 0
-      for (int r = r_lo; r < r_hi; ++r, ++n) {
-        mbar_wait(full_bar(s), (n / S) & 1);
+      const int r_lo = pc.r0 < 0 ? 0 : pc.r0, r_hi = pc.r1 > p.H ? p.H : pc.r1;
+      const int j0 = pc.seg * BM - HALO;               // pixel-pair index of slab pixel 0
+      for (int r = r_lo; r < r_hi; ++r) {
+        mbar_wait(bars.full(ring.s), ring.parity());
         if (xform) {
-          uint8_t* fs = gen + (sA - base) + s * STAGE + rbase * 128 + pchunk * 16;
+          uint8_t* fs = sm.stage_ptr(ring.s, SH.stage_bytes) + rbase * 128 + pchunk * 16;
           // (loads of a slab batched ahead of the arithmetic, no branches: rows 128..135 exist only for rbase < 8 -- those threads'
           // ninth chunk -- and out-of-plane pixels are forced to 0 by a select)
           const __nv_bfloat162 zero2 = __floats2bfloat162_rn(0.f, 0.f);
@@ -388,17 +195,12 @@ down_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
           fence_proxy_async();
         }
         __syncwarp();
-        if (lane == 0) mbar_arrive(xf_bar(s));
-        if (++s == S) s = 0;
+        if (lane == 0) mbar_arrive(bars.xf(ring.s));
+        ring.advance();
       }
     }
   }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-  }
+  teardown(warp, tmem_base);
 }
 
 }  // namespace
@@ -418,8 +220,7 @@ extern "C" int msg_down_ring(const msg_down_ring_desc* d, const void* x, const d
   MSG_REQUIRE(in_stats == nullptr || (d->cs_off >= 0 && d->cs_off + 64 <= d->Cs_total), MSG_ERR_SHAPE, "down_ring: stats layout");
   MSG_REQUIRE((((uintptr_t)x | (uintptr_t)w_stacks | (uintptr_t)y) & 15) == 0, MSG_ERR_ALIGN, "down_ring: operands must be 16-byte aligned");
   MSG_REQUIRE(!(d->flags & MSG_CONV_STATS) || stats != nullptr, MSG_ERR_SHAPE, "down_ring: stats buffer missing");
-  EncodeTiledFn enc = get_encode();
-  MSG_REQUIRE(enc != nullptr, MSG_ERR_CUDA, "down_ring: cuTensorMapEncodeTiled unavailable");
+  MSG_REQUIRE(get_encode() != nullptr, MSG_ERR_CUDA, "down_ring: cuTensorMapEncodeTiled unavailable");
   const int G = d->Cout / 64, Ho = d->H / 2, Wo = d->W / 2;
 
   DnParams p;
@@ -433,55 +234,22 @@ extern "C" int msg_down_ring(const msg_down_ring_desc* d, const void* x, const d
   CUtensorMap mapA, mapB, mapY;
   {
     // the input row as [W/2][2] pixels: coordinate 1 selects the even or the odd pixels, coordinate 2 the pixel pair
-    cuuint64_t dims[5] = {64, 2, (cuuint64_t)Wo, (cuuint64_t)d->H, (cuuint64_t)d->N};
-    cuuint64_t strides[4] = {(cuuint64_t)d->Ci_total * 2, (cuuint64_t)2 * d->Ci_total * 2, (cuuint64_t)d->W * d->Ci_total * 2,
-                             (cuuint64_t)d->H * d->W * d->Ci_total * 2};
-    cuuint32_t box[5] = {64, 1, (cuuint32_t)SLAB_PX, 1, 1};
-    cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    void* b0 = (void*)((const __nv_bfloat16*)x + d->ci_off);
-    CUresult r = enc(&mapA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, b0, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const cuuint64_t dims[5] = {64, 2, (cuuint64_t)Wo, (cuuint64_t)d->H, (cuuint64_t)d->N};
+    const cuuint64_t strides[4] = {(cuuint64_t)d->Ci_total * 2, (cuuint64_t)2 * d->Ci_total * 2, (cuuint64_t)d->W * d->Ci_total * 2,
+                                   (cuuint64_t)d->H * d->W * d->Ci_total * 2};
+    const cuuint32_t box[5] = {64, 1, (cuuint32_t)SLAB_PX, 1, 1};
+    const CUresult r = encode(&mapA, 5, (const __nv_bfloat16*)x + d->ci_off, dims, strides, box, true);
     MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "down_ring: cuTensorMapEncodeTiled(x) failed with %d", (int)r);
   }
-  {
-    cuuint64_t dims[2] = {64, (cuuint64_t)G * W_ROWS};
-    cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, 64};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = enc(&mapB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)w_stacks, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "down_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
-  }
-  {
-    cuuint64_t dims[4] = {(cuuint64_t)d->Co_total, (cuuint64_t)Wo, (cuuint64_t)Ho, (cuuint64_t)d->N};
-    cuuint64_t strides[3] = {(cuuint64_t)d->Co_total * 2, (cuuint64_t)Wo * d->Co_total * 2, (cuuint64_t)Ho * Wo * d->Co_total * 2};
-    cuuint32_t box[4] = {32, 32, 1, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = enc(&mapY, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "down_ring: cuTensorMapEncodeTiled(y) failed with %d", (int)r);
-  }
-  const int fixed = W_BYTES + NC * 4 + 128 + NEW * 2048 + 8 + 8 * (3 * 8 + 1 + 2 * NBAR) + 64 + 1024;
-  int stages = (227 * 1024 - fixed) / STAGE;
-  if (stages > 8) stages = 8;
-  MSG_REQUIRE(stages >= 2, MSG_ERR_UNSUPPORTED, "down_ring: the slab ring does not fit shared memory");
-  p.stages = stages;
-  const size_t smem = (size_t)stages * STAGE + fixed;
-  static DeviceOnce attr_set;
-  if (attr_set.needed()) {
-    cudaError_t e = cudaFuncSetAttribute(down_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    MSG_REQUIRE(e == cudaSuccess, MSG_ERR_CUDA, "down_ring: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    attr_set.done();
-  }
-  const int sms = sm_count();
-  const long long grid_ll = p.total_rows / 4;
-  const int grid = grid_ll < 1 ? 1 : (grid_ll > sms ? sms : (int)grid_ll);
+  CUresult r = encode_weights(&mapB, w_stacks, (long long)G * W_ROWS);
+  MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "down_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
+  r = encode_store(&mapY, y, d->Co_total, Wo, Ho, d->N, 32, 1);
+  MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "down_ring: cuTensorMapEncodeTiled(y) failed with %d", (int)r);
   for (int g = 0; g < G; ++g) {
     p.co_off = d->co_off + 64 * g;
     p.bias = bias ? bias + 64 * g : nullptr;
     p.w_row0 = g * W_ROWS;
-    down_ring_kernel<<<grid, NTHREADS, smem, st>>>(mapA, mapB, mapY, p);
-    const int rc = check_launch("down_ring_kernel");
+    const int rc = launch<down_ring_kernel>("down_ring_kernel", dn_shape(), NTHREADS, p.total_rows, 4, p, mapA, mapB, mapY, st);
     if (rc) return rc;
   }
   return MSG_OK;

@@ -1,5 +1,6 @@
 // MultiScaleBlock branches (enhanced_generator.py:52-71: 1x1 | 3x3 dil 1 | 3x3 dil 2 | 3x3 dil 4, C -> 4 x C/4 channels) as a ROW
 // RING of tensor-memory accumulators (sm_100a, bf16 operands, fp32 accumulate), C = 64 (one pass) and C = 128 (three passes).
+// The mechanics shared with the other ring kernels are in ring.cuh.
 //
 // The per-tap row-slab kernel (conv_slab.cu) issues 25 MMAs of N = C/4 per K step and output row; a tcgen05.mma with M = 128
 // costs ~45 cycles however small N is, so that kernel runs at 15-25 % of the tensor pipe, and it loads seven input row slabs per
@@ -9,8 +10,7 @@
 //     whose accumulators sit in ADJACENT tensor-memory columns -- every branch keeps one ring of C/4-column row accumulators per
 //     residue class (row mod d) -- so they are ONE MMA of N = 3C/4 over a weight stack [ky = 2 | ky = 1 | ky = 0];
 //   * the row finished by input row r (branch 1: r, branch 2: r - 1, branch 3: r - 2, branch 4: r - 4) is drained by that
-//     branch's epilogue group (bias, IN statistics, bf16, per-warp TMA store of its channel slice of its own output row) and its
-//     slot is ZEROED with tcgen05.st, so every MMA accumulates and the first touch of a slot needs no special case.
+//     branch's epilogue group (bias, IN statistics, bf16, per-warp TMA store of its channel slice of its own output row).
 // C = 128 (32 columns per row accumulator) does not fit 512 tensor-memory columns in one go: branches 1 + 2, branch 3 and
 // branch 4 run as three launches (passes), each with its own resident weight stacks.
 // The schedule is stated (and run on tensors) in slab.py: RING_PASSES / ring_col / ring_row_mmas; this file restates it.
@@ -21,22 +21,13 @@
 //               runs change every row), so ONE issuer ran the MMAs at ~85 cycles each; the branches of a pass are spread over up
 //               to three issuers (disjoint column ranges: the streams need no ordering)
 //   warps 4-    epilogue: one group of four warps per branch of the pass (thread = strip pixel = TMEM lane)
-#include <cuda.h>
+#include "ring.cuh"
 
 #include <type_traits>
 
-#include "common.cuh"
-#include "tcgen05.cuh"
-
 namespace msg {
 namespace {
-using namespace tc;
-
-constexpr int BM = 128;                 // strip width (output pixels)
-constexpr int HALO = 4;
-constexpr int SLAB_PX = BM + 2 * HALO;  // 136
-constexpr int SLAB_BYTES = SLAB_PX * 128;          // one 64-channel block of a row slab: 17408 = 17 * 1024
-constexpr int EPI0 = 4;                 // first epilogue warp (warp & 3 = TMEM lane quarter)
+using namespace ring;
 
 // ---- pass tables (slab.py: RING_PASSES): branch ids and ring lengths of pass PS at width C
 __host__ __device__ constexpr int ring_nb(int C, int ps) { return C == 64 ? 4 : (ps == 0 ? 2 : 1); }
@@ -50,7 +41,6 @@ __host__ __device__ constexpr int ring_slots(int C, int ps, int i) {
   return b == 0 ? 4 : (b == 1 ? 6 : (b == 2 ? 8 : 4));          // pass 0: 128 + 2 x 192 (two sets) | pass 1: 512 | pass 2: 512
 }
 __host__ __device__ constexpr int ring_lead(int C, int ps) { return C == 64 ? 3 : (ps == 0 ? 4 : 8); }
-constexpr int NBAR = 8;                 // row-done / drained barrier rings (>= the largest LEAD)
 __host__ __device__ constexpr int ring_dil(int b) { return b == 0 ? 1 : (1 << (b - 1)); }
 // a branch whose accumulators are DUPLICATED by input-row parity (C = 128 pass 0, the dilation-1 3x3): even and odd input rows
 // accumulate into two separate rings, so two issuers share the branch without touching the same columns; the epilogue adds them
@@ -75,11 +65,14 @@ __host__ __device__ constexpr int ring_rows(int C, int ps) { return ring_wrow0(C
 __host__ __device__ constexpr int ring_issuer(int C, int ps, int i) { return C == 64 ? (i <= 1 ? 0 : i - 1) : (ps == 0 ? i : 0); }
 __host__ __device__ constexpr int ring_split(int C, int ps, int i) { return (C == 128 && (ps >= 1 || i == 1)) ? 2 : 1; }
 __host__ __device__ constexpr int ring_nissue(int C, int ps) { return C == 64 ? 3 : (ps == 0 ? 3 : 2); }
-// epilogue groups per branch (they alternate steps)
-#ifndef RING_EG128
-#define RING_EG128 1
-#endif
-__host__ __device__ constexpr int ring_eg(int C) { return C == 64 ? 1 : RING_EG128; }
+
+// shared memory of pass PS: weight stacks [KB][rows][128 B], slabs of KB 64-channel blocks, bias [C], and per epilogue warp
+// [16 ch][32 px] fp32 for the statistics and the staging of its piece, 32 pixels x C/4 channels (bf16).  C = 128: one 2 KB buffer
+// serves both in turn (it buys a slab stage); C = 64: statistics + two 1 KB staging buffers
+template <int C, int PS>
+__host__ __device__ constexpr Shape ring_shape() {
+  return Shape{C / 64 * ring_rows(C, PS) * 128, C / 64 * SLAB_BYTES, C, 4 * ring_nb(C, PS) * (C == 64 ? 4096 : 2048), 2};
+}
 
 struct RingParams {
   int N, H, W, Co_total, co_off;
@@ -98,221 +91,105 @@ __device__ __forceinline__ uint32_t ring_col(int y) {       // TMEM column of th
 }
 
 template <int C, int PS>
-__global__ void __launch_bounds__(32 * (EPI0 + 4 * ring_nb(C, PS) * ring_eg(C)), 1)
+__global__ void __launch_bounds__(32 * (EPI0 + 4 * ring_nb(C, PS)), 1)
 msb_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                 const __grid_constant__ CUtensorMap mapY, const RingParams p) {
   constexpr int Q = C / 4, KB = C / 64, NB = ring_nb(C, PS), NISSUE = ring_nissue(C, PS);
   constexpr int ROWS = ring_rows(C, PS);                  // weight rows per 64-channel block
-  constexpr int W_BYTES = KB * ROWS * 128;
-  constexpr int STAGE = KB * SLAB_BYTES;
-  constexpr int EG = ring_eg(C);                          // epilogue groups per branch
-  constexpr int NEW = 4 * NB * EG;                        // epilogue warps
-  // per-warp scratch: [16 ch][32 px] fp32 for the statistics and the staging of the warp's piece, 32 pixels x Q channels (bf16).
-  // C = 128: one 2 KB buffer serves both in turn (it buys a slab stage); C = 64: statistics + two 1 KB staging buffers
+  constexpr Shape SH = ring_shape<C, PS>();
+  constexpr int NEW = 4 * NB;                             // epilogue warps
   constexpr int NBUF = C == 64 ? 2 : 1;
   constexpr int OUT_B = C == 64 ? 4096 : 2048;
   constexpr int HV = ring_halo(C, PS);                    // input rows above / below a piece = the largest dilation of the pass
+  constexpr uint32_t LEAD = (uint32_t)ring_lead(C, PS);
+  using Walk = Pieces<1, HV>;
   extern __shared__ uint8_t smem_raw[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int S = p.stages;
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t sB = base;                               // weight stacks [KB][ROWS][128 B], SW128
-  const uint32_t sA = sB + W_BYTES;                       // slab ring
-  const uint32_t sBias = sA + S * STAGE;                  // bias [C]
-  const uint32_t sOut = (sBias + C * 4 + 127u) & ~127u;   // per-warp scratch [NEW][OUT_B]
-  const uint32_t sBar = (sOut + NEW * OUT_B + 7u) & ~7u;
-  float* sbias = reinterpret_cast<float*>(gen + (sBias - base));
-  auto full_bar = [&](int s) { return sBar + 8u * s; };
-  auto empty_bar = [&](int s) { return sBar + 8u * (S + s); };
-  const uint32_t wres_bar = sBar + 8u * (2 * S);
-  auto rowdone_bar = [&](uint32_t k) { return sBar + 8u * (2 * S + 1 + (k & (NBAR - 1))); };
-  auto drained_bar = [&](uint32_t k) { return sBar + 8u * (2 * S + 1 + NBAR + (k & (NBAR - 1))); };
-  constexpr uint32_t LEAD = (uint32_t)ring_lead(C, PS);
-  static_assert(LEAD <= NBAR, "barrier rings shorter than the lead");
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(gen + (sBar - base) + 8 * (2 * S + 1 + 2 * NBAR));
+  const Smem sm(smem_raw, SH, p.stages);
+  const Bars& bars = sm.b;
+  float* sbias = sm.bias();
 
   if (tid < C) sbias[tid] = p.bias ? p.bias[tid] : 0.f;
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < S; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), NISSUE); }
-      mbar_init(wres_bar, 1);
-      for (int k = 0; k < NBAR; ++k) { mbar_init(rowdone_bar(k), NISSUE); mbar_init(drained_bar(k), NEW); }
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  } else if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapB)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapY)) : "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  if (warp >= EPI0 && warp < EPI0 + 4) {  // every accumulator starts at zero: each MMA of the kernel accumulates
-    const uint32_t lane_addr = (uint32_t)((warp & 3) * 32) << 16;
-    uint32_t z[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) z[i] = 0u;
-    for (int c = 0; c < 512; c += 32) tmem_st32(tmem_base + lane_addr + (uint32_t)c, z);
-    tmem_st_wait();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-
-  // Work = the rows of all column strips laid end to end (strip = (image, 128-pixel segment), H rows each); CTA i takes the i-th
-  // equal share of that range, i.e. at most a few pieces of consecutive strips: every SM gets the same number of rows (whole-strip
-  // segments left 20 of 148 SMs idle at 16 x 512 x 512) and a piece re-reads only its 8 halo rows.
-  const long long g_lo = (long long)blockIdx.x * p.total_rows / gridDim.x, g_hi = (long long)(blockIdx.x + 1) * p.total_rows / gridDim.x;
-  auto item = [&](long long g, int& img, int& seg, int& y0, int& y1) {
-    const int strip = (int)(g / p.H);
-    y0 = (int)(g - (long long)strip * p.H);
-    const long long left = g_hi - g;
-    y1 = (long long)(p.H - y0) < left ? p.H : y0 + (int)left;
-    img = strip / p.segs;
-    seg = strip - img * p.segs;
-  };
+  const uint32_t tmem_base = prologue(sm, warp, lane, NISSUE, NEW, 0, &mapA, &mapB, &mapY);
+  const Walk pieces(p.total_rows, p.H, p.segs);
 
   if (warp == 0) {
-    // ===================================== TMA producer =====================================
-    if (lane == 0) {
-      mbar_expect_tx(wres_bar, (uint32_t)W_BYTES);
-      for (int r = 0; r < KB * ROWS; r += 64) tma_load_2d(sB + r * 128, &mapB, wres_bar, 0, p.w_row0 + r);
-      int s = 0;
-      uint32_t n = 0;                      // slabs issued
-      for (long long g = g_lo; g < g_hi;) {
-        int img, seg, y0, y1;
-        item(g, img, seg, y0, y1);
-        g += y1 - y0;
-        const int r_lo = y0 - HV < 0 ? 0 : y0 - HV, r_hi = y1 + HV > p.H ? p.H : y1 + HV;
-        for (int r = r_lo; r < r_hi; ++r, ++n) {
-          if (n >= (uint32_t)S) mbar_wait(empty_bar(s), ((n / S) - 1) & 1);
-          mbar_expect_tx(full_bar(s), (uint32_t)STAGE);
+    if (lane == 0)
+      producer(sm, pieces, p.H, &mapB, SH.w_bytes, p.w_row0, SH.stage_bytes, [&](const Walk& pc, int r, uint32_t dst, uint32_t bar) {
 #pragma unroll
-          for (int kb = 0; kb < KB; ++kb)
-            tma_load_4d(sA + s * STAGE + kb * SLAB_BYTES, &mapA, full_bar(s), kb * 64, seg * BM - HALO, r, img);
-          if (++s == S) s = 0;
-        }
-      }
-    }
+        for (int kb = 0; kb < KB; ++kb) tma_load_4d(dst + kb * SLAB_BYTES, &mapA, bar, kb * 64, pc.seg * BM - HALO, r, pc.img);
+      });
   } else if (warp < EPI0) {
-    // ===================================== MMA issuers =====================================
     const int me = warp - 1;
     if (me < NISSUE) {
-    const bool leader = elect_one();
-    const uint32_t hi = (uint32_t)(make_sw128_desc(0) >> 32);
-    const uint32_t idesc0 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BM >> 4) << 24);      // + N
-    const uint32_t b_base = sB >> 4;
-    int s = 0;
-    uint32_t n = 0, k = 0;                 // slabs consumed, global step count
-    mbar_wait(wres_bar, 0);
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      for (int r = y0 - HV; r < y1 + HV; ++r, ++k) {
-        // the epilogue must have drained (and zeroed) everything up to step k - LEAD: the slot this row first touches belonged to
-        // a row finished no later than that (ring_slots)
-        if (k >= LEAD) mbar_wait(drained_bar(k - LEAD), ((k - LEAD) / NBAR) & 1);
-        // a new piece maps its rows onto the slots afresh: everything of the previous piece must have been drained
-        if (r == y0 - HV && k > 0) mbar_wait(drained_bar(k - 1), ((k - 1) / NBAR) & 1);
-        if (r >= 0 && r < p.H) {
-          mbar_wait(full_bar(s), (n / S) & 1);
-          tc_fence_after();
-          if (leader) {
-            const uint32_t a0 = (sA + s * STAGE) >> 4;
-            // the branches of this issuer: compile-time loop, the others fold away
-            auto branch = [&](auto IC) {
-              constexpr int I = decltype(IC)::value;
-              constexpr int b = ring_branch(C, PS, I);
-              constexpr uint32_t wr0 = (uint32_t)ring_wrow0(C, PS, I);
-              if constexpr (b == 0) {
-                if (r >= y0 && r < y1) {       // the 1x1 conv, output row r
-                  const uint32_t dcol = tmem_base + ring_col<C, PS, I>(r);
-                  const uint32_t idesc = idesc0 | ((uint32_t)(Q >> 3) << 17);
+      const bool leader = elect_one();
+      const uint32_t hi = (uint32_t)(make_sw128_desc(0) >> 32);
+      const uint32_t b_base = sm.sB() >> 4;
+      issuer<LEAD, false>(bars, pieces, p.H, leader, [&](const Walk& pc, int r, int s) {
+        const uint32_t a0 = sm.sA(s, SH.stage_bytes) >> 4;
+        // the branches of this issuer: compile-time loop, the others fold away
+        auto branch = [&](auto IC) {
+          constexpr int I = decltype(IC)::value;
+          constexpr int b = ring_branch(C, PS, I);
+          constexpr uint32_t wr0 = (uint32_t)ring_wrow0(C, PS, I);
+          if constexpr (b == 0) {
+            if (r >= pc.y0 && r < pc.y1) {     // the 1x1 conv, output row r
+              const uint32_t dcol = tmem_base + ring_col<C, PS, I>(r);
+#pragma unroll
+              for (int kb = 0; kb < KB; ++kb)
+#pragma unroll
+                for (int ks = 0; ks < 4; ++ks)
+                  umma_bf16_lo(dcol, a0 + (uint32_t)(kb * (SLAB_BYTES >> 4) + HALO * 8 + 2 * ks),
+                               b_base + (uint32_t)((kb * ROWS + (int)wr0) * 8 + 2 * ks), hi, idesc_bf16(Q), true);
+            }
+          } else {
+            // entries e = 0, 1, 2 = output rows r - d, r, r + d (vertical taps ky = 2, 1, 0); those of this piece are an interval
+            // of entries whose slots in the residue class's ring are adjacent except where the ring wraps
+            constexpr int d = ring_dil(b);
+            constexpr int R = ring_slots(C, PS, I);
+            const uint32_t set = ring_dup(C, PS, I) > 1 ? (uint32_t)((r & 1) * ring_width(C, PS, I)) : 0u;
+            const int e_lo = r - d >= pc.y0 ? 0 : (r >= pc.y0 ? 1 : 2);          // r + d >= y0 holds for every row of the piece's halo
+            const int e_hi = r + d < pc.y1 ? 2 : (r < pc.y1 ? 1 : 0);            // r - d < y1 likewise
+            if (e_lo <= e_hi && r + d >= pc.y0 && r - d < pc.y1) {
+              const int ylo = r + (e_lo - 1) * d;                                // first output row (>= y0 >= 0)
+              const int cls = ylo % d;
+              runs(e_hi - e_lo + 1, (ylo / d) % R, R, [&](int e, int nrun, int idx) {
+                const uint32_t idesc = idesc_bf16(Q * nrun);
+                const uint32_t dcol = tmem_base + (uint32_t)(ring_base(C, PS, I) + (cls * R + idx) * Q) + set;
+#pragma unroll
+                for (int kx = 0; kx < 3; ++kx) {
+                  const uint32_t wrow = wr0 + (uint32_t)(kx * 3 * Q + Q * (e_lo + e));
+                  const uint32_t av = a0 + (uint32_t)((HALO + (kx - 1) * d) * 8);
 #pragma unroll
                   for (int kb = 0; kb < KB; ++kb)
 #pragma unroll
                     for (int ks = 0; ks < 4; ++ks)
-                      umma_bf16_lo(dcol, a0 + (uint32_t)(kb * (SLAB_BYTES >> 4) + HALO * 8 + 2 * ks),
-                                   b_base + (uint32_t)((kb * ROWS + (int)wr0) * 8 + 2 * ks), hi, idesc, true);
+                      umma_bf16_lo(dcol, av + (uint32_t)(kb * (SLAB_BYTES >> 4) + 2 * ks),
+                                   b_base + (uint32_t)(kb * ROWS * 8) + wrow * 8u + (uint32_t)(2 * ks), hi, idesc, true);
                 }
-              } else {
-                constexpr int d = ring_dil(b);
-                // entries e = 0, 1, 2 = output rows r - d, r, r + d (vertical taps ky = 2, 1, 0); those of this piece are an interval
-                // of entries whose slots in the residue class's ring are adjacent except where the ring wraps: one or two runs,
-                // found by arithmetic (no run table in local memory)
-                constexpr int R = ring_slots(C, PS, I);
-                const uint32_t set = ring_dup(C, PS, I) > 1 ? (uint32_t)((r & 1) * ring_width(C, PS, I)) : 0u;
-                auto issue_run = [&](int e, int nrun, int idx, int cls) {
-                  const uint32_t idesc = idesc0 | ((uint32_t)((Q * nrun) >> 3) << 17);
-                  const uint32_t dcol = tmem_base + (uint32_t)(ring_base(C, PS, I) + (cls * R + idx) * Q) + set;
-#pragma unroll
-                  for (int kx = 0; kx < 3; ++kx) {
-                    const uint32_t wrow = wr0 + (uint32_t)(kx * 3 * Q + Q * e);
-                    const uint32_t av = a0 + (uint32_t)((HALO + (kx - 1) * d) * 8);
-#pragma unroll
-                    for (int kb = 0; kb < KB; ++kb)
-#pragma unroll
-                      for (int ks = 0; ks < 4; ++ks)
-                        umma_bf16_lo(dcol, av + (uint32_t)(kb * (SLAB_BYTES >> 4) + 2 * ks),
-                                     b_base + (uint32_t)(kb * ROWS * 8) + wrow * 8u + (uint32_t)(2 * ks), hi, idesc, true);
-                  }
-                };
-                const int e_lo = r - d >= y0 ? 0 : (r >= y0 ? 1 : 2);                // r + d >= y0 holds for every row of the piece's halo
-                const int e_hi = r + d < y1 ? 2 : (r < y1 ? 1 : 0);                  // r - d < y1 likewise
-                if (e_lo <= e_hi && r + d >= y0 && r - d < y1) {
-                  const int ylo = r + (e_lo - 1) * d;                                // first output row (>= y0 >= 0)
-                  const int cnt = e_hi - e_lo + 1, idx = (ylo / d) % R, cls = ylo % d;
-                  const int n1 = cnt < R - idx ? cnt : R - idx;
-                  issue_run(e_lo, n1, idx, cls);
-                  if (cnt > n1) issue_run(e_lo + n1, cnt - n1, 0, cls);
-                }
-              }
-            };
-            auto mine = [&](int i) { return ring_issuer(C, PS, i) + (r & (ring_split(C, PS, i) - 1)) == me; };
-            if (mine(0)) branch(std::integral_constant<int, 0>{});
-            if constexpr (NB > 1) { if (mine(1)) branch(std::integral_constant<int, 1>{}); }
-            if constexpr (NB > 2) { if (mine(2)) branch(std::integral_constant<int, 2>{}); }
-            if constexpr (NB > 3) { if (mine(3)) branch(std::integral_constant<int, 3>{}); }
-            umma_commit(empty_bar(s));
+              });
+            }
           }
-          __syncwarp();
-          if (++s == S) s = 0;
-          ++n;
-        }
-        if (leader) umma_commit(rowdone_bar(k));     // arrives when every MMA issued so far has completed
-        __syncwarp();
-      }
-    }
+        };
+        auto mine = [&](int i) { return ring_issuer(C, PS, i) + (r & (ring_split(C, PS, i) - 1)) == me; };
+        if (mine(0)) branch(std::integral_constant<int, 0>{});
+        if constexpr (NB > 1) { if (mine(1)) branch(std::integral_constant<int, 1>{}); }
+        if constexpr (NB > 2) { if (mine(2)) branch(std::integral_constant<int, 2>{}); }
+        if constexpr (NB > 3) { if (mine(3)) branch(std::integral_constant<int, 3>{}); }
+      });
     }
   } else {
-    // ===================================== epilogue (EG groups of four warps per branch) =====================================
+    // ===================================== epilogue: four warps per branch =====================================
     const int q = warp & 3;
     const int ew = warp - EPI0;                       // epilogue warp index
-    const int grp = ew >> 2;
-    const int bi = grp / EG;                          // branch index inside the pass
-    const int gpar = grp % EG;                        // the group drains the steps k with k % EG == gpar
+    const int bi = ew >> 2;                           // branch index inside the pass
     const int b = ring_branch(C, PS, bi);
     const int lag = b == 0 ? 0 : (1 << (b - 1));      // input row r completes output row r - lag of branch b
     const int row = q * 32 + lane;                    // strip pixel = TMEM lane
     const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-    uint8_t* buf = gen + (sOut - base) + ew * OUT_B;
-    float2 ws = make_float2(0.f, 0.f), wq = make_float2(0.f, 0.f);     // lane l < Q: running sum / sum of squares of channel l
+    uint8_t* buf = sm.scratch(ew, OUT_B);
+    Stats stats;                                      // lane l < Q: channel l of the branch
     const bool do_stats = p.stats != nullptr;
-    int stat_img = -1;
-    auto flush_stats = [&]() {
-      if (stat_img >= 0 && lane < Q) {
-        double* st = p.stats + ((size_t)stat_img * p.Co_total + p.co_off + Q * b + lane) * 2;
-        atomicAdd(st, f2sum_value(ws));
-        atomicAdd(st + 1, f2sum_value(wq));
-      }
-      ws = make_float2(0.f, 0.f); wq = make_float2(0.f, 0.f);
-    };
     uint32_t col_dup = 0;                             // column distance to the second accumulator set of a duplicated branch
     auto col_of = [&](int y) -> uint32_t {            // (bi is warp-uniform; the table folds per case)
       switch (bi) {
@@ -325,155 +202,60 @@ msb_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
     };
     if constexpr (NB > 1) { if (bi == 1 && ring_dup(C, PS, 1) > 1) col_dup = (uint32_t)ring_width(C, PS, 1); }
     if (bi == 0 && ring_dup(C, PS, 0) > 1) col_dup = (uint32_t)ring_width(C, PS, 0);
-    uint32_t zeroq[Q];
-#pragma unroll
-    for (int i = 0; i < Q; ++i) zeroq[i] = 0u;
     uint32_t k = 0;                        // steps
     uint32_t nst = 0;                      // pieces stored by this warp
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      const int xcol = seg * BM + row;
-      const bool valid = xcol < p.W;
-      if (do_stats && img != stat_img) { flush_stats(); stat_img = img; }
-      for (int r = y0 - HV; r < y1 + HV; ++r, ++k) {
+    for (Walk pc = pieces; pc.next();) {
+      const bool valid = pc.seg * BM + row < p.W;
+      if (do_stats && pc.img != stats.img) { stats.flush<Q>(p.stats, p.Co_total, p.co_off + Q * b, lane); stats.img = pc.img; }
+      for (int r = pc.r0; r < pc.r1; ++r, ++k) {
         const int y = r - lag;                                       // the row this input row completed for this branch
         // every warp follows every step (also those that finish nothing for it): a warp that ran ahead would arrive on a
         // drained barrier whose previous phase is still open
-        mbar_wait(rowdone_bar(k), (k / NBAR) & 1);
-        if (y >= y0 && y < y1 && (EG == 1 || (int)(k % EG) == gpar)) {      // (warp-uniform)
+        bars.wait_rowdone(k);
+        if (y >= pc.y0 && y < pc.y1) {                               // (warp-uniform)
           tc_fence_after();
           const uint32_t taddr = tmem_base + lane_addr + col_of(y);
           float v[Q];
-          if constexpr (Q == 16) tmem_ld16(taddr, v); else tmem_ld32(taddr, v);
+          tmem_ld_n(taddr, v);
           if (col_dup) {                                             // (warp-uniform) even-row set + odd-row set
             float v2[Q];
-            if constexpr (Q == 16) tmem_ld16(taddr + col_dup, v2); else tmem_ld32(taddr + col_dup, v2);
+            tmem_ld_n(taddr + col_dup, v2);
             tmem_ld_wait();
 #pragma unroll
             for (int c = 0; c < Q; ++c) v[c] += v2[c];
-            if constexpr (Q == 16) tmem_st16(taddr + col_dup, zeroq); else tmem_st32(taddr + col_dup, zeroq);
+            tmem_zero<Q>(taddr + col_dup);
           } else {
             tmem_ld_wait();
           }
-          if constexpr (Q == 16) tmem_st16(taddr, zeroq); else tmem_st32(taddr, zeroq);      // the slot is free for the row that wraps onto it
+          tmem_zero<Q>(taddr);
           tmem_st_wait();
           tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(drained_bar(k));           // handed back before anything else: the issuers wait on this
+          arrive_drained(bars, k, lane);
 #pragma unroll
           for (int c = 0; c < Q; ++c) v[c] += sbias[Q * b + c];
           uint8_t* stg = NBUF == 2 ? buf + 2048 + (nst & 1) * 1024 : buf;
-          if (nst >= (uint32_t)NBUF) {                               // the store issued NBUF pieces ago has read its buffer
-            if (lane == 0) {
-              if constexpr (NBUF == 2) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-              else asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            }
-            __syncwarp();
-          }
-          if (do_stats) {
-            // per-channel sums over the warp's 32 pixels: 16 channels at a time through buf as [16 ch][32 px] fp32 (pixel index
-            // XOR channel: conflict-free both ways); lane (c, half) sums 16 pixels of channel c in a fixed order on two chains,
-            // one shuffle joins the halves; lane l accumulates channel l
-            float* sc = reinterpret_cast<float*>(buf);
-#pragma unroll
-            for (int h = 0; h < Q / 16; ++h) {
-#pragma unroll
-              for (int c = 0; c < 16; ++c) sc[c * 32 + (lane ^ c)] = valid ? v[16 * h + c] : 0.f;
-              __syncwarp();
-              const int c = lane & 15, r0 = lane & 16;
-              float cs0 = 0.f, cs1 = 0.f, q0 = 0.f, q1 = 0.f;
-#pragma unroll
-              for (int j = 0; j < 16; j += 2) {
-                const float x0 = sc[c * 32 + ((r0 + j) ^ c)], x1 = sc[c * 32 + ((r0 + j + 1) ^ c)];
-                cs0 += x0; cs1 += x1;
-                q0 = fmaf(x0, x0, q0); q1 = fmaf(x1, x1, q1);
-              }
-              float cs = cs0 + cs1, qs = q0 + q1;
-              const float cs_o = __shfl_xor_sync(0xffffffffu, cs, 16), qs_o = __shfl_xor_sync(0xffffffffu, qs, 16);
-              cs = r0 ? cs_o + cs : cs + cs_o;                       // pixels 0-15 first on both halves: the same bits
-              qs = r0 ? qs_o + qs : qs + qs_o;
-              if ((lane >> 4) == h) { f2sum_add(ws, cs); f2sum_add(wq, qs); }
-              __syncwarp();
-            }
-          }
-          {
-            // the warp's [32 pixels x Q channels] piece into its staging buffer, then ONE TMA store (the tensor map clips pixels beyond the
-            // plane).  Per-thread global stores -- 32 scattered sectors per warp instruction, each output line assembled from four
-            // branches at four different times -- held the whole kernel back (profiles/r2_msb_ring.md).
-            // The 16-byte chunk a lane writes at step j is rotated by the lane, so the eight lanes of a store phase cover all 32
-            // banks: rows are Q * 2 = 32 / 64 bytes, dense -- the TMA store reads them un-swizzled.
-            uint4 pk[Q / 8];
-#pragma unroll
-            for (int c8 = 0; c8 < Q / 8; ++c8) {
-              float o8[8];
-#pragma unroll
-              for (int c = 0; c < 8; ++c) o8[c] = v[c8 * 8 + c];
-              pk[c8] = pack8(o8);
-            }
-            const int rot = Q == 16 ? ((lane >> 2) & 1) : ((lane >> 1) & 3);
-#pragma unroll
-            for (int bit = 1; bit < Q / 8; bit <<= 1) {
-              const bool sw = (rot & bit) != 0;
-#pragma unroll
-              for (int j = 0; j < Q / 8; ++j) {
-                if (j & bit) continue;
-                const uint4 a = pk[j], c2 = pk[j | bit];
-                pk[j] = sw ? c2 : a;
-                pk[j | bit] = sw ? a : c2;
-              }
-            }
-#pragma unroll
-            for (int j = 0; j < Q / 8; ++j) *reinterpret_cast<uint4*>(stg + lane * (Q * 2) + (j ^ rot) * 16) = pk[j];
-            fence_proxy_async();
-            __syncwarp();
-            if (lane == 0) {
-              tma_store_4d(&mapY, smem_u32(stg), p.co_off + Q * b, seg * BM + q * 32, y, img);
-              asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            }
-            ++nst;
-          }
+          if (nst >= (uint32_t)NBUF) wait_store_read<NBUF - 1>(lane);   // the store issued NBUF pieces ago has read its buffer
+          if (do_stats) piece_stats<Q>(reinterpret_cast<float*>(buf), v, valid, lane, stats);
+          store_piece_bf16<Q>(stg, v, lane, &mapY, p.co_off + Q * b, pc.seg * BM + q * 32, y, pc.img);
+          ++nst;
         } else {
-          if (lane == 0) mbar_arrive(drained_bar(k));           // nothing for this group at this step
+          if (lane == 0) mbar_arrive(bars.drained(k));           // nothing for this group at this step
         }
       }
     }
-    if (do_stats) flush_stats();
+    if (do_stats) stats.flush<Q>(p.stats, p.Co_total, p.co_off + Q * b, lane);
     if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-  }
+  teardown(warp, tmem_base);
 }
 
 template <int C, int PS>
-int launch_pass(const msg_msb_ring_desc* d, const CUtensorMap& mapA, const CUtensorMap& mapB, const CUtensorMap& mapY, RingParams p,
-                int w_row0, cudaStream_t st) {
-  constexpr int KB = C / 64, NB = ring_nb(C, PS), NEW = 4 * NB * ring_eg(C);
-  constexpr int W_BYTES = KB * ring_rows(C, PS) * 128, STAGE = KB * SLAB_BYTES;
-  const int fixed = W_BYTES + C * 4 + 128 + NEW * (C == 64 ? 4096 : 2048) + 8 + 384 + 1024;
-  int stages = (227 * 1024 - fixed) / STAGE;
-  if (stages > 8) stages = 8;
-  MSG_REQUIRE(stages >= 2, MSG_ERR_UNSUPPORTED, "msb_ring: the slab ring does not fit shared memory (C=%d pass %d)", C, PS);
-  p.stages = stages;
+int launch_pass(const CUtensorMap& mapA, const CUtensorMap& mapB, const CUtensorMap& mapY, RingParams p, int w_row0, cudaStream_t st) {
+  static_assert(ring_shape<C, PS>().stages() >= 2, "msb_ring: the slab ring of this pass does not fit shared memory");
   p.w_row0 = w_row0;
-  const size_t smem = (size_t)stages * STAGE + fixed;
-  static DeviceOnce attr_set;
-  if (attr_set.needed()) {
-    cudaError_t e = cudaFuncSetAttribute(msb_ring_kernel<C, PS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    MSG_REQUIRE(e == cudaSuccess, MSG_ERR_CUDA, "msb_ring: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    attr_set.done();
-  }
-  const int sms = sm_count();
-  const long long grid_ll = p.total_rows / 8;       // at least 8 rows per CTA (each piece re-reads 8 halo rows)
-  const int grid = grid_ll < 1 ? 1 : (grid_ll > sms ? sms : (int)grid_ll);
-  (void)d;
-  msb_ring_kernel<C, PS><<<grid, 32 * (EPI0 + NEW), smem, st>>>(mapA, mapB, mapY, p);
-  return check_launch("msb_ring_kernel");
+  // at least 8 rows per CTA (each piece re-reads 8 halo rows)
+  return launch<msb_ring_kernel<C, PS>>("msb_ring_kernel", ring_shape<C, PS>(), 32 * (EPI0 + 4 * ring_nb(C, PS)), p.total_rows, 8, p,
+                                        mapA, mapB, mapY, st);
 }
 
 int msb_ring_impl(const msg_msb_ring_desc* d, int C, const void* x, const void* w_stacks, const float* bias, void* y, double* stats,
@@ -486,8 +268,7 @@ int msb_ring_impl(const msg_msb_ring_desc* d, int C, const void* x, const void* 
   MSG_REQUIRE((d->Co_total & 7) == 0 && (d->co_off & 7) == 0 && d->co_off + C <= d->Co_total, MSG_ERR_SHAPE, "msb_ring: output channel layout");
   MSG_REQUIRE((((uintptr_t)x | (uintptr_t)w_stacks | (uintptr_t)y) & 15) == 0, MSG_ERR_ALIGN, "msb_ring: operands must be 16-byte aligned");
   MSG_REQUIRE(!(d->flags & MSG_CONV_STATS) || stats != nullptr, MSG_ERR_SHAPE, "msb_ring: stats buffer missing");
-  EncodeTiledFn enc = get_encode();
-  MSG_REQUIRE(enc != nullptr, MSG_ERR_CUDA, "msb_ring: cuTensorMapEncodeTiled unavailable");
+  MSG_REQUIRE(get_encode() != nullptr, MSG_ERR_CUDA, "msb_ring: cuTensorMapEncodeTiled unavailable");
 
   RingParams p;
   p.N = d->N; p.H = d->H; p.W = d->W; p.Co_total = d->Co_total; p.co_off = d->co_off;
@@ -495,48 +276,26 @@ int msb_ring_impl(const msg_msb_ring_desc* d, int C, const void* x, const void* 
   p.segs = (d->W + BM - 1) / BM;
   p.total_rows = (long long)d->N * p.segs * d->H;
   MSG_REQUIRE(p.total_rows < (1LL << 40), MSG_ERR_SHAPE, "msb_ring: too many rows");
-  const int Q = C / 4, KB = C / 64;
+  const int KB = C / 64;
   int total_w_rows = 0;
   for (int ps = 0; ps < (C == 64 ? 1 : 3); ++ps) total_w_rows += KB * ring_rows(C, ps);
 
   CUtensorMap mapA, mapB, mapY;
-  {
-    cuuint64_t dims[4] = {(cuuint64_t)d->Co_total, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-    cuuint64_t strides[3] = {(cuuint64_t)d->Co_total * 2, (cuuint64_t)d->W * d->Co_total * 2, (cuuint64_t)d->H * d->W * d->Co_total * 2};
-    cuuint32_t box[4] = {(cuuint32_t)Q, 32, 1, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = enc(&mapY, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "msb_ring: cuTensorMapEncodeTiled(y) failed with %d", (int)r);
-  }
-  {
-    cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-    cuuint64_t strides[3] = {(cuuint64_t)d->Ci_total * 2, (cuuint64_t)d->W * d->Ci_total * 2, (cuuint64_t)d->H * d->W * d->Ci_total * 2};
-    cuuint32_t box[4] = {64, (cuuint32_t)SLAB_PX, 1, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    void* b0 = (void*)((const __nv_bfloat16*)x + d->ci_off);
-    CUresult r = enc(&mapA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, b0, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "msb_ring: cuTensorMapEncodeTiled(x) failed with %d", (int)r);
-  }
-  {
-    cuuint64_t dims[2] = {64, (cuuint64_t)total_w_rows};
-    cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, 64};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = enc(&mapB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)w_stacks, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "msb_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
-  }
-  if (C == 64) return launch_pass<64, 0>(d, mapA, mapB, mapY, p, 0, st);
+  CUresult r = encode_store(&mapY, y, d->Co_total, d->W, d->H, d->N, C / 4, 1);
+  MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "msb_ring: cuTensorMapEncodeTiled(y) failed with %d", (int)r);
+  r = encode_slab(&mapA, (const __nv_bfloat16*)x + d->ci_off, C, d->Ci_total, d->W, d->H, d->N);
+  MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "msb_ring: cuTensorMapEncodeTiled(x) failed with %d", (int)r);
+  r = encode_weights(&mapB, w_stacks, total_w_rows);
+  MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "msb_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
+  if (C == 64) return launch_pass<64, 0>(mapA, mapB, mapY, p, 0, st);
   int row0 = 0;
-  int rc = launch_pass<128, 0>(d, mapA, mapB, mapY, p, row0, st);
+  int rc = launch_pass<128, 0>(mapA, mapB, mapY, p, row0, st);
   if (rc) return rc;
   row0 += KB * ring_rows(128, 0);
-  rc = launch_pass<128, 1>(d, mapA, mapB, mapY, p, row0, st);
+  rc = launch_pass<128, 1>(mapA, mapB, mapY, p, row0, st);
   if (rc) return rc;
   row0 += KB * ring_rows(128, 1);
-  return launch_pass<128, 2>(d, mapA, mapB, mapY, p, row0, st);
+  return launch_pass<128, 2>(mapA, mapB, mapY, p, row0, st);
 }
 
 }  // namespace

@@ -1,6 +1,7 @@
 // The generator's output layer (enhanced_generator.py:130-133: Conv2d(c, 3, 7, padding 3) + Tanh) fused with the InstanceNorm + ReLU
 // + residual of the MultiScaleBlock in front of it (enhanced_generator.py:78-84), as a ROW RING of tensor-memory accumulators
-// (sm_100a, bf16 operands, fp32 accumulate; c = 64) -- the third member of the msb_ring.cu / convt_ring.cu family.
+// (sm_100a, bf16 operands, fp32 accumulate; c = 64) -- the third member of the msb_ring.cu / convt_ring.cu family (shared mechanics in
+// ring.cuh).
 //
 //   a2 = a1 + ReLU(IN(f))        f: raw output of the block's 1x1 fusion conv with its plane statistics, a1: the block's input
 //   y  = tanh(conv7x7(a2) + b)   fp32 NCHW, 3 channels
@@ -23,31 +24,21 @@
 //   warp 1      MMA issuer (also allocates TMEM)
 //   warps 4-7   epilogue
 //   warps 8-11  transform
-#include <cuda.h>
-
-#include "common.cuh"
-#include "tcgen05.cuh"
+#include "ring.cuh"
 
 namespace msg {
 namespace {
-using namespace tc;
+using namespace ring;
 
-constexpr int BM = 128;
-constexpr int HALO = 4;                 // slab pixels left of the strip (3 needed)
-constexpr int SLAB_PX = BM + 2 * HALO;  // 136
-constexpr int SLAB_BYTES = SLAB_PX * 128;
-constexpr int STAGE = 2 * SLAB_BYTES;   // f (becomes the operand) + a1
 constexpr int NCOL = 16;                // columns per row accumulator (3 output channels padded)
 constexpr int SLOTS = 32;
 constexpr int HV = 3;                   // input rows above / below a piece
-constexpr int NBAR = 8;
 constexpr uint32_t LEAD = 6;            // a slot is touched again 26 steps after its row completed: any lead <= NBAR would do
 constexpr int W_ROWS = 7 * 128;         // per horizontal tap: 8 entries (7 vertical taps + one zero block) x 16 rows
-constexpr int W_BYTES = W_ROWS * 128;
 constexpr int NTHREADS = 32 * 12;
-#ifndef O7_PREFETCH
-#define O7_PREFETCH 0                   // input rows pulled into L2 ahead of the slab ring: 0 / 6 measured 0.3375 / 0.3328 ms (16 x 512^2): not kept
-#endif
+constexpr int XF0 = 8;
+// weights [7 kx][8 e][16 co][128 B] | stages [f slab | a1 slab]; full / empty / transformed per stage
+__host__ __device__ constexpr Shape o7_shape() { return Shape{W_ROWS * 128, 2 * SLAB_BYTES, 0, 0, 3}; }
 
 struct O7Params {
   int N, H, W;
@@ -63,225 +54,96 @@ struct O7Params {
 __global__ void __launch_bounds__(NTHREADS, 1)
 out7_ring_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_constant__ CUtensorMap mapR,
                  const __grid_constant__ CUtensorMap mapB, const O7Params p) {
+  constexpr Shape SH = o7_shape();
+  using Walk = Pieces<1, HV>;
   extern __shared__ uint8_t smem_raw[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int S = p.stages;
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t sB = base;                               // weight stacks [7 kx][8 e][16 co][128 B], SW128
-  const uint32_t sA = sB + W_BYTES;                       // stages: [f slab | a1 slab]
-  const uint32_t sBar = sA + S * STAGE;
-  auto full_bar = [&](int s) { return sBar + 8u * s; };
-  auto empty_bar = [&](int s) { return sBar + 8u * (S + s); };
-  auto xf_bar = [&](int s) { return sBar + 8u * (2 * S + s); };
-  const uint32_t wres_bar = sBar + 8u * (3 * S);
-  auto rowdone_bar = [&](uint32_t k) { return sBar + 8u * (3 * S + 1 + (k & (NBAR - 1))); };
-  auto drained_bar = [&](uint32_t k) { return sBar + 8u * (3 * S + 1 + NBAR + (k & (NBAR - 1))); };
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(gen + (sBar - base) + 8 * (3 * S + 1 + 2 * NBAR));
-
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < S; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); mbar_init(xf_bar(s), 4); }
-      mbar_init(wres_bar, 1);
-      for (int k = 0; k < NBAR; ++k) { mbar_init(rowdone_bar(k), 1); mbar_init(drained_bar(k), 4); }
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  } else if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapF)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapR)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapB)) : "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  if (warp >= 4 && warp < 8) {            // every accumulator starts at zero: each MMA of the kernel accumulates
-    const uint32_t lane_addr = (uint32_t)((warp & 3) * 32) << 16;
-    uint32_t z[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) z[i] = 0u;
-    for (int c = 0; c < 512; c += 32) tmem_st32(tmem_base + lane_addr + (uint32_t)c, z);
-    tmem_st_wait();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-
-  // Work = the rows of all column strips laid end to end, an equal share per CTA (msb_ring.cu)
-  const long long g_lo = (long long)blockIdx.x * p.total_rows / gridDim.x, g_hi = (long long)(blockIdx.x + 1) * p.total_rows / gridDim.x;
-  auto item = [&](long long g, int& img, int& seg, int& y0, int& y1) {
-    const int strip = (int)(g / p.H);
-    y0 = (int)(g - (long long)strip * p.H);
-    const long long left = g_hi - g;
-    y1 = (long long)(p.H - y0) < left ? p.H : y0 + (int)left;
-    img = strip / p.segs;
-    seg = strip - img * p.segs;
-  };
+  const Smem sm(smem_raw, SH, p.stages);
+  const Bars& bars = sm.b;
+  const uint32_t tmem_base = prologue(sm, warp, lane, 1, 4, 4, &mapF, &mapR, &mapB);
+  const Walk pieces(p.total_rows, p.H, p.segs);
 
   if (warp == 0) {
-    // ===================================== TMA producer =====================================
-    if (lane == 0) {
-      mbar_expect_tx(wres_bar, (uint32_t)W_BYTES);
-      for (int r = 0; r < W_ROWS; r += 64) tma_load_2d(sB + r * 128, &mapB, wres_bar, 0, r);
-      int s = 0;
-      uint32_t n = 0;
-      for (long long g = g_lo; g < g_hi;) {
-        int img, seg, y0, y1;
-        item(g, img, seg, y0, y1);
-        g += y1 - y0;
-        const int r_lo = y0 - HV < 0 ? 0 : y0 - HV, r_hi = y1 + HV > p.H ? p.H : y1 + HV;
-        for (int r = r_lo; r < r_hi; ++r, ++n) {
-#if O7_PREFETCH > 0
-          // (experiment: rows further ahead pulled into L2 so that the load filling a freed stage pays L2 latency; the kernel turned
-          // out to be bound by its issuing thread -- a run table in local memory -- not by load latency)
-          if (r == r_lo)
-            for (int a = 1; a < O7_PREFETCH && r + a < r_hi; ++a) {
-              tma_prefetch_4d(&mapF, 0, seg * BM - HALO, r + a, img);
-              tma_prefetch_4d(&mapR, 0, seg * BM - HALO, r + a, img);
-            }
-          if (r + O7_PREFETCH < r_hi) {
-            tma_prefetch_4d(&mapF, 0, seg * BM - HALO, r + O7_PREFETCH, img);
-            tma_prefetch_4d(&mapR, 0, seg * BM - HALO, r + O7_PREFETCH, img);
-          }
-#endif
-          if (n >= (uint32_t)S) mbar_wait(empty_bar(s), ((n / S) - 1) & 1);
-          mbar_expect_tx(full_bar(s), (uint32_t)STAGE);
-          tma_load_4d(sA + s * STAGE, &mapF, full_bar(s), 0, seg * BM - HALO, r, img);
-          tma_load_4d(sA + s * STAGE + SLAB_BYTES, &mapR, full_bar(s), 0, seg * BM - HALO, r, img);
-          if (++s == S) s = 0;
-        }
-      }
-    }
+    if (lane == 0)
+      producer(sm, pieces, p.H, &mapB, SH.w_bytes, 0, SH.stage_bytes, [&](const Walk& pc, int r, uint32_t dst, uint32_t bar) {
+        tma_load_4d(dst, &mapF, bar, 0, pc.seg * BM - HALO, r, pc.img);
+        tma_load_4d(dst + SLAB_BYTES, &mapR, bar, 0, pc.seg * BM - HALO, r, pc.img);
+      });
   } else if (warp == 1) {
-    // ===================================== MMA issuer =====================================
     const bool leader = elect_one();
     const uint32_t hi = (uint32_t)(make_sw128_desc(0) >> 32);
-    const uint32_t idesc0 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BM >> 4) << 24);      // + N
-    const uint32_t b_base = sB >> 4;
-    int s = 0;
-    uint32_t n = 0, k = 0;
-    mbar_wait(wres_bar, 0);
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      for (int r = y0 - HV; r < y1 + HV; ++r, ++k) {
-        if (k >= LEAD) mbar_wait(drained_bar(k - LEAD), ((k - LEAD) / NBAR) & 1);
-        // a new piece maps its rows onto the slots afresh: everything of the previous piece must have been drained
-        if (r == y0 - HV && k > 0) mbar_wait(drained_bar(k - 1), ((k - 1) / NBAR) & 1);
-        if (r >= 0 && r < p.H) {
-          mbar_wait(xf_bar(s), (n / S) & 1);           // the transform warps have turned the landed f slab into the operand
-          tc_fence_after();
-          if (leader) {
-            const uint32_t a0 = (sA + s * STAGE) >> 4;
-            // entries e = 0..6 = output rows r-3 .. r+3 (ky = 6 - e); those of this piece are an interval, and its ring slots are
-            // adjacent except where the ring wraps: one or two runs, found by arithmetic (a run table in local memory cost the
-            // issuing thread ~1000 cycles per row)
-            auto issue_run = [&](int e, int nrun, int slot) {
-              const uint32_t idesc = idesc0 | ((uint32_t)((NCOL * nrun) >> 3) << 17);
-              const uint32_t dcol = tmem_base + (uint32_t)(slot * NCOL);
+    const uint32_t b_base = sm.sB() >> 4;
+    // (waits for the transform warps to have turned the landed f slab into the operand)
+    issuer<LEAD, true>(bars, pieces, p.H, leader, [&](const Walk& pc, int r, int s) {
+      const uint32_t a0 = sm.sA(s, SH.stage_bytes) >> 4;
+      // entries e = 0..6 = output rows r-3 .. r+3 (ky = 6 - e); those of this piece are an interval of adjacent ring slots
+      const int o_lo = r - 3 > pc.y0 ? r - 3 : pc.y0, o_hi = r + 3 < pc.y1 - 1 ? r + 3 : pc.y1 - 1;      // inclusive
+      if (o_lo <= o_hi)
+        runs(o_hi - o_lo + 1, o_lo & (SLOTS - 1), SLOTS, [&](int e, int nrun, int slot) {
+          const uint32_t idesc = idesc_bf16(NCOL * nrun);
+          const uint32_t dcol = tmem_base + (uint32_t)(slot * NCOL);
 #pragma unroll
-              for (int kx = 0; kx < 7; ++kx) {
-                const uint32_t av = a0 + (uint32_t)((HALO + kx - 3) * 8);
-                const uint32_t bv = b_base + (uint32_t)((kx * 128 + NCOL * e) * 8);
+          for (int kx = 0; kx < 7; ++kx) {
+            const uint32_t av = a0 + (uint32_t)((HALO + kx - 3) * 8);
+            const uint32_t bv = b_base + (uint32_t)((kx * 128 + NCOL * (o_lo - (r - 3) + e)) * 8);
 #pragma unroll
-                for (int ks = 0; ks < 4; ++ks) umma_bf16_lo(dcol, av + (uint32_t)(2 * ks), bv + (uint32_t)(2 * ks), hi, idesc, true);
-              }
-            };
-            const int o_lo = r - 3 > y0 ? r - 3 : y0, o_hi = r + 3 < y1 - 1 ? r + 3 : y1 - 1;      // inclusive
-            if (o_lo <= o_hi) {
-              const int cnt = o_hi - o_lo + 1, slot = o_lo & (SLOTS - 1);
-              const int n1 = cnt < SLOTS - slot ? cnt : SLOTS - slot;
-              issue_run(o_lo - (r - 3), n1, slot);
-              if (cnt > n1) issue_run(o_lo - (r - 3) + n1, cnt - n1, 0);
-            }
-            umma_commit(empty_bar(s));
+            for (int ks = 0; ks < 4; ++ks) umma_bf16_lo(dcol, av + (uint32_t)(2 * ks), bv + (uint32_t)(2 * ks), hi, idesc, true);
           }
-          __syncwarp();
-          if (++s == S) s = 0;
-          ++n;
-        }
-        if (leader) umma_commit(rowdone_bar(k));
-        __syncwarp();
-      }
-    }
-  } else if (warp >= 4 && warp < 8) {
+        });
+    });
+  } else if (warp >= EPI0 && warp < XF0) {
     // ===================================== epilogue =====================================
     const int q = warp & 3;
     const int row = q * 32 + lane;
     const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
     const float b0 = p.bias ? p.bias[0] : 0.f, b1 = p.bias ? p.bias[1] : 0.f, b2 = p.bias ? p.bias[2] : 0.f;
-    uint32_t zero16[16];
-#pragma unroll
-    for (int i = 0; i < 16; ++i) zero16[i] = 0u;
     uint32_t k = 0;
     const size_t plane = (size_t)p.H * p.W;
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      const int xcol = seg * BM + row;
+    for (Walk pc = pieces; pc.next();) {
+      const int xcol = pc.seg * BM + row;
       const bool valid = xcol < p.W;
-      for (int r = y0 - HV; r < y1 + HV; ++r, ++k) {
-        mbar_wait(rowdone_bar(k), (k / NBAR) & 1);
+      for (int r = pc.r0; r < pc.r1; ++r, ++k) {
+        bars.wait_rowdone(k);
         const int o = r - 3;                                         // the output row this input row completed
-        const bool okr = o >= y0 && o < y1;                          // (warp-uniform)
+        const bool okr = o >= pc.y0 && o < pc.y1;                    // (warp-uniform)
         float v[4];
         if (okr) {
           tc_fence_after();
           const uint32_t taddr = tmem_base + lane_addr + (uint32_t)((o & (SLOTS - 1)) * NCOL);
           tmem_ld4(taddr, v);
           tmem_ld_wait();
-          tmem_st16(taddr, zero16);                                  // (columns 3..15 only ever received zero weights)
+          tmem_zero<16>(taddr);                                      // (columns 3..15 only ever received zero weights)
           tmem_st_wait();
           tc_fence_before();
         }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(drained_bar(k));
+        arrive_drained(bars, k, lane);
         if (okr && valid) {
-          float* y = p.y + (size_t)img * 3 * plane + (size_t)o * p.W + xcol;
+          float* y = p.y + (size_t)pc.img * 3 * plane + (size_t)o * p.W + xcol;
           y[0] = tanhf(v[0] + b0);
           y[plane] = tanhf(v[1] + b1);
           y[2 * plane] = tanhf(v[2] + b2);
         }
       }
     }
-  } else if (warp >= 8) {
+  } else if (warp >= XF0) {
     // ===================================== transform: f slab -> a2 operand, in place =====================================
-    // Thread t owns the physical 16-byte chunk (t & 7) of the slab rows (t >> 3) + 16 i: a warp touches 512 contiguous bytes per
-    // access, and because the 128-byte swizzle only uses row & 7 the LOGICAL channel chunk of a thread is the same for all its rows:
-    // its 8 scales / shifts live in registers (conv_tma.cu's fused input norm).
-    const int xt = tid - 32 * 8;                       // 0..127
+    const int xt = tid - 32 * XF0;                     // 0..127
     const int pchunk = xt & 7, rbase = xt >> 3;
     const int lchunk = pchunk ^ (rbase & 7);
     const double inv_hw = 1.0 / ((double)p.H * (double)p.W);
     float sc[8], sh[8];
     int cur_img = -1;
-    int s = 0;
-    uint32_t n = 0;
-    for (long long g = g_lo; g < g_hi;) {
-      int img, seg, y0, y1;
-      item(g, img, seg, y0, y1);
-      g += y1 - y0;
-      if (img != cur_img) {
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          const double* st = p.in_stats + ((size_t)img * p.Cs_total + p.cs_off + lchunk * 8 + e) * 2;
-          float mean, rstd;
-          finalize_stats(st[0], st[1], inv_hw, mean, rstd);
-          sc[e] = rstd;
-          sh[e] = 0.f - mean * rstd;
-        }
-        cur_img = img;
+    SlabRing ring(bars.S);
+    for (Walk pc = pieces; pc.next();) {
+      if (pc.img != cur_img) {
+        load_scale_shift(p.in_stats, pc.img, p.Cs_total, p.cs_off, lchunk, inv_hw, sc, sh);
+        cur_img = pc.img;
       }
-      const int r_lo = y0 - HV < 0 ? 0 : y0 - HV, r_hi = y1 + HV > p.H ? p.H : y1 + HV;
-      const int x0 = seg * BM - HALO;                  // image column of slab pixel 0
-      for (int r = r_lo; r < r_hi; ++r, ++n) {
-        mbar_wait(full_bar(s), (n / S) & 1);
-        uint8_t* fs = gen + (sA - base) + s * STAGE + rbase * 128 + pchunk * 16;
+      const int r_lo = pc.r0 < 0 ? 0 : pc.r0, r_hi = pc.r1 > p.H ? p.H : pc.r1;
+      const int x0 = pc.seg * BM - HALO;               // image column of slab pixel 0
+      for (int r = r_lo; r < r_hi; ++r) {
+        mbar_wait(bars.full(ring.s), ring.parity());
+        uint8_t* fs = sm.stage_ptr(ring.s, SH.stage_bytes) + rbase * 128 + pchunk * 16;
         // (loads batched ahead of the arithmetic, no branches: rows 128..135 exist only for rbase < 8 -- those threads' ninth chunk --
         // and out-of-plane pixels are forced to 0 by a select: the conv's zero padding is a padding of a2)
         {
@@ -316,17 +178,12 @@ out7_ring_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_constant
         }
         fence_proxy_async();                           // generic-proxy writes -> visible to the tensor core
         __syncwarp();
-        if (lane == 0) mbar_arrive(xf_bar(s));
-        if (++s == S) s = 0;
+        if (lane == 0) mbar_arrive(bars.xf(ring.s));
+        ring.advance();
       }
     }
   }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-  }
+  teardown(warp, tmem_base);
 }
 
 }  // namespace
@@ -344,8 +201,7 @@ extern "C" int msg_out7_ring(const msg_out7_ring_desc* d, const void* f, const d
   MSG_REQUIRE((d->Cr_total & 7) == 0 && (d->cr_off & 7) == 0 && d->cr_off + 64 <= d->Cr_total, MSG_ERR_SHAPE, "out7_ring: residual channel layout");
   MSG_REQUIRE(d->cs_off >= 0 && d->cs_off + 64 <= d->Cs_total, MSG_ERR_SHAPE, "out7_ring: stats layout");
   MSG_REQUIRE((((uintptr_t)f | (uintptr_t)residual | (uintptr_t)w_stacks) & 15) == 0, MSG_ERR_ALIGN, "out7_ring: operands must be 16-byte aligned");
-  EncodeTiledFn enc = get_encode();
-  MSG_REQUIRE(enc != nullptr, MSG_ERR_CUDA, "out7_ring: cuTensorMapEncodeTiled unavailable");
+  MSG_REQUIRE(get_encode() != nullptr, MSG_ERR_CUDA, "out7_ring: cuTensorMapEncodeTiled unavailable");
 
   O7Params p;
   p.N = d->N; p.H = d->H; p.W = d->W;
@@ -355,43 +211,11 @@ extern "C" int msg_out7_ring(const msg_out7_ring_desc* d, const void* f, const d
   p.bias = bias; p.in_stats = in_stats; p.Cs_total = d->Cs_total; p.cs_off = d->cs_off; p.y = y;
 
   CUtensorMap mapF, mapR, mapB;
-  auto slab_map = [&](CUtensorMap* m, const void* ptr, int Ct, int off) -> CUresult {
-    cuuint64_t dims[4] = {64, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-    cuuint64_t strides[3] = {(cuuint64_t)Ct * 2, (cuuint64_t)d->W * Ct * 2, (cuuint64_t)d->H * d->W * Ct * 2};
-    cuuint32_t box[4] = {64, (cuuint32_t)SLAB_PX, 1, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    void* b0 = (void*)((const __nv_bfloat16*)ptr + off);
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, b0, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  };
-  CUresult r = slab_map(&mapF, f, d->Cf_total, d->cf_off);
+  CUresult r = encode_slab(&mapF, (const __nv_bfloat16*)f + d->cf_off, 64, d->Cf_total, d->W, d->H, d->N);
   MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "out7_ring: cuTensorMapEncodeTiled(f) failed with %d", (int)r);
-  r = slab_map(&mapR, residual, d->Cr_total, d->cr_off);
+  r = encode_slab(&mapR, (const __nv_bfloat16*)residual + d->cr_off, 64, d->Cr_total, d->W, d->H, d->N);
   MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "out7_ring: cuTensorMapEncodeTiled(residual) failed with %d", (int)r);
-  {
-    cuuint64_t dims[2] = {64, (cuuint64_t)W_ROWS};
-    cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, 64};
-    cuuint32_t es[2] = {1, 1};
-    r = enc(&mapB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)w_stacks, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "out7_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
-  }
-  const int fixed = W_BYTES + 8 * (3 * 8 + 1 + 2 * NBAR) + 64 + 1024;
-  int stages = (227 * 1024 - fixed) / STAGE;
-  if (stages > 8) stages = 8;
-  MSG_REQUIRE(stages >= 2, MSG_ERR_UNSUPPORTED, "out7_ring: the slab ring does not fit shared memory");
-  p.stages = stages;
-  const size_t smem = (size_t)stages * STAGE + fixed;
-  static DeviceOnce attr_set;
-  if (attr_set.needed()) {
-    cudaError_t e = cudaFuncSetAttribute(out7_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    MSG_REQUIRE(e == cudaSuccess, MSG_ERR_CUDA, "out7_ring: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    attr_set.done();
-  }
-  const int sms = sm_count();
-  const long long grid_ll = p.total_rows / 8;
-  const int grid = grid_ll < 1 ? 1 : (grid_ll > sms ? sms : (int)grid_ll);
-  out7_ring_kernel<<<grid, NTHREADS, smem, st>>>(mapF, mapR, mapB, p);
-  return check_launch("out7_ring_kernel");
+  r = encode_weights(&mapB, w_stacks, W_ROWS);
+  MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "out7_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
+  return launch<out7_ring_kernel>("out7_ring_kernel", o7_shape(), NTHREADS, p.total_rows, 8, p, mapF, mapR, mapB, st);
 }
