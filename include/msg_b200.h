@@ -267,6 +267,27 @@ int msg_nhwc_to_nchw(int dtype, const void* x, int N, int C, int H, int W, int C
 int msg_blend_outputs(const float* const* ys, const float* w, int S, const float* x, float w_x,
                       float gain, int do_clip, float clip_lo, float clip_hi, long long numel,
                       float* out_f32, uint8_t* out_u8, void* stream);
+/* Per-pixel multi-style blend (enhanced_local_style.py:126-176, 232-236): the weights of each output pixel come from maps.
+ * ys: S (1..8) device pointers (host array) to fp32 NCHW [N,C,H,W]; x: the input image, same shape (needed when K = S+1,
+ * ignored otherwise); maps: fp32 [map_batch][K][h][w] with map_batch in {1, N} (1: one map set for every image), K in {S, S+1}
+ * (map S weights x), 1 <= h <= H and 1 <= w <= W.  For output pixel (n, c, i, j):
+ *   1. sample m_k = bilinear(maps[n or 0][k], i, j) with F.interpolate(mode="bilinear", align_corners=False)'s source index:
+ *      scale = (float)h / H, src = max(scale * (i + 0.5) - 0.5, 0), i0 = (int)src, i1 = min(i0 + 1, h - 1), t = src - i0
+ *      (columns alike), interpolated as a + t * (b - a), rows first, then columns -- a constant map is returned exactly, so
+ *      a 1x1 map is a per-image weight;
+ *   2. normalize != 0: m_k /= sum_k m_k (all weights 0 where the sum is 0);
+ *   3. v = 0; v = fmaf(m_s, ys[s], v) for s < S; v = fmaf(m_S, x, v) if K = S+1; v *= gain; optional clamp; fp32 and/or
+ *      uint8 output as msg_blend_outputs.
+ * With normalize = 0, constant maps equal to (w, w_x) give msg_blend_outputs' result bit for bit. */
+int msg_blend_maps(const float* const* ys, int S, const float* x, const float* maps, int map_batch, int K, int h, int w,
+                   int N, int C, int H, int W, int normalize, float gain, int do_clip, float clip_lo, float clip_hi,
+                   float* out_f32, uint8_t* out_u8, void* stream);
+/* Feathering of weight maps: scipy.ndimage.gaussian_filter(plane, sigma, mode="reflect", truncate=4.0) of each of `planes`
+ * fp32 h x w planes.  Radius r = int(4 sigma + 0.5) (<= 255), taps exp(-x^2 / 2 sigma^2) normalised to sum 1 (computed in
+ * double, rounded to float), vertical pass into tmp then horizontal pass into out, fp32 accumulation; indices outside [0, n)
+ * reflect half-sample-symmetrically (i mod 2n, then 2n-1-i if >= n), also when r >= n.  sigma = 0 copies.
+ * tmp: caller-owned [planes][h][w] fp32 workspace. */
+int msg_gaussian_blur(const float* in, long long planes, int h, int w, float sigma, float* tmp, float* out, void* stream);
 
 /* MultiScaleBlock branches at C = 64 (enhanced_generator.py:52-71: 1x1 | 3x3 dil 1 | 3x3 dil 2 | 3x3 dil 4, 64 -> 4 x 16
  * channels written as ONE 64-channel slice, bias added, optional IN statistics) as a row ring of tensor-memory accumulators:

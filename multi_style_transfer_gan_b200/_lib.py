@@ -111,6 +111,9 @@ SIGNATURES = {
     "msg_nhwc_to_nchw": [c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "msg_blend_outputs": [ctypes.POINTER(_P), ctypes.POINTER(c_float), c_int, _P, c_float, c_float,
                           c_int, c_float, c_float, c_ll, _P, _P, _P],
+    "msg_blend_maps": [ctypes.POINTER(_P), c_int, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                       c_float, c_int, c_float, c_float, _P, _P, _P],
+    "msg_gaussian_blur": [_P, c_ll, c_int, c_int, c_float, _P, _P, _P],
     "msg_mse_loss": [_P, _P, c_float, c_ll, c_float, _P, _P, _P],
     "msg_l1_loss": [_P, _P, c_float, c_ll, c_float, _P, _P, _P, _P],
     "msg_msb64_ring": [ctypes.POINTER(MsbRingDesc), _P, _P, _P, _P, _P, _P],

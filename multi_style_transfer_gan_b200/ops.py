@@ -363,6 +363,48 @@ def blend_outputs(ys, w, x=None, w_x=0.0, gain=1.0, clip=None, out_uint8=False, 
     return (out, u8) if out_uint8 else out
 
 
+def blend_maps(ys, maps, x=None, gain=1.0, clip=None, normalize=False, out_uint8=False, out=None):
+    """Per-pixel blend: out[n,:,i,j] = gain * (sum_k m_k(n,i,j) * plane_k[n,:,i,j]), optional clip / uint8 as blend_outputs.
+    ys: S fp32 CUDA tensors [N,C,H,W]; maps: fp32 CUDA [Bm,K,h,w] with Bm in {1, N}, K in {S, S+1} (map S weights x),
+    h <= H, w <= W, sampled bilinearly (align_corners=False) at each pixel; normalize divides the K weights by their sum."""
+    ys = [y.detach().contiguous() for y in ys]
+    _dev(ys[0])
+    S = len(ys)
+    N, C, H, W = ys[0].shape
+    maps = maps.detach()
+    assert maps.dtype == torch.float32 and maps.dim() == 4 and maps.is_contiguous(), "maps: contiguous fp32 [Bm,K,h,w]"
+    _dev(maps)
+    Bm, K, h, w = maps.shape
+    ptrs = (ctypes.c_void_p * S)(*[y.data_ptr() for y in ys])
+    if out is not None and out.dtype == torch.uint8:
+        u8, out = out, None
+        assert u8.is_contiguous() and u8.shape == ys[0].shape
+    else:
+        if out is None:
+            out = torch.empty_like(ys[0])
+        assert out.is_contiguous() and out.shape == ys[0].shape and out.dtype == torch.float32
+        u8 = torch.empty(ys[0].shape, device=ys[0].device, dtype=torch.uint8) if out_uint8 else None
+    lo, hi = (clip if clip is not None else (0.0, 0.0))
+    xx = None if x is None else x.detach().contiguous()
+    _lib.call("msg_blend_maps", ptrs, S, _p(xx), _p(maps), Bm, K, h, w, N, C, H, W, int(bool(normalize)), float(gain),
+              int(clip is not None), float(lo), float(hi), _p(out), _p(u8), _stream())
+    if out is None:
+        return u8
+    return (out, u8) if out_uint8 else out
+
+
+def gaussian_blur(planes, sigma):
+    """scipy.ndimage.gaussian_filter(mode="reflect", truncate=4.0) of every trailing [h, w] plane of an fp32 CUDA tensor."""
+    _dev(planes)
+    assert planes.dtype == torch.float32 and planes.dim() >= 2
+    src = planes.detach().contiguous()
+    h, w = src.shape[-2:]
+    tmp = torch.empty_like(src)
+    out = torch.empty_like(src)
+    _lib.call("msg_gaussian_blur", _p(src), src.numel() // max(h * w, 1), h, w, float(sigma), _p(tmp), _p(out), _stream())
+    return out
+
+
 # ---- misc ----------------------------------------------------------------------------------------
 def tanh_bwd_nchw(y, dy, dtype, Cp):
     N, C, H, W = y.shape

@@ -12,11 +12,39 @@ amortise the persistent kernels' ramp-up/tail and the small-plane launches, smal
 activation footprint); host input is staged through pinned memory on a copy stream so H2D of
 micro-batch i+1 overlaps the compute of micro-batch i.
 """
+import math
 import os
 
 import torch
 
 from . import _lib, ops
+
+
+def check_blend_args(S, B, H, W, weights, w_x, weight_maps, feather_sigma):
+    """Validates the blend arguments of MultiStyleStylizer.__call__ for S styles and B images of HxW before any device work:
+    exactly one of `weights` (S global weights) and `weight_maps` (fp [Bm, K, h, w], Bm in {1, B}, K in {S, S+1}, h <= H,
+    w <= W; map S weights the input image, so w_x must be 0) and a finite feather_sigma >= 0.  Raises ValueError."""
+    if (weights is None) == (weight_maps is None):
+        raise ValueError("give exactly one of `weights` (global) and `weight_maps` (per pixel)")
+    if weight_maps is None:
+        if len(weights) != S:
+            raise ValueError(f"{S} styles but {len(weights)} weights")
+        return
+    if w_x != 0.0:
+        raise ValueError("w_x must be 0 with weight_maps: map S (of S+1) weights the input image")
+    if not torch.is_tensor(weight_maps) or not weight_maps.is_floating_point():
+        raise ValueError("weight_maps must be a floating-point tensor [Bm, K, h, w]")
+    if weight_maps.dim() != 4:
+        raise ValueError(f"weight_maps must be [Bm, K, h, w], got shape {tuple(weight_maps.shape)}")
+    Bm, K, h, w = weight_maps.shape
+    if K not in (S, S + 1):
+        raise ValueError(f"{K} weight maps for {S} styles: need {S} (styles) or {S + 1} (styles and the input image)")
+    if Bm not in (1, B):
+        raise ValueError(f"{Bm} map sets for {B} images: need 1 (shared) or {B} (one per image)")
+    if not (1 <= h <= H and 1 <= w <= W):
+        raise ValueError(f"{h}x{w} weight maps for {H}x{W} images: maps must be non-empty and no larger than the image")
+    if not math.isfinite(feather_sigma) or feather_sigma < 0:
+        raise ValueError(f"feather_sigma must be finite and >= 0, got {feather_sigma}")
 
 
 def shard_range(num_images, rank, world_size):
@@ -49,8 +77,9 @@ class MultiStyleStylizer:
         self.use_graph = bool(use_graph)
         self._graphs = {}
 
-    def _forward_chunk(self, xi, weights, w_x, gain, clip, dst):
-        """All styles of one micro-batch + the blend into dst, enqueued on the current stream (and the style streams)."""
+    def _forward_chunk(self, xi, weights, w_x, gain, clip, dst, maps=None, normalize=False):
+        """All styles of one micro-batch + the blend into dst, enqueued on the current stream (and the style streams).
+        maps: the micro-batch's weight maps [Bm, K, h, w] on the device (per-pixel blend) instead of `weights`."""
         cur = torch.cuda.current_stream(self.device)
         capturing = torch.cuda.is_current_stream_capturing()
         if self.style_streams:
@@ -74,42 +103,52 @@ class MultiStyleStylizer:
                 cur.wait_event(ev_s)
         else:
             ys = [g(xi) for g in self.generators]
-        ops.blend_outputs(ys, weights, x=xi if w_x != 0.0 else None, w_x=w_x, gain=gain, clip=clip, out=dst)
+        if maps is None:
+            ops.blend_outputs(ys, weights, x=xi if w_x != 0.0 else None, w_x=w_x, gain=gain, clip=clip, out=dst)
+        else:
+            ops.blend_maps(ys, maps, x=xi if maps.shape[1] > len(ys) else None, gain=gain, clip=clip, normalize=normalize,
+                           out=dst)
 
-    def _replay(self, xi, weights, w_x, gain, clip, dst, pver=None):
+    def _replay(self, xi, weights, w_x, gain, clip, dst, pver=None, maps=None, normalize=False):
         """CUDA-graph path: the ~210 launches of a micro-batch (S forwards + blend) are captured once per
         (shape, blend parameters) and replayed, so the host cost of a micro-batch is one graph launch.  Weights are
-        read through the per-generator pack caches at capture time: `invalidate_graphs()` after changing them."""
-        key = (tuple(xi.shape), tuple(float(w) for w in weights), float(w_x), float(gain), clip, dst.dtype,
+        read through the per-generator pack caches at capture time: `invalidate_graphs()` after changing them.
+        Weight maps are a graph input like the images: the key holds their shape and `normalize`, each replay copies the
+        micro-batch's maps into the entry's static buffer."""
+        key = (tuple(xi.shape), tuple(float(w) for w in weights) if maps is None else ("maps", tuple(maps.shape), bool(normalize)),
+               float(w_x), float(gain), clip, dst.dtype,
                pver if pver is not None else tuple(g.param_version() for g in self.generators))
         ent = self._graphs.get(key)
         if ent is None:
             sx = torch.empty_like(xi)
             sd = torch.empty_like(dst)
             sx.copy_(xi)
+            sm = None if maps is None else maps.clone()
             for _ in range(2):                    # warm-up outside capture: weight packs, function attributes, allocator
-                self._forward_chunk(sx, weights, w_x, gain, clip, sd)
+                self._forward_chunk(sx, weights, w_x, gain, clip, sd, sm, normalize)
             torch.cuda.current_stream(self.device).synchronize()
             gr = torch.cuda.CUDAGraph()
             l0 = _lib.launches
             try:
                 with torch.cuda.graph(gr):
-                    self._forward_chunk(sx, weights, w_x, gain, clip, sd)
+                    self._forward_chunk(sx, weights, w_x, gain, clip, sd, sm, normalize)
             except Exception as e:                # capture refused (e.g. a user-supplied transformer block that syncs):
                 import warnings                   # same kernels, launched one by one
                 warnings.warn(f"MultiStyleStylizer: CUDA-graph capture failed ({e!r}); continuing without graphs")
                 self.use_graph = False
                 torch.cuda.synchronize(self.device)
-                self._forward_chunk(xi, weights, w_x, gain, clip, dst)
+                self._forward_chunk(xi, weights, w_x, gain, clip, dst, maps, normalize)
                 return
             while len(self._graphs) >= 8:         # stale keys (old parameter versions, other shapes): drop the oldest
                 self._graphs.pop(next(iter(self._graphs)))
             # the captured launches address the packed weights of each generator's cache (allocated during the warm-up, outside
             # the graph's pool): the entry keeps them alive, so invalidate_packed_weights() cannot free memory a graph reads
             keep = [list(g._engine._cache.values()) for g in self.generators]
-            ent = self._graphs[key] = (gr, sx, sd, _lib.launches - l0, keep)
-        gr, sx, sd, n_launches = ent[:4]
+            ent = self._graphs[key] = (gr, sx, sd, _lib.launches - l0, keep, sm)
+        gr, sx, sd, n_launches, _, sm = ent
         sx.copy_(xi)
+        if sm is not None:
+            sm.copy_(maps)
         gr.replay()
         _lib.launches += n_launches               # kernels inside the replayed graph (the launch counter is per C-ABI call)
         dst.copy_(sd)
@@ -118,20 +157,31 @@ class MultiStyleStylizer:
         self._graphs.clear()
 
     @torch.no_grad()
-    def __call__(self, x, weights, w_x=0.0, gain=1.0, clip=None, out_uint8=False, out=None):
+    def __call__(self, x, weights=None, w_x=0.0, gain=1.0, clip=None, out_uint8=False, out=None, *, weight_maps=None,
+                 feather_sigma=0.0, normalize_maps=False):
         """x: float32 [B,3,H,W] in [-1,1], or uint8 [B,H,W,3] (PIL layout: ToTensor + Normalize(0.5, 0.5) then run on the
         device, batch_process_images.py:287-291 -- a quarter of the host-to-device bytes), on the device or on the host
         (pinned for overlap).
         Returns the blended fp32 images [B,3,H,W] on the device, or -- with out_uint8=True -- the
         uint8 images ((v+1)/2 -> clamp -> *255, direct_transform.py:66-71) in `out` (host or device
-        uint8 tensor [B,3,H,W]; allocated on the device if None)."""
+        uint8 tensor [B,3,H,W]; allocated on the device if None).
+        weight_maps (instead of `weights`): per-pixel style weights [Bm, K, h, w] (host or device, Bm in {1, B}, K in {S, S+1}
+        with map S weighting the input image, h <= H, w <= W), sampled bilinearly at every pixel (ops.blend_maps;
+        enhanced_local_style.py:126-176, 232-236).  A [B, S, 1, 1] tensor gives each image its own global mix.
+        feather_sigma > 0 blurs each map plane with a Gaussian first (ops.gaussian_blur); normalize_maps divides the
+        sampled weights of each pixel by their sum."""
         S = len(self.generators)
-        if len(weights) != S:
-            raise ValueError(f"{S} styles but {len(weights)} weights")
+        hw = (tuple(x.shape[1:3]) if x.dtype == torch.uint8 else tuple(x.shape[2:4])) if x.dim() == 4 else (0, 0)
+        check_blend_args(S, x.shape[0], *hw, weights, w_x, weight_maps, float(feather_sigma))
         with torch.cuda.device(self.device):
-            return self._run(x, weights, w_x, gain, clip, out_uint8, out)
+            maps = None
+            if weight_maps is not None:            # moved and feathered once per call, sliced per micro-batch
+                maps = weight_maps.to(self.device, torch.float32).contiguous()
+                if feather_sigma > 0:
+                    maps = ops.gaussian_blur(maps, feather_sigma)
+            return self._run(x, weights, w_x, gain, clip, out_uint8, out, maps, bool(normalize_maps))
 
-    def _run(self, x, weights, w_x, gain, clip, out_uint8, out):
+    def _run(self, x, weights, w_x, gain, clip, out_uint8, out, maps=None, normalize=False):
         B = x.shape[0]
         mb = self.micro_batch
         host_in = not x.is_cuda
@@ -174,10 +224,11 @@ class MultiStyleStylizer:
             dst = None if host_out else out[lo:hi]      # device result: the blend writes it in place
             if dst is None:
                 dst = torch.empty((hi - lo,) + tuple(out.shape[1:]), device=self.device, dtype=out.dtype)
+            mi = None if maps is None else (maps if maps.shape[0] == 1 else maps[lo:hi])
             if self.use_graph:
-                self._replay(xi, weights, w_x, gain, clip, dst, pver)
+                self._replay(xi, weights, w_x, gain, clip, dst, pver, mi, normalize)
             else:
-                self._forward_chunk(xi, weights, w_x, gain, clip, dst)
+                self._forward_chunk(xi, weights, w_x, gain, clip, dst, mi, normalize)
             if host_out:
                 out[lo:hi].copy_(dst, non_blocking=True)
         if host_out:
