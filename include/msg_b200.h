@@ -218,6 +218,25 @@ int msg_instnorm_apply(int dtype, const void* x, const double* stats, int N, lon
  * (d residual = dy is the caller's business.)  scratch: fp64 [N][C][2], zeroed by the callee. */
 int msg_instnorm_bwd(int dtype, const void* x, const double* stats, const void* dy, int N,
                      long long HW, int C, int act, double* scratch, void* dx, void* stream);
+/* The two halves of msg_instnorm_bwd, for a backward that runs a collective between them
+ * (synchronised BatchNorm: sum the per-channel reductions over the ranks, then apply).
+ * gamma, beta: optional per-channel affine, fp32 [C] (both NULL: none).  The forward was
+ * y = act(z), z = fmaf(x, scale, shift), scale = rstd * gamma, shift = beta - mean * scale
+ * (msg_instnorm_apply with S = 1, w = {1}); g = dy * act'(z) takes its mask from z rebuilt with
+ * that same arithmetic, so it equals the sign of the stored y and y need not be read.
+ *   reduce: zeroes sums, then sums[n][c] = (sum g, sum g * xhat) in fp64.
+ *   apply:  dx = gamma * rstd * (g - sums[n][c][0] / HW - xhat * sums[n][c][1] / HW), rounded to
+ *           the storage type once.
+ * Statistics convention: every stats / sums a kernel sees is normalised to the LOCAL element
+ * count HW.  A caller that reduces over M_global elements held on several ranks scales the
+ * all-reduced global sums by HW_local / M_global (in fp64) before handing them to a kernel; with
+ * one rank that factor is exactly 1, and msg_instnorm_apply serves the synchronised forward. */
+int msg_instnorm_bwd_reduce(int dtype, const void* x, const double* stats, const void* dy, int N,
+                            long long HW, int C, int act, const float* gamma, const float* beta,
+                            double* sums, void* stream);
+int msg_instnorm_bwd_apply(int dtype, const void* x, const double* stats, const void* dy, int N,
+                           long long HW, int C, int act, const float* gamma, const float* beta,
+                           const double* sums, void* dx, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * LocalAttention core (enhanced_generator.py:22-35) on a [N,H,W,3C] qkv map (the 1x1 qkv conv is

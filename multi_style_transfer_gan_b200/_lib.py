@@ -102,6 +102,8 @@ SIGNATURES = {
     "msg_instnorm_stats": [c_int, _P, c_int, c_ll, c_int, _P, _P],
     "msg_instnorm_apply": [c_int, _P, _P, c_int, c_ll, c_int, c_int, _P, c_int, _P, _P, _P, _P, _P],
     "msg_instnorm_bwd": [c_int, _P, _P, _P, c_int, c_ll, c_int, c_int, _P, _P, _P],
+    "msg_instnorm_bwd_reduce": [c_int, _P, _P, _P, c_int, c_ll, c_int, c_int, _P, _P, _P, _P],
+    "msg_instnorm_bwd_apply": [c_int, _P, _P, _P, c_int, c_ll, c_int, c_int, _P, _P, _P, _P, _P],
     "msg_local_attn_fwd": [c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "msg_local_attn_bwd": [c_int, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "msg_la_stage_set_trace": [_P],

@@ -225,12 +225,34 @@ in_apply_fast_kernel(const T* __restrict__ x, const double* __restrict__ stats, 
 }
 
 // ---- backward -------------------------------------------------------------------------------
-// pass 1: scratch[n][c] += (sum g, sum g*xhat) with g = dy * act'(xhat)
-template <typename T, bool FAST>
+// Per-channel constants of the backward.  xhat = (x - mean) * rstd.  With an affine (gamma, beta: fp32 [C]) the
+// activation's input is rebuilt as z = fmaf(x, scale, shift), scale = rstd * gamma, shift = beta - mean * scale: the
+// arithmetic of the forward apply, so the ReLU / LeakyReLU mask is the sign of the stored forward output bit for bit.
+// Without one, z = xhat and scale = rstd.
+template <bool AFFINE>
+__device__ __forceinline__ void bwd_channel(const double* st, double inv_hw, const float* gamma, const float* beta, int c,
+                                            float& mean, float& rstd, float& scale, float& shift) {
+  finalize_stats(st[0], st[1], inv_hw, mean, rstd);
+  scale = rstd;
+  shift = 0.f;
+  if constexpr (AFFINE) {
+    scale = rstd * gamma[c];
+    shift = beta[c] - mean * scale;
+  }
+}
+
+// g = dy * act'(z)
+template <bool AFFINE>
+__device__ __forceinline__ float bwd_grad(float t, float dy, float xh, float scale, float shift, int act) {
+  return dy * act_grad_from_pre(AFFINE ? fmaf(t, scale, shift) : xh, act);
+}
+
+// pass 1: scratch[n][c] += (sum g, sum g*xhat)
+template <typename T, bool FAST, bool AFFINE>
 __global__ void __launch_bounds__(TPB)
 in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
-                     const T* __restrict__ dy, long long HW, int C, int act,
-                     double* __restrict__ scratch) {
+                     const T* __restrict__ dy, long long HW, int C, int act, const float* __restrict__ gamma,
+                     const float* __restrict__ beta, double* __restrict__ scratch) {
   constexpr int W = FAST ? Vec<T>::W : 1;
   __shared__ float red[TPB][2 * W + 1];
   const int n = blockIdx.y;
@@ -240,12 +262,11 @@ in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
     const long long nvec = HW * C / W;
     const long long stride = (long long)gridDim.x * TPB;
     long long v0 = (long long)blockIdx.x * TPB + threadIdx.x;
-    float mean[W], rstd[W], sg[W], sgx[W];
+    float mean[W], rstd[W], scale[W], shift[W], sg[W], sgx[W];
     int c0 = (int)((v0 * W) % C);
 #pragma unroll
     for (int e = 0; e < W; ++e) {
-      const double* st = stats + ((size_t)n * C + c0 + e) * 2;
-      finalize_stats(st[0], st[1], inv_hw, mean[e], rstd[e]);
+      bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, c0 + e, mean[e], rstd[e], scale[e], shift[e]);
       sg[e] = 0.f; sgx[e] = 0.f;
     }
     constexpr int U = 4;          // 2 x U raw 16-byte loads in flight per thread (unpacked only when consumed)
@@ -268,7 +289,7 @@ in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
 #pragma unroll
           for (int e = 0; e < W; ++e) {
             float xh = (t[e] - mean[e]) * rstd[e];
-            float gg = g[e] * act_grad_from_pre(xh, act);
+            float gg = bwd_grad<AFFINE>(t[e], g[e], xh, scale[e], shift[e], act);
             sg[e] += gg; sgx[e] = fmaf(gg, xh, sgx[e]);
           }
         }
@@ -289,13 +310,13 @@ in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
   } else {
     // generic: grid.x == C, one block per plane
     const int c = blockIdx.x;
-    const double* st = stats + ((size_t)n * C + c) * 2;
-    float mean, rstd;
-    finalize_stats(st[0], st[1], inv_hw, mean, rstd);
+    float mean, rstd, scale, shift;
+    bwd_channel<AFFINE>(stats + ((size_t)n * C + c) * 2, inv_hw, gamma, beta, c, mean, rstd, scale, shift);
     float sg = 0.f, sgx = 0.f;
     for (long long p = threadIdx.x; p < HW; p += TPB) {
-      float xh = (to_f<T>(x[base + (size_t)p * C + c]) - mean) * rstd;
-      float gg = to_f<T>(dy[base + (size_t)p * C + c]) * act_grad_from_pre(xh, act);
+      float t = to_f<T>(x[base + (size_t)p * C + c]);
+      float xh = (t - mean) * rstd;
+      float gg = bwd_grad<AFFINE>(t, to_f<T>(dy[base + (size_t)p * C + c]), xh, scale, shift, act);
       sg += gg; sgx = fmaf(gg, xh, sgx);
     }
     sg = warp_sum(sg); sgx = warp_sum(sgx);
@@ -310,12 +331,12 @@ in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
   }
 }
 
-// pass 2: dx = rstd * (g - mean(g) - xhat * mean(g*xhat))
-template <typename T, bool FAST>
+// pass 2: dx = gamma * rstd * (g - mean(g) - xhat * mean(g*xhat)), the means taken from scratch / HW
+template <typename T, bool FAST, bool AFFINE>
 __global__ void __launch_bounds__(TPB)
 in_bwd_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats,
-                    const T* __restrict__ dy, long long HW, int C, int act,
-                    const double* __restrict__ scratch, T* __restrict__ dx) {
+                    const T* __restrict__ dy, long long HW, int C, int act, const float* __restrict__ gamma,
+                    const float* __restrict__ beta, const double* __restrict__ scratch, T* __restrict__ dx) {
   constexpr int W = FAST ? Vec<T>::W : 1;
   const int n = blockIdx.y;
   const double inv_hw = 1.0 / (double)HW;
@@ -323,14 +344,13 @@ in_bwd_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats,
   const long long nvec = HW * C / W;
   const long long stride = (long long)gridDim.x * TPB;
   long long v0 = (long long)blockIdx.x * TPB + threadIdx.x;
-  float mean[W], rstd[W], mg[W], mgx[W];
+  float mean[W], rstd[W], scale[W], shift[W], mg[W], mgx[W];
   if constexpr (FAST) {
     // channel group of a thread is loop-invariant (stride * W is a multiple of C); 2 x U raw loads in flight per thread
     const int c0 = (int)((v0 * W) % C);
 #pragma unroll
     for (int e = 0; e < W; ++e) {
-      const double* st = stats + ((size_t)n * C + c0 + e) * 2;
-      finalize_stats(st[0], st[1], inv_hw, mean[e], rstd[e]);
+      bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, c0 + e, mean[e], rstd[e], scale[e], shift[e]);
       const double* sc = scratch + ((size_t)n * C + c0 + e) * 2;
       mg[e] = (float)(sc[0] * inv_hw); mgx[e] = (float)(sc[1] * inv_hw);
     }
@@ -355,8 +375,8 @@ in_bwd_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats,
 #pragma unroll
           for (int e = 0; e < W; ++e) {
             float xh = (t[e] - mean[e]) * rstd[e];
-            float gg = g[e] * act_grad_from_pre(xh, act);
-            t[e] = rstd[e] * (gg - mg[e] - xh * mgx[e]);
+            float gg = bwd_grad<AFFINE>(t[e], g[e], xh, scale[e], shift[e], act);
+            t[e] = scale[e] * (gg - mg[e] - xh * mgx[e]);
           }
           *reinterpret_cast<uint4*>(dx + base + vv * W) = raw_pack<T>(t);
         }
@@ -371,8 +391,7 @@ in_bwd_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats,
       c_cached = c0;
 #pragma unroll
       for (int e = 0; e < W; ++e) {
-        const double* st = stats + ((size_t)n * C + c0 + e) * 2;
-        finalize_stats(st[0], st[1], inv_hw, mean[e], rstd[e]);
+        bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, c0 + e, mean[e], rstd[e], scale[e], shift[e]);
         const double* sc = scratch + ((size_t)n * C + c0 + e) * 2;
         mg[e] = (float)(sc[0] * inv_hw); mgx[e] = (float)(sc[1] * inv_hw);
       }
@@ -387,8 +406,8 @@ in_bwd_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats,
 #pragma unroll
     for (int e = 0; e < W; ++e) {
       float xh = (t[e] - mean[e]) * rstd[e];
-      float gg = g[e] * act_grad_from_pre(xh, act);
-      t[e] = rstd[e] * (gg - mg[e] - xh * mgx[e]);
+      float gg = bwd_grad<AFFINE>(t[e], g[e], xh, scale[e], shift[e], act);
+      t[e] = scale[e] * (gg - mg[e] - xh * mgx[e]);
     }
     if constexpr (FAST) VecIO<Vec<T>::W>::st(dx + base + v * W, reinterpret_cast<float(&)[Vec<T>::W]>(t));
     else dx[base + v] = from_f<T>(t[0]);
@@ -456,20 +475,41 @@ int apply_impl(const T* x, const double* stats, int N, long long HW, int C, int 
 }
 
 template <typename T>
-int bwd_impl(const T* x, const double* stats, const T* dy, int N, long long HW, int C, int act,
-             double* scratch, T* dx, cudaStream_t st) {
+int bwd_reduce_impl(const T* x, const double* stats, const T* dy, int N, long long HW, int C, int act,
+                    const float* gamma, const float* beta, double* scratch, cudaStream_t st) {
   cudaMemsetAsync(scratch, 0, (size_t)N * C * 2 * sizeof(double), st);
   if (fast_ok<T>(C, HW)) {
     dim3 grid(blocks_per_image(N, HW * C / Vec<T>::W), N);
-    in_bwd_reduce_kernel<T, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, scratch);
-    in_bwd_apply_kernel<T, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, scratch, dx);
+    if (gamma) in_bwd_reduce_kernel<T, true, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, scratch);
+    else in_bwd_reduce_kernel<T, true, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, scratch);
   } else {
     dim3 grid(C, N);
-    in_bwd_reduce_kernel<T, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, scratch);
-    dim3 grid2(blocks_per_image(N, HW * C), N);
-    in_bwd_apply_kernel<T, false><<<grid2, TPB, 0, st>>>(x, stats, dy, HW, C, act, scratch, dx);
+    if (gamma) in_bwd_reduce_kernel<T, false, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, scratch);
+    else in_bwd_reduce_kernel<T, false, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, scratch);
   }
-  return check_launch("in_bwd kernels");
+  return check_launch("in_bwd_reduce_kernel");
+}
+
+template <typename T>
+int bwd_apply_impl(const T* x, const double* stats, const T* dy, int N, long long HW, int C, int act,
+                   const float* gamma, const float* beta, const double* scratch, T* dx, cudaStream_t st) {
+  if (fast_ok<T>(C, HW)) {
+    dim3 grid(blocks_per_image(N, HW * C / Vec<T>::W), N);
+    if (gamma) in_bwd_apply_kernel<T, true, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, scratch, dx);
+    else in_bwd_apply_kernel<T, true, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, scratch, dx);
+  } else {
+    dim3 grid(blocks_per_image(N, HW * C), N);
+    if (gamma) in_bwd_apply_kernel<T, false, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, scratch, dx);
+    else in_bwd_apply_kernel<T, false, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, scratch, dx);
+  }
+  return check_launch("in_bwd_apply_kernel");
+}
+
+template <typename T>
+int bwd_impl(const T* x, const double* stats, const T* dy, int N, long long HW, int C, int act,
+             double* scratch, T* dx, cudaStream_t st) {
+  int rc = bwd_reduce_impl<T>(x, stats, dy, N, HW, C, act, nullptr, nullptr, scratch, st);
+  return rc ? rc : bwd_apply_impl<T>(x, stats, dy, N, HW, C, act, nullptr, nullptr, scratch, dx, st);
 }
 
 }  // namespace
@@ -507,4 +547,33 @@ extern "C" int msg_instnorm_bwd(int dtype, const void* x, const double* stats, c
   if (dtype == MSG_BF16)
     return bwd_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, (const __nv_bfloat16*)dy, N, HW, C, act, scratch, (__nv_bfloat16*)dx, as_stream(stream));
   MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_bwd: bad dtype");
+}
+
+extern "C" int msg_instnorm_bwd_reduce(int dtype, const void* x, const double* stats, const void* dy, int N,
+                                       long long HW, int C, int act, const float* gamma, const float* beta,
+                                       double* sums, void* stream) {
+  MSG_REQUIRE(N > 0 && HW > 0 && C > 0, MSG_ERR_SHAPE, "instnorm_bwd_reduce: bad shape");
+  MSG_REQUIRE(act == MSG_ACT_NONE || act == MSG_ACT_RELU || act == MSG_ACT_LRELU, MSG_ERR_UNSUPPORTED, "instnorm_bwd_reduce: bad act");
+  MSG_REQUIRE((gamma == nullptr) == (beta == nullptr), MSG_ERR_SHAPE, "instnorm_bwd_reduce: gamma and beta go together");
+  if (dtype == MSG_F32)
+    return bwd_reduce_impl<float>((const float*)x, stats, (const float*)dy, N, HW, C, act, gamma, beta, sums, as_stream(stream));
+  if (dtype == MSG_BF16)
+    return bwd_reduce_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, (const __nv_bfloat16*)dy, N, HW, C, act, gamma, beta, sums,
+                                          as_stream(stream));
+  MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_bwd_reduce: bad dtype");
+}
+
+extern "C" int msg_instnorm_bwd_apply(int dtype, const void* x, const double* stats, const void* dy, int N,
+                                      long long HW, int C, int act, const float* gamma, const float* beta,
+                                      const double* sums, void* dx, void* stream) {
+  MSG_REQUIRE(N > 0 && HW > 0 && C > 0, MSG_ERR_SHAPE, "instnorm_bwd_apply: bad shape");
+  MSG_REQUIRE(act == MSG_ACT_NONE || act == MSG_ACT_RELU || act == MSG_ACT_LRELU, MSG_ERR_UNSUPPORTED, "instnorm_bwd_apply: bad act");
+  MSG_REQUIRE((gamma == nullptr) == (beta == nullptr), MSG_ERR_SHAPE, "instnorm_bwd_apply: gamma and beta go together");
+  if (dtype == MSG_F32)
+    return bwd_apply_impl<float>((const float*)x, stats, (const float*)dy, N, HW, C, act, gamma, beta, sums, (float*)dx,
+                                 as_stream(stream));
+  if (dtype == MSG_BF16)
+    return bwd_apply_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, (const __nv_bfloat16*)dy, N, HW, C, act, gamma, beta, sums,
+                                         (__nv_bfloat16*)dx, as_stream(stream));
+  MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_bwd_apply: bad dtype");
 }

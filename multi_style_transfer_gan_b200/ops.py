@@ -277,6 +277,39 @@ def instnorm_bwd(x, stats, dy, act=ACT_RELU, out=None, return_scratch=False):
     return (out, scratch) if return_scratch else out
 
 
+def _affine(gamma, beta, C):
+    if (gamma is None) != (beta is None):
+        raise _lib.MsgError("instnorm backward: gamma and beta go together")
+    if gamma is not None and not (gamma.dtype == beta.dtype == torch.float32 and gamma.numel() == beta.numel() == C
+                                  and gamma.is_contiguous() and beta.is_contiguous()):
+        raise _lib.MsgError(f"instnorm backward: gamma / beta must be contiguous float32 [{C}]")
+
+
+def instnorm_bwd_reduce(x, stats, dy, act=ACT_RELU, gamma=None, beta=None):
+    """First half of instnorm_bwd: the fp64 per-(n, c) sums [N, C, 2] = (sum g, sum g * xhat), g = dy * act'(z) with
+    z = xhat * gamma + beta (gamma / beta: optional fp32 [C]).  A synchronised BatchNorm all-reduces them (for a BatchNorm,
+    N = 1 view, the local sums are d(beta) and d(gamma)) and rescales them to the local count before instnorm_bwd_apply."""
+    _dev(x)
+    N, H, W, C = x.shape
+    _affine(gamma, beta, C)
+    sums = torch.empty((N, C, 2), device=x.device, dtype=torch.float64)
+    _lib.call("msg_instnorm_bwd_reduce", _dt(x), _p(x), _p(stats), _p(dy), N, H * W, C, act, _p(gamma), _p(beta), _p(sums),
+              _stream())
+    return sums
+
+
+def instnorm_bwd_apply(x, stats, dy, sums, act=ACT_RELU, gamma=None, beta=None, out=None):
+    """Second half of instnorm_bwd: dx = gamma * rstd * (g - sums[..., 0] / HW - xhat * sums[..., 1] / HW)."""
+    _dev(x)
+    N, H, W, C = x.shape
+    _affine(gamma, beta, C)
+    if out is None:
+        out = torch.empty_like(x)
+    _lib.call("msg_instnorm_bwd_apply", _dt(x), _p(x), _p(stats), _p(dy), N, H * W, C, act, _p(gamma), _p(beta), _p(sums),
+              _p(out), _stream())
+    return out
+
+
 # ---- LocalAttention core -------------------------------------------------------------------------
 def local_attn_fwd(qkv, ws=4):
     _dev(qkv)

@@ -9,32 +9,79 @@ in the same RNG order as the reference, so a seeded construction is bit-identica
 Kernels: the same conv / convT engines as the EnhancedGenerator (tcgen05 where Cin % 64 == 0).  BatchNorm over
 (N, H, W) of an NHWC tensor IS InstanceNorm of the [1, N*H, W, C] view, so it reuses the IN machinery: statistics come
 from the conv epilogue (summed over the batch), the apply kernel carries gamma / beta through its per-style affine
-path, and the backward kernel's per-channel reductions (sum g, sum g*xhat) are exactly d(beta), d(gamma).  Running
-statistics follow torch.nn.BatchNorm2d (momentum 0.1, unbiased variance for the running estimate).  Training is
-data-parallel-incompatible without SyncBN (batch statistics couple samples): replicas only, see DESIGN.md 6.
+path, and the backward is two kernels, msg_instnorm_bwd_reduce -> msg_instnorm_bwd_apply with the affine, whose
+per-channel reductions (sum g, sum g*xhat) are exactly d(beta), d(gamma).  Running statistics follow torch.nn.BatchNorm2d
+(momentum 0.1, unbiased variance for the running estimate).
+
+Data-parallel training: convert with torch.nn.SyncBatchNorm.convert_sync_batchnorm and wrap in DistributedDataParallel.
+In train mode each SyncBatchNorm whose process group has more than one rank all-reduces its batch sums and element count in
+the forward and its (sum g, sum g*xhat) between the two backward kernels, so N ranks of B/N images compute the step of one
+process on B images (DESIGN.md 6).  d(gamma), d(beta) stay the local sums, which DDP averages.  DDP waits for a gradient of
+every parameter: the engine returns all of them, including the analytically-zero ones of the conv biases in front of a
+BatchNorm.  Plain BatchNorm2d layers, eval mode and a group of one rank exchange nothing.
 """
 import torch
+import torch.distributed as dist
 import torch.nn as nn
 
 from . import ops
 from .generator_engine import _pad_dim
 from .losses import l1
-from .ops import ACT_LRELU, ACT_NONE, ACT_RELU, ACT_TANH, ConvGeom
+from .ops import ACT_LRELU, ACT_RELU, ACT_TANH, ConvGeom
 
 ENC = ((0, None), (2, 3), (5, 6), (8, 9))      # (conv index, BatchNorm index) inside `encoder`  (pretrain.py:65-77)
 DEC = ((0, 1), (3, 4), (6, 7), (9, None))      # (convT index, BatchNorm index) inside `decoder` (pretrain.py:80-91)
-BN_EPS, BN_MOMENTUM = 1e-5, 0.1
+BN_MOMENTUM = 0.1                              # eps 1e-5 is the IN kernels' (kInEps, csrc/common.cuh)
 
 
 def _edge_pad(dtype):
     return 4 if dtype == torch.float32 else 8
 
 
-def _unit_stats(M, C, device):
-    """Raw sums that make the IN apply kernel a pure per-channel affine: mean 0, var + eps = 1."""
-    st = torch.zeros((1, C, 2), device=device, dtype=torch.float64)
-    st[0, :, 1] = M * (1.0 - BN_EPS)
-    return st
+def bn_batch_stats(st, M, rm, rv, nbt, group=None):
+    """Train-mode statistics of one BatchNorm layer, and the torch.nn.BatchNorm2d running-statistics update (momentum 0.1,
+    unbiased variance).  Pure torch, no kernel: st holds the conv epilogue's per-image fp64 sums [N, C, 2] = (sum x,
+    sum x^2) over this rank's M = N*H*W elements.
+
+    group: None for a plain BatchNorm.  Otherwise the process group of a SyncBatchNorm: the batch sums and the element
+    count, [2*C + 1] fp64, are summed over it by one all-reduce, the running statistics follow the global mean and the
+    unbiased global variance (identical on every rank), and the returned sums are the global sums scaled by M / M_global,
+    the local count the kernels normalise by (include/msg_b200.h).
+
+    Returns (sums [1, C, 2] fp64, M / M_global as a 0-dim fp64 tensor, or None without a group)."""
+    C = st.shape[1]
+    stb = st.sum(0, keepdim=True)
+    if group is None:
+        Mg, unbias, scale = M, M / max(M - 1, 1), None
+    else:
+        buf = torch.cat([stb.reshape(-1), stb.new_full((1,), float(M))])
+        dist.all_reduce(buf, group=group)
+        stb, Mg = buf[:-1].view(1, C, 2), buf[-1]
+        unbias, scale = Mg / (Mg - 1).clamp_min(1.0), M / Mg
+    with torch.no_grad():
+        mean = stb[0, :, 0] / Mg
+        var = (stb[0, :, 1] / Mg - mean * mean).clamp_min(0.0)
+        rm.mul_(1 - BN_MOMENTUM).add_((BN_MOMENTUM * mean).to(rm.dtype))
+        rv.mul_(1 - BN_MOMENTUM).add_((BN_MOMENTUM * var * unbias).to(rv.dtype))
+        nbt.add_(1)
+    if scale is not None:
+        stb = stb * scale
+    return stb.contiguous(), scale
+
+
+def bn_sync_groups(model):
+    """BatchNorm name -> the process group its batch statistics are reduced over: the ``SyncBatchNorm`` layers of a
+    model whose group (``process_group``, None meaning WORLD) has more than one rank.  Plain BatchNorm2d layers, and every
+    layer when torch.distributed is not initialised, are absent: they normalise over the local batch."""
+    if not (dist.is_available() and dist.is_initialized()):
+        return {}
+    out = {}
+    for name, m in model.named_modules():
+        if isinstance(m, nn.SyncBatchNorm):
+            group = m.process_group if m.process_group is not None else dist.group.WORLD
+            if dist.get_world_size(group) > 1:
+                out[name] = group
+    return out
 
 
 class _Engine:
@@ -47,17 +94,12 @@ class _Engine:
 
     # ---- BatchNorm = InstanceNorm of the [1, N*H, W, C] view -------------------------------------------
     @staticmethod
-    def _bn_fwd(y, st, gamma, beta, rm, rv, nbt, act, training):
+    def _bn_fwd(y, st, gamma, beta, rm, rv, nbt, act, training, group):
         N, H, W, C = y.shape
         M = N * H * W
+        scale = None
         if training:
-            stb = st.sum(0, keepdim=True).contiguous()                       # batch sums [1, C, 2] (fp64)
-            with torch.no_grad():                                            # torch.nn.BatchNorm2d bookkeeping
-                mean = stb[0, :, 0] / M
-                var = (stb[0, :, 1] / M - mean * mean).clamp_min(0.0)
-                rm.mul_(1 - BN_MOMENTUM).add_((BN_MOMENTUM * mean).to(rm.dtype))
-                rv.mul_(1 - BN_MOMENTUM).add_((BN_MOMENTUM * var * (M / max(M - 1, 1))).to(rv.dtype))
-                nbt.add_(1)
+            stb, scale = bn_batch_stats(st, M, rm, rv, nbt, group)
         else:
             stb = torch.empty((1, C, 2), device=y.device, dtype=torch.float64)
             stb[0, :, 0] = rm.double() * M
@@ -65,24 +107,27 @@ class _Engine:
         one = torch.ones(1, device=y.device, dtype=torch.float32)
         out = ops.instnorm_apply(y.view(1, N * H, W, C), stb, act, gammas=gamma.detach().float().view(1, C).contiguous(),
                                  betas=beta.detach().float().view(1, C).contiguous(), w=one)
-        return out.view(N, H, W, C), stb
+        return out.view(N, H, W, C), stb, scale
 
     @staticmethod
-    def _bn_bwd(y, stb, a_out, da_out, gamma, act):
-        """y: pre-norm conv output, a_out = act(gamma * xhat + beta), da_out its gradient.
-        Returns (d y, d gamma, d beta)."""
+    def _bn_bwd(y, stb, da_out, gamma, beta, act, group, scale):
+        """y: pre-norm conv output, da_out: gradient of act(gamma * xhat + beta).  reduce -> [all-reduce] -> apply.
+        Returns (d y, d gamma, d beta); d gamma and d beta are this rank's sums, taken before the all-reduce: DDP averages
+        them like every other parameter gradient (as torch.nn.SyncBatchNorm does)."""
         N, H, W, C = y.shape
-        g = ops.act_bwd(a_out, da_out, act)                                   # through the activation (sign of the output)
-        dx, scratch = ops.instnorm_bwd(y.view(1, N * H, W, C), stb, g.view(1, N * H, W, C), ACT_NONE, return_scratch=True)
-        dbeta, dgamma = scratch[0, :, 0].float(), scratch[0, :, 1].float()    # sum g, sum g * xhat
-        one = torch.ones(1, device=y.device, dtype=torch.float32)
-        zero = torch.zeros((1, C), device=y.device, dtype=torch.float32)
-        dy = ops.instnorm_apply(dx, _unit_stats(N * H * W, C, y.device), ACT_NONE,       # dx * gamma[c], our own kernel
-                                gammas=gamma.detach().float().view(1, C).contiguous(), betas=zero, w=one)
+        x, g = y.view(1, N * H, W, C), da_out.view(1, N * H, W, C)
+        gam, bet = gamma.detach().float().contiguous(), beta.detach().float().contiguous()
+        sums = ops.instnorm_bwd_reduce(x, stb, g, act, gam, bet)                    # (sum g, sum g * xhat)
+        dbeta, dgamma = sums[0, :, 0].float(), sums[0, :, 1].float()
+        if group is not None:
+            dist.all_reduce(sums, group=group)
+            sums.mul_(scale)                                                        # normalised to the local count
+        dy = ops.instnorm_bwd_apply(x, stb, g, sums, act, gam, bet)
         return dy.view(N, H, W, C), dgamma, dbeta
 
     # ---- forward -----------------------------------------------------------------------------------------
-    def forward(self, P, B, x, dtype, training, save):
+    def forward(self, P, B, x, dtype, training, save, groups):
+        """groups: bn_sync_groups of the model (train mode only)."""
         pad = _edge_pad(dtype)
         a = ops.nchw_to_nhwc(x, dtype, pad)
         tape = []
@@ -102,9 +147,10 @@ class _Engine:
                 st = ops.new_stats(a.shape[0], cout, a.device)
                 y = g.forward(a, wp, bias, stats=st)
                 pre = f"encoder.{bi}"
-                an, stb = self._bn_fwd(y, st, P[pre + ".weight"], P[pre + ".bias"], B[pre + ".running_mean"],
-                                       B[pre + ".running_var"], B[pre + ".num_batches_tracked"], ACT_LRELU, training)
-                tape.append(("conv_bn", f"encoder.{ci}", pre, g, w, a, y, stb, an, ACT_LRELU))
+                an, stb, scale = self._bn_fwd(y, st, P[pre + ".weight"], P[pre + ".bias"], B[pre + ".running_mean"],
+                                              B[pre + ".running_var"], B[pre + ".num_batches_tracked"], ACT_LRELU, training,
+                                              groups.get(pre))
+                tape.append(("conv_bn", f"encoder.{ci}", pre, g, w, a, y, (stb, groups.get(pre), scale), an, ACT_LRELU))
                 a = an
         out = None
         for li, (ci, bi) in enumerate(DEC):
@@ -125,9 +171,10 @@ class _Engine:
                 st = ops.new_stats(a.shape[0], cout, a.device)
                 y = g.forward(a, wp, bias, stats=st)
                 pre = f"decoder.{bi}"
-                an, stb = self._bn_fwd(y, st, P[pre + ".weight"], P[pre + ".bias"], B[pre + ".running_mean"],
-                                       B[pre + ".running_var"], B[pre + ".num_batches_tracked"], ACT_RELU, training)
-                tape.append(("convT_bn", f"decoder.{ci}", pre, g, w, a, y, stb, an, ACT_RELU))
+                an, stb, scale = self._bn_fwd(y, st, P[pre + ".weight"], P[pre + ".bias"], B[pre + ".running_mean"],
+                                              B[pre + ".running_var"], B[pre + ".num_batches_tracked"], ACT_RELU, training,
+                                              groups.get(pre))
+                tape.append(("convT_bn", f"decoder.{ci}", pre, g, w, a, y, (stb, groups.get(pre), scale), an, ACT_RELU))
                 a = an
         return out[:, :3].contiguous(), (tape if save else None), out
 
@@ -136,9 +183,9 @@ class _Engine:
         pad = _edge_pad(dtype)
         G = {}
         d = ops.tanh_bwd_nchw(y_full[:, :3].contiguous(), dy.float().contiguous(), dtype, pad)   # [N, H, W, pad]
-        for kind, cname, bname, g, w, a_in, y, stb, a_out, act in reversed(tape):
+        for kind, cname, bname, g, w, a_in, y, bn, a_out, act in reversed(tape):
             if kind in ("conv_bn", "convT_bn"):
-                d, dgamma, dbeta = self._bn_bwd(y, stb, a_out, d, P[bname + ".weight"], act)
+                d, dgamma, dbeta = self._bn_bwd(y, bn[0], d, P[bname + ".weight"], P[bname + ".bias"], act, bn[1], bn[2])
                 G[bname + ".weight"], G[bname + ".bias"] = dgamma, dbeta
             elif kind == "conv_act":
                 d = ops.act_bwd(a_out, d, act)
@@ -164,7 +211,8 @@ class _PretrainFn(torch.autograd.Function):
         if need and not training:
             raise NotImplementedError("pretrain.Generator (msg_b200): backward is implemented for train() mode "
                                       "(batch statistics); use no_grad for eval-mode inference")
-        y, tape, y_full = model._engine.forward(P, dict(model.named_buffers()), x, dtype, training, need)
+        groups = bn_sync_groups(model) if training else {}
+        y, tape, y_full = model._engine.forward(P, dict(model.named_buffers()), x, dtype, training, need, groups)
         if need:
             ctx.model, ctx.dtype, ctx.keys, ctx.tape, ctx.y_full = model, dtype, keys, tape, y_full
             ctx.save_for_backward(*params)
