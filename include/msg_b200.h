@@ -100,6 +100,35 @@ int msg_conv2d(const msg_conv_desc* d, const void* x, const void* w, const float
 int msg_conv2d_path(const msg_conv_desc* d, const void* x, const void* w, const void* y);
 
 /* ---------------------------------------------------------------------------------------------
+ * InstanceNorm affine of a style-conditional generator.  Every site that applies an InstanceNorm
+ * (the stand-alone apply, and the convs / stages below that normalise their input on load) can
+ * take an optional affine, passed as (gamma, beta, img_stride), fp32:
+ *   gamma[n * img_stride + c] is indexed exactly like the statistics it accompanies (channel
+ *   offsets ci_off / cs_off included); img_stride 0 is one [C] affine for the whole batch;
+ *   gamma = beta = NULL is no affine (the entry points without the _affine suffix pass NULL).
+ * The apply is z = fmaf(x, scale, shift), scale = rstd * gamma[..], shift = beta[..] - mean * scale,
+ * so gamma = 1, beta = 0 gives the affine-free result bit for bit.
+ * ------------------------------------------------------------------------------------------- */
+/* msg_conv2d with an input affine for MSG_CONV_IN_NORM.  Only the TMA + tcgen05 kernel applies one
+ * (msg_conv2d_path == 2): a descriptor that would run on another engine returns MSG_ERR_SHAPE. */
+int msg_conv2d_affine(const msg_conv_desc* d, const void* x, const void* w, const float* bias, void* y, double* stats,
+                      const double* in_stats, const float* in_gamma, const float* in_beta, int in_img_stride, void* stream);
+/* Per-image affine tables of all the normalisation sites of a forward in one launch:
+ *   gamma_out[n][c] = sum_s w[n][s] * gammas[s][c]  (beta alike), c < Ct,
+ * an fmaf chain over s in ascending order starting from 0 -- the chain msg_instnorm_apply runs
+ * over its w[S], so a row equals that apply's blended affine bit for bit.
+ * w fp32 [N][S] (weights used as given, no normalisation); gammas, betas fp32 [S][Ct];
+ * gamma_out, beta_out fp32 [N][Ct]. */
+int msg_style_affine(const float* w, int N, int S, const float* gammas, const float* betas, int Ct, float* gamma_out,
+                     float* beta_out, void* stream);
+/* Backward of msg_style_affine for one sums arena [N][Ct][2] fp64 (the per-(image, channel)
+ * (sum g, sum g * xhat) = (d beta_n, d gamma_n) of msg_instnorm_bwd_reduce_affine):
+ *   dgammas[s][c] += sum_n w[n][s] * sums[n][c][1],  dbetas[s][c] += sum_n w[n][s] * sums[n][c][0]
+ * (fp64 sum over n in ascending order, one fp32 add).  dgammas, dbetas fp32 [S][Ct]. */
+int msg_style_affine_bwd(const double* sums, const float* w, int N, int S, int Ct, float* dgammas, float* dbetas,
+                         void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * "Row-slab" convolution (bf16, W % 8 == 0): stride-1, same-size convs with small N, several taps
  * sharing one input row slab -- the 7x7 convs (enhanced_generator.py:92,137) and the fused
  * MultiScaleBlock branches (:52-71, one launch writes the concatenated tensor).  A k-block is an
@@ -214,6 +243,11 @@ int msg_instnorm_stats(int dtype, const void* x, int N, long long HW, int C, dou
 int msg_instnorm_apply(int dtype, const void* x, const double* stats, int N, long long HW, int C,
                        int act, const void* residual, int S, const float* gammas,
                        const float* betas, const float* w, void* y, void* stream);
+/* msg_instnorm_apply with an affine table (gamma, beta, img_stride) instead of the blend; S > 0
+ * together with a table is refused.  msg_instnorm_apply is this with a NULL table. */
+int msg_instnorm_apply_affine(int dtype, const void* x, const double* stats, int N, long long HW, int C, int act,
+                              const void* residual, int S, const float* gammas, const float* betas, const float* w,
+                              const float* gamma, const float* beta, int img_stride, void* y, void* stream);
 /* backward of y = act(IN(x)) [+ residual]:  given dy, x (pre-norm) and stats, writes dx.
  * (d residual = dy is the caller's business.)  scratch: fp64 [N][C][2], zeroed by the callee. */
 int msg_instnorm_bwd(int dtype, const void* x, const double* stats, const void* dy, int N,
@@ -237,6 +271,16 @@ int msg_instnorm_bwd_reduce(int dtype, const void* x, const double* stats, const
 int msg_instnorm_bwd_apply(int dtype, const void* x, const double* stats, const void* dy, int N,
                            long long HW, int C, int act, const float* gamma, const float* beta,
                            const double* sums, void* dx, void* stream);
+/* The same with a per-image affine (gamma, beta, img_stride): the reductions of image n are then
+ * d beta_n and d gamma_n.  With img_stride > 0 the sums rows are img_stride apart as well
+ * (sums [N][img_stride][2], the columns of this call written, the others untouched), so the calls
+ * of one backward fill one arena laid out like the affine tables.  The functions above are these
+ * with img_stride 0. */
+int msg_instnorm_bwd_reduce_affine(int dtype, const void* x, const double* stats, const void* dy, int N, long long HW, int C,
+                                   int act, const float* gamma, const float* beta, int img_stride, double* sums, void* stream);
+int msg_instnorm_bwd_apply_affine(int dtype, const void* x, const double* stats, const void* dy, int N, long long HW, int C,
+                                  int act, const float* gamma, const float* beta, int img_stride, const double* sums, void* dx,
+                                  void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * LocalAttention core (enhanced_generator.py:22-35) on a [N,H,W,3C] qkv map (the 1x1 qkv conv is
@@ -270,6 +314,10 @@ int msg_la_stage_set_trace(void* buf);
 int msg_la_stage_fwd(int dtype, const void* x, const double* in_stats, int in_act, const void* wqkv,
                      const float* bqkv, const void* wproj, const float* bproj, int N, int H, int W, int C,
                      void* out, void* stream);
+/* with an affine (in_gamma, in_beta, in_img_stride) of the fused input norm (needs in_stats) */
+int msg_la_stage_fwd_affine(int dtype, const void* x, const double* in_stats, const float* in_gamma, const float* in_beta,
+                            int in_img_stride, int in_act, const void* wqkv, const float* bqkv, const void* wproj,
+                            const float* bproj, int N, int H, int W, int C, void* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * layout / image helpers
@@ -358,6 +406,10 @@ typedef struct {
 } msg_out7_ring_desc;
 int msg_out7_ring(const msg_out7_ring_desc* d, const void* f, const double* in_stats, const void* residual,
                   const void* w_stacks, const float* bias, float* y, void* stream);
+/* with an affine (in_gamma, in_beta, in_img_stride) of f's norm, indexed like in_stats */
+int msg_out7_ring_affine(const msg_out7_ring_desc* d, const void* f, const double* in_stats, const float* in_gamma,
+                         const float* in_beta, int in_img_stride, const void* residual, const void* w_stacks, const float* bias,
+                         float* y, void* stream);
 
 /* First down-sampling conv of the encoder, Conv2d(64, Cout, 4, stride 2, padding 1) (enhanced_generator.py:99-104), optionally fused
  * with the InstanceNorm + ReLU in front of it (in_stats != NULL: x is the RAW output of the previous conv and in_stats its plane sums),
@@ -374,6 +426,10 @@ typedef struct {
 } msg_down_ring_desc;
 int msg_down_ring(const msg_down_ring_desc* d, const void* x, const double* in_stats, const void* w_stacks, const float* bias,
                   void* y, double* stats, void* stream);
+/* with an affine (in_gamma, in_beta, in_img_stride) of the fused input norm (needs in_stats), indexed like in_stats */
+int msg_down_ring_affine(const msg_down_ring_desc* d, const void* x, const double* in_stats, const float* in_gamma,
+                         const float* in_beta, int in_img_stride, const void* w_stacks, const float* bias, void* y,
+                         double* stats, void* stream);
 
 /* uint8 pre-processing on the device (batch_process_images.py:193-205, 287-291): paste the [N,h,w,3] uint8 images (PIL layout) at
  * (off_y, off_x) on an HxW canvas filled with `fill` (the reference's white canvas), then ToTensor + Normalize(0.5, 0.5):

@@ -93,6 +93,9 @@ SIGNATURES = {
     "msg_sm_count": [],
     "msg_conv2d": [ctypes.POINTER(ConvDesc), _P, _P, _P, _P, _P, _P, _P],
     "msg_conv2d_path": [ctypes.POINTER(ConvDesc), _P, _P, _P],
+    "msg_conv2d_affine": [ctypes.POINTER(ConvDesc), _P, _P, _P, _P, _P, _P, _P, _P, c_int, _P],
+    "msg_style_affine": [_P, c_int, c_int, _P, _P, c_int, _P, _P, _P],
+    "msg_style_affine_bwd": [_P, _P, c_int, c_int, c_int, _P, _P, _P],
     "msg_conv2d_wgrad": [ctypes.POINTER(ConvDesc), _P, _P, _P, _P],
     "msg_conv_slab": [ctypes.POINTER(SlabDesc), _P, _P, _P, _P, _P, _P],
     "msg_conv_shift": [ctypes.POINTER(ShiftDesc), _P, _P, _P, _P, _P, _P],
@@ -104,11 +107,15 @@ SIGNATURES = {
     "msg_instnorm_bwd": [c_int, _P, _P, _P, c_int, c_ll, c_int, c_int, _P, _P, _P],
     "msg_instnorm_bwd_reduce": [c_int, _P, _P, _P, c_int, c_ll, c_int, c_int, _P, _P, _P, _P],
     "msg_instnorm_bwd_apply": [c_int, _P, _P, _P, c_int, c_ll, c_int, c_int, _P, _P, _P, _P, _P],
+    "msg_instnorm_apply_affine": [c_int, _P, _P, c_int, c_ll, c_int, c_int, _P, c_int, _P, _P, _P, _P, _P, c_int, _P, _P],
+    "msg_instnorm_bwd_reduce_affine": [c_int, _P, _P, _P, c_int, c_ll, c_int, c_int, _P, _P, c_int, _P, _P],
+    "msg_instnorm_bwd_apply_affine": [c_int, _P, _P, _P, c_int, c_ll, c_int, c_int, _P, _P, c_int, _P, _P, _P],
     "msg_local_attn_fwd": [c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "msg_local_attn_bwd": [c_int, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "msg_la_stage_set_trace": [_P],
     "msg_la_stage_supported": [c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P],
     "msg_la_stage_fwd": [c_int, _P, _P, c_int, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P, _P],
+    "msg_la_stage_fwd_affine": [c_int, _P, _P, _P, _P, c_int, c_int, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P, _P],
     "msg_nchw_to_nhwc": [c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "msg_nhwc_to_nchw": [c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "msg_blend_outputs": [ctypes.POINTER(_P), ctypes.POINTER(c_float), c_int, _P, c_float, c_float,
@@ -123,6 +130,8 @@ SIGNATURES = {
     "msg_convt_ring": [ctypes.POINTER(ConvtRingDesc), _P, _P, _P, _P, _P, _P],
     "msg_out7_ring": [ctypes.POINTER(Out7RingDesc), _P, _P, _P, _P, _P, _P, _P],
     "msg_down_ring": [ctypes.POINTER(DownRingDesc), _P, _P, _P, _P, _P, _P, _P],
+    "msg_out7_ring_affine": [ctypes.POINTER(Out7RingDesc), _P, _P, _P, _P, c_int, _P, _P, _P, _P, _P],
+    "msg_down_ring_affine": [ctypes.POINTER(DownRingDesc), _P, _P, _P, _P, c_int, _P, _P, _P, _P, _P],
     "msg_u8_canvas_to_nchw": [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P],
     "msg_u8_strength_blend": [_P, _P, c_int, c_int, c_int, ctypes.c_double, _P, _P],
     "msg_adam_step": [_P, _P, _P, _P, c_ll, c_float, c_float, c_float, c_float, c_int, c_float, _P],

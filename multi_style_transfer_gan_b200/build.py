@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libmsg_b200.so")
 SOURCES = ["api.cu", "conv_simt.cu", "conv_tc.cu", "conv_tma.cu", "conv_slab.cu", "conv_shift.cu", "msb_ring.cu", "convt_ring.cu", "out7_ring.cu", "down_ring.cu", "conv_wgrad_tc.cu", "instnorm.cu", "local_attn.cu", "local_attn_tc.cu", "local_attn_bwd_tc.cu", "la_stage.cu",
-           "elementwise.cu", "blend_maps.cu", "gram.cu"]
+           "elementwise.cu", "blend_maps.cu", "gram.cu", "style_affine.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
          "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

@@ -47,7 +47,7 @@ int conv2d_simt(const msg_conv_desc* d, const void* x, const void* w, const floa
                 double* stats, const double* in_stats, cudaStream_t st);
 bool conv2d_tma_supported(const msg_conv_desc* d, const void* x, const void* w, const void* y);
 int conv2d_tma(const msg_conv_desc* d, const void* x, const void* w, const float* bias, void* y,
-               double* stats, const double* in_stats, cudaStream_t st);
+               double* stats, const double* in_stats, const float* in_gamma, const float* in_beta, int in_img_stride, cudaStream_t st);
 bool conv2d_tc_supported(const msg_conv_desc* d, const void* x, const void* w, const void* y);
 int conv2d_tc(const msg_conv_desc* d, const void* x, const void* w, const float* bias, void* y,
               double* stats, const double* in_stats, cudaStream_t st);
@@ -65,7 +65,7 @@ int conv2d_dispatch(const msg_conv_desc* d, const void* x, const void* w, const 
     if (!(d->flags & MSG_CONV_FORCE_GATHER) && conv2d_dot_supported(d, x, w))
       return conv2d_dot(d, x, w, bias, y, st);                              // one useful GEMM column: warp-per-pixel dot products
     if (!(d->flags & MSG_CONV_FORCE_GATHER) && conv2d_tma_supported(d, x, w, y))
-      return conv2d_tma(d, x, w, bias, y, stats, in_stats, st);            // persistent TMA + tcgen05 kernel
+      return conv2d_tma(d, x, w, bias, y, stats, in_stats, nullptr, nullptr, 0, st);   // persistent TMA + tcgen05 kernel
     MSG_REQUIRE(!(d->flags & MSG_CONV_PER_IMAGE_W), MSG_ERR_UNSUPPORTED,
                 "conv: MSG_CONV_PER_IMAGE_W needs the TMA kernel (bf16, Cin % 64 == 0, plane a multiple of 128 pixels)");
     if (conv2d_tc_supported(d, x, w, y))
@@ -103,7 +103,23 @@ extern "C" int msg_conv2d_path(const msg_conv_desc* d, const void* x, const void
   return 0;
 }
 
+extern "C" int msg_conv2d_affine(const msg_conv_desc* d, const void* x, const void* w, const float* bias, void* y, double* stats,
+                                 const double* in_stats, const float* in_gamma, const float* in_beta, int in_img_stride, void* stream) {
+  if (in_gamma == nullptr && in_beta == nullptr) return conv2d_dispatch(d, x, w, bias, y, stats, in_stats, as_stream(stream));
+  // only the TMA kernel's transform warps apply an input affine: every other engine refuses one instead of dropping it
+  MSG_REQUIRE(d != nullptr, MSG_ERR_SHAPE, "conv: null descriptor");
+  int rc = conv_validate(d);
+  if (rc) return rc;
+  MSG_REQUIRE(in_gamma && in_beta && in_img_stride >= 0 && (d->flags & MSG_CONV_IN_NORM) && in_stats != nullptr, MSG_ERR_SHAPE,
+              "conv: an input affine needs gamma, beta and MSG_CONV_IN_NORM with in_stats");
+  MSG_REQUIRE(!(d->flags & MSG_CONV_STATS) || stats != nullptr, MSG_ERR_SHAPE, "conv: MSG_CONV_STATS without a stats buffer");
+  MSG_REQUIRE(!(d->flags & (MSG_CONV_FORCE_SIMT | MSG_CONV_FORCE_GATHER)) && !conv2d_dot_supported(d, x, w) &&
+              conv2d_tma_supported(d, x, w, y), MSG_ERR_SHAPE,
+              "conv: an input affine runs only on the TMA kernel (bf16 1x1, Cin %% 64 == 0, tiles inside one image)");
+  return conv2d_tma(d, x, w, bias, y, stats, in_stats, in_gamma, in_beta, in_img_stride, as_stream(stream));
+}
+
 extern "C" int msg_conv2d(const msg_conv_desc* d, const void* x, const void* w, const float* bias,
                           void* y, double* stats, const double* in_stats, void* stream) {
-  return conv2d_dispatch(d, x, w, bias, y, stats, in_stats, as_stream(stream));
+  return msg_conv2d_affine(d, x, w, bias, y, stats, in_stats, nullptr, nullptr, 0, stream);
 }

@@ -122,6 +122,24 @@ __device__ __forceinline__ void finalize_stats(double s, double ss, double inv_h
   rstd = (float)(1.0 / sqrt(var + (double)kInEps));
 }
 
+// The one place that turns statistics and an affine into the constants every InstanceNorm apply site uses,
+// z = fmaf(x, scale, shift):  scale = rstd * gamma,  shift = beta - mean * scale.
+// gamma = 1, beta = 0 (no affine) gives scale = rstd and shift = -mean * rstd bit for bit.
+__device__ __forceinline__ void in_scale_shift(const double* st, double inv_hw, float gamma, float beta,
+                                               float& mean, float& rstd, float& scale, float& shift) {
+  finalize_stats(st[0], st[1], inv_hw, mean, rstd);
+  scale = rstd * gamma;
+  shift = beta - mean * scale;
+}
+
+// An affine is passed as (gamma, beta, img_stride): element ai = n * img_stride + c is indexed like the statistics it
+// accompanies (channel offsets included); img_stride 0 is one [C] affine for the whole batch; a null gamma is no affine.
+__device__ __forceinline__ void in_affine(const float* gamma, const float* beta, size_t ai, float& g, float& b) {
+  g = 1.f;
+  b = 0.f;
+  if (gamma != nullptr) { g = gamma[ai]; b = beta[ai]; }
+}
+
 int sm_count();
 
 // once-per-device latch for cudaFuncSetAttribute (a function attribute belongs to the current device's context, so a

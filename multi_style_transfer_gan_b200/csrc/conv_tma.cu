@@ -49,6 +49,9 @@ struct TmaParams {
   double* stats;
   int BN, n_tiles, m_tiles, stages, tmem_cols;
   const double* in_stats;   // MSG_CONV_IN_NORM: raw plane sums [N][Ci_total][2] of the INPUT tensor
+  const float* in_gamma;    // MSG_CONV_IN_NORM: optional affine of the input norm (common.cuh: in_affine), or null
+  const float* in_beta;
+  int in_img_stride;
   int xform;          // 1: four transform warps apply InstanceNorm + activation to every A tile in smem (1x1 convs)
   int b_resident;     // 1: all nkb weight tiles of the (single) N tile stay in smem for the whole kernel
   int epi_groups;     // 1: warps 2-5 drain both accumulator buffers; 2: warps 2-5 own buffer 0, warps 6-9 buffer 1
@@ -212,11 +215,10 @@ conv_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
       if (img != cur_img) {                                      // new image: rebuild the per-channel table
         asm volatile("bar.sync 2, 128;" ::: "memory");           // everyone is done reading the old table
         for (int ci = xt; ci < d.Cin; ci += 128) {
-          const double* st = p.in_stats + ((size_t)img * d.Ci_total + d.ci_off + ci) * 2;
-          float mean, rstd;
-          finalize_stats(st[0], st[1], inv_hw, mean, rstd);
-          xf_tab[ci] = rstd;
-          xf_tab[512 + ci] = 0.f - mean * rstd;
+          const int c = d.ci_off + ci;
+          float g, b, mean, rstd;
+          in_affine(p.in_gamma, p.in_beta, (size_t)img * p.in_img_stride + c, g, b);
+          in_scale_shift(p.in_stats + ((size_t)img * d.Ci_total + c) * 2, inv_hw, g, b, mean, rstd, xf_tab[ci], xf_tab[512 + ci]);
         }
         asm volatile("bar.sync 2, 128;" ::: "memory");
         cur_img = img; cur_cb = -1;
@@ -536,13 +538,14 @@ bool conv2d_tma_supported(const msg_conv_desc* d, const void* x, const void* w, 
 }
 
 int conv2d_tma(const msg_conv_desc* d, const void* x, const void* w, const float* bias, void* y,
-               double* stats, const double* in_stats, cudaStream_t st) {
+               double* stats, const double* in_stats, const float* in_gamma, const float* in_beta, int in_img_stride, cudaStream_t st) {
   EncodeTiledFn enc = get_encode();
   MSG_REQUIRE(enc != nullptr, MSG_ERR_CUDA, "conv_tma: cuTensorMapEncodeTiled unavailable");
   Tiling tl;
   MSG_REQUIRE(pick_tiling(d, &tl), MSG_ERR_UNSUPPORTED, "conv_tma: unsupported plane geometry");
   TmaParams p;
   p.d = *d; p.bias = bias; p.y = y; p.stats = stats; p.in_stats = in_stats;
+  p.in_gamma = in_gamma; p.in_beta = in_beta; p.in_img_stride = in_img_stride;
   p.xform = (d->flags & MSG_CONV_IN_NORM) ? 1 : 0;
   p.BN = pick_bn(d->Cout);
   p.n_tiles = (d->Cout + p.BN - 1) / p.BN;

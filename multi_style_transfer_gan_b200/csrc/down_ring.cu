@@ -52,6 +52,9 @@ struct DnParams {
   double* stats;
   const double* in_stats;               // [N][Cs_total][2] raw plane sums of x, or null (x is used as it is)
   int Cs_total, cs_off;
+  const float* in_gamma;                // optional affine of the input norm (common.cuh: in_affine), or null
+  const float* in_beta;
+  int in_img_stride;
 };
 
 __global__ void __launch_bounds__(NTHREADS, 1)
@@ -154,7 +157,7 @@ down_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     SlabRing ring(bars.S);
     for (Walk pc = pieces; pc.next();) {
       if (xform && pc.img != cur_img) {
-        load_scale_shift(p.in_stats, pc.img, p.Cs_total, p.cs_off, lchunk, inv_hw, sc, sh);
+        load_scale_shift(p.in_stats, p.in_gamma, p.in_beta, p.in_img_stride, pc.img, p.Cs_total, p.cs_off, lchunk, inv_hw, sc, sh);
         cur_img = pc.img;
       }
       const int r_lo = pc.r0 < 0 ? 0 : pc.r0, r_hi = pc.r1 > p.H ? p.H : pc.r1;
@@ -208,8 +211,9 @@ down_ring_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
 
 using namespace msg;
 
-extern "C" int msg_down_ring(const msg_down_ring_desc* d, const void* x, const double* in_stats, const void* w_stacks, const float* bias,
-                             void* y, double* stats, void* stream) {
+extern "C" int msg_down_ring_affine(const msg_down_ring_desc* d, const void* x, const double* in_stats, const float* in_gamma,
+                                    const float* in_beta, int in_img_stride, const void* w_stacks, const float* bias, void* y, double* stats,
+                                    void* stream) {
   cudaStream_t st = as_stream(stream);
   MSG_REQUIRE(d != nullptr && x && w_stacks && y, MSG_ERR_SHAPE, "down_ring: null argument");
   MSG_REQUIRE(d->dtype == MSG_BF16, MSG_ERR_UNSUPPORTED, "down_ring: bf16 only");
@@ -218,6 +222,8 @@ extern "C" int msg_down_ring(const msg_down_ring_desc* d, const void* x, const d
   MSG_REQUIRE((d->Ci_total & 7) == 0 && (d->ci_off & 7) == 0 && d->ci_off + 64 <= d->Ci_total, MSG_ERR_SHAPE, "down_ring: input channel layout (Cin = 64)");
   MSG_REQUIRE((d->Co_total & 7) == 0 && (d->co_off & 7) == 0 && d->co_off + d->Cout <= d->Co_total, MSG_ERR_SHAPE, "down_ring: output channel layout");
   MSG_REQUIRE(in_stats == nullptr || (d->cs_off >= 0 && d->cs_off + 64 <= d->Cs_total), MSG_ERR_SHAPE, "down_ring: stats layout");
+  MSG_REQUIRE((in_gamma == nullptr) == (in_beta == nullptr) && (in_gamma == nullptr || in_stats != nullptr) && in_img_stride >= 0,
+              MSG_ERR_SHAPE, "down_ring: an input affine needs gamma, beta and in_stats");
   MSG_REQUIRE((((uintptr_t)x | (uintptr_t)w_stacks | (uintptr_t)y) & 15) == 0, MSG_ERR_ALIGN, "down_ring: operands must be 16-byte aligned");
   MSG_REQUIRE(!(d->flags & MSG_CONV_STATS) || stats != nullptr, MSG_ERR_SHAPE, "down_ring: stats buffer missing");
   MSG_REQUIRE(get_encode() != nullptr, MSG_ERR_CUDA, "down_ring: cuTensorMapEncodeTiled unavailable");
@@ -227,6 +233,7 @@ extern "C" int msg_down_ring(const msg_down_ring_desc* d, const void* x, const d
   p.N = d->N; p.H = d->H; p.W = d->W; p.Co_total = d->Co_total;
   p.stats = (d->flags & MSG_CONV_STATS) ? stats : nullptr;
   p.in_stats = in_stats; p.Cs_total = d->Cs_total; p.cs_off = d->cs_off;
+  p.in_gamma = in_gamma; p.in_beta = in_beta; p.in_img_stride = in_img_stride;
   p.segs = (Wo + BM - 1) / BM;
   p.total_rows = (long long)d->N * p.segs * Ho;
   MSG_REQUIRE(p.total_rows < (1LL << 40), MSG_ERR_SHAPE, "down_ring: too many rows");
@@ -253,4 +260,9 @@ extern "C" int msg_down_ring(const msg_down_ring_desc* d, const void* x, const d
     if (rc) return rc;
   }
   return MSG_OK;
+}
+
+extern "C" int msg_down_ring(const msg_down_ring_desc* d, const void* x, const double* in_stats, const void* w_stacks, const float* bias,
+                             void* y, double* stats, void* stream) {
+  return msg_down_ring_affine(d, x, in_stats, nullptr, nullptr, 0, w_stacks, bias, y, stats, stream);
 }

@@ -1,5 +1,5 @@
-// InstanceNorm2d (affine-free, eps 1e-5, biased variance) on NHWC tensors: statistics, fused
-// apply (+ optional blended per-style affine, activation, residual add) and backward.
+// InstanceNorm2d (eps 1e-5, biased variance) on NHWC tensors: statistics, fused apply (+ optional affine -- a blend of
+// per-style gammas / betas shared by the batch, or a per-image table -- activation, residual add) and backward.
 // Bandwidth-bound: 16-byte vector accesses, per-thread channel groups fixed across the pixel loop
 // (so scale/shift live in registers), block reduction in shared memory, one atomic per
 // (block, channel).   Reference: nn.InstanceNorm2d at enhanced_generator.py:54..129, 242..263.
@@ -89,11 +89,29 @@ in_stats_generic_kernel(const T* __restrict__ x, long long HW, int C, double* __
 }
 
 // ---- apply ----------------------------------------------------------------------------------
+// The affine of channel c: with S > 0 the blend gamma = sum_s w[s] * gammas[s][c] (beta alike) as an fmaf chain over s in
+// ascending order from 0 -- msg_style_affine's chain, so its per-image tables reproduce these bits --, else the (agamma,
+// abeta) table at row offset `row` (in_affine: null = none).
+__device__ __forceinline__ void blend_or_affine(int S, const float* gammas, const float* betas, const float* w, int C,
+                                                const float* agamma, const float* abeta, size_t row, int c, float& g, float& b) {
+  if (S > 0) {
+    g = 0.f;
+    b = 0.f;
+    for (int s = 0; s < S; ++s) {
+      g = fmaf(w[s], gammas[(size_t)s * C + c], g);
+      b = fmaf(w[s], betas[(size_t)s * C + c], b);
+    }
+  } else {
+    in_affine(agamma, abeta, row + c, g, b);
+  }
+}
+
 template <typename T, bool FAST>
 __global__ void __launch_bounds__(TPB)
 in_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats, long long HW, int C,
                 int act, const T* __restrict__ residual, int S, const float* __restrict__ gammas,
-                const float* __restrict__ betas, const float* __restrict__ w, T* __restrict__ y) {
+                const float* __restrict__ betas, const float* __restrict__ w, const float* __restrict__ agamma,
+                const float* __restrict__ abeta, int astride, T* __restrict__ y) {
   constexpr int W = FAST ? Vec<T>::W : 1;
   const int n = blockIdx.y;
   const double inv_hw = 1.0 / (double)HW;
@@ -109,19 +127,9 @@ in_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats, long 
       c_cached = c0;
 #pragma unroll
       for (int e = 0; e < W; ++e) {
-        const double* st = stats + ((size_t)n * C + c0 + e) * 2;
-        float mean, rstd;
-        finalize_stats(st[0], st[1], inv_hw, mean, rstd);
-        float g = 1.f, b = 0.f;
-        if (S > 0) {
-          g = 0.f;
-          for (int s = 0; s < S; ++s) {
-            g = fmaf(w[s], gammas[(size_t)s * C + c0 + e], g);
-            b = fmaf(w[s], betas[(size_t)s * C + c0 + e], b);
-          }
-        }
-        scale[e] = rstd * g;
-        shift[e] = b - mean * scale[e];
+        float g, b, mean, rstd;
+        blend_or_affine(S, gammas, betas, w, C, agamma, abeta, (size_t)n * astride, c0 + e, g, b);
+        in_scale_shift(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, g, b, mean, rstd, scale[e], shift[e]);
       }
     }
     float t[W], r[W];
@@ -161,7 +169,8 @@ template <typename T, int ACT, bool HAS_RES>
 __global__ void __launch_bounds__(TPB, 3)
 in_apply_fast_kernel(const T* __restrict__ x, const double* __restrict__ stats, long long HW, int C,
                      const T* __restrict__ residual, int S, const float* __restrict__ gammas,
-                     const float* __restrict__ betas, const float* __restrict__ w, T* __restrict__ y) {
+                     const float* __restrict__ betas, const float* __restrict__ w, const float* __restrict__ agamma,
+                     const float* __restrict__ abeta, int astride, T* __restrict__ y) {
   constexpr int W = Vec<T>::W;
   constexpr int U = 4;
   const int n = blockIdx.y;
@@ -174,19 +183,9 @@ in_apply_fast_kernel(const T* __restrict__ x, const double* __restrict__ stats, 
   float scale[W], shift[W];
 #pragma unroll
   for (int e = 0; e < W; ++e) {
-    const double* st = stats + ((size_t)n * C + c0 + e) * 2;
-    float mean, rstd;
-    finalize_stats(st[0], st[1], inv_hw, mean, rstd);
-    float g = 1.f, b = 0.f;
-    if (S > 0) {
-      g = 0.f;
-      for (int s = 0; s < S; ++s) {
-        g = fmaf(w[s], gammas[(size_t)s * C + c0 + e], g);
-        b = fmaf(w[s], betas[(size_t)s * C + c0 + e], b);
-      }
-    }
-    scale[e] = rstd * g;
-    shift[e] = b - mean * scale[e];
+    float g, b, mean, rstd;
+    blend_or_affine(S, gammas, betas, w, C, agamma, abeta, (size_t)n * astride, c0 + e, g, b);
+    in_scale_shift(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, g, b, mean, rstd, scale[e], shift[e]);
   }
   const T* xb = x + base;
   const T* rb = HAS_RES ? residual + base : nullptr;
@@ -225,20 +224,16 @@ in_apply_fast_kernel(const T* __restrict__ x, const double* __restrict__ stats, 
 }
 
 // ---- backward -------------------------------------------------------------------------------
-// Per-channel constants of the backward.  xhat = (x - mean) * rstd.  With an affine (gamma, beta: fp32 [C]) the
-// activation's input is rebuilt as z = fmaf(x, scale, shift), scale = rstd * gamma, shift = beta - mean * scale: the
-// arithmetic of the forward apply, so the ReLU / LeakyReLU mask is the sign of the stored forward output bit for bit.
-// Without one, z = xhat and scale = rstd.
+// Per-channel constants of the backward.  xhat = (x - mean) * rstd.  With an affine (gamma, beta at element ai =
+// n * img_stride + c) the activation's input is rebuilt as z = fmaf(x, scale, shift) by in_scale_shift: the arithmetic of
+// the forward apply, so the ReLU / LeakyReLU mask is the sign of the stored forward output bit for bit.  Without one,
+// z = xhat and scale = rstd.
 template <bool AFFINE>
-__device__ __forceinline__ void bwd_channel(const double* st, double inv_hw, const float* gamma, const float* beta, int c,
+__device__ __forceinline__ void bwd_channel(const double* st, double inv_hw, const float* gamma, const float* beta, size_t ai,
                                             float& mean, float& rstd, float& scale, float& shift) {
-  finalize_stats(st[0], st[1], inv_hw, mean, rstd);
-  scale = rstd;
-  shift = 0.f;
-  if constexpr (AFFINE) {
-    scale = rstd * gamma[c];
-    shift = beta[c] - mean * scale;
-  }
+  float g = 1.f, b = 0.f;
+  if constexpr (AFFINE) { g = gamma[ai]; b = beta[ai]; }
+  in_scale_shift(st, inv_hw, g, b, mean, rstd, scale, shift);
 }
 
 // g = dy * act'(z)
@@ -247,17 +242,18 @@ __device__ __forceinline__ float bwd_grad(float t, float dy, float xh, float sca
   return dy * act_grad_from_pre(AFFINE ? fmaf(t, scale, shift) : xh, act);
 }
 
-// pass 1: scratch[n][c] += (sum g, sum g*xhat)
+// pass 1: scratch[n][c] += (sum g, sum g*xhat); scratch rows are img_stride apart for a per-image affine, else C
 template <typename T, bool FAST, bool AFFINE>
 __global__ void __launch_bounds__(TPB)
 in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
                      const T* __restrict__ dy, long long HW, int C, int act, const float* __restrict__ gamma,
-                     const float* __restrict__ beta, double* __restrict__ scratch) {
+                     const float* __restrict__ beta, int astride, double* __restrict__ scratch) {
   constexpr int W = FAST ? Vec<T>::W : 1;
   __shared__ float red[TPB][2 * W + 1];
   const int n = blockIdx.y;
   const double inv_hw = 1.0 / (double)HW;
   const size_t base = (size_t)n * HW * C;
+  const int sstride = astride ? astride : C;      // sums rows follow a per-image affine table
   if constexpr (FAST) {
     const long long nvec = HW * C / W;
     const long long stride = (long long)gridDim.x * TPB;
@@ -266,7 +262,7 @@ in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
     int c0 = (int)((v0 * W) % C);
 #pragma unroll
     for (int e = 0; e < W; ++e) {
-      bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, c0 + e, mean[e], rstd[e], scale[e], shift[e]);
+      bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, (size_t)n * astride + c0 + e, mean[e], rstd[e], scale[e], shift[e]);
       sg[e] = 0.f; sgx[e] = 0.f;
     }
     constexpr int U = 4;          // 2 x U raw 16-byte loads in flight per thread (unpacked only when consumed)
@@ -303,7 +299,7 @@ in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
       int gi = c / W, e = c - gi * W;
       float a = 0.f, b = 0.f;
       for (int t = gi; t < TPB; t += groups) { a += red[t][e]; b += red[t][W + e]; }
-      double* sc = scratch + ((size_t)n * C + c) * 2;
+      double* sc = scratch + ((size_t)n * sstride + c) * 2;
       atomicAdd(sc, (double)a);
       atomicAdd(sc + 1, (double)b);
     }
@@ -311,7 +307,7 @@ in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
     // generic: grid.x == C, one block per plane
     const int c = blockIdx.x;
     float mean, rstd, scale, shift;
-    bwd_channel<AFFINE>(stats + ((size_t)n * C + c) * 2, inv_hw, gamma, beta, c, mean, rstd, scale, shift);
+    bwd_channel<AFFINE>(stats + ((size_t)n * C + c) * 2, inv_hw, gamma, beta, (size_t)n * astride + c, mean, rstd, scale, shift);
     float sg = 0.f, sgx = 0.f;
     for (long long p = threadIdx.x; p < HW; p += TPB) {
       float t = to_f<T>(x[base + (size_t)p * C + c]);
@@ -325,7 +321,7 @@ in_bwd_reduce_kernel(const T* __restrict__ x, const double* __restrict__ stats,
     if (threadIdx.x == 0) {
       float a = 0.f, b = 0.f;
       for (int i = 0; i < TPB / 32; ++i) { a += red[i][0]; b += red[i][1]; }
-      double* sc = scratch + ((size_t)n * C + c) * 2;
+      double* sc = scratch + ((size_t)n * sstride + c) * 2;
       sc[0] += (double)a; sc[1] += (double)b;
     }
   }
@@ -336,7 +332,7 @@ template <typename T, bool FAST, bool AFFINE>
 __global__ void __launch_bounds__(TPB)
 in_bwd_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats,
                     const T* __restrict__ dy, long long HW, int C, int act, const float* __restrict__ gamma,
-                    const float* __restrict__ beta, const double* __restrict__ scratch, T* __restrict__ dx) {
+                    const float* __restrict__ beta, int astride, const double* __restrict__ scratch, T* __restrict__ dx) {
   constexpr int W = FAST ? Vec<T>::W : 1;
   const int n = blockIdx.y;
   const double inv_hw = 1.0 / (double)HW;
@@ -344,14 +340,15 @@ in_bwd_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats,
   const long long nvec = HW * C / W;
   const long long stride = (long long)gridDim.x * TPB;
   long long v0 = (long long)blockIdx.x * TPB + threadIdx.x;
+  const int sstride = astride ? astride : C;
   float mean[W], rstd[W], scale[W], shift[W], mg[W], mgx[W];
   if constexpr (FAST) {
     // channel group of a thread is loop-invariant (stride * W is a multiple of C); 2 x U raw loads in flight per thread
     const int c0 = (int)((v0 * W) % C);
 #pragma unroll
     for (int e = 0; e < W; ++e) {
-      bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, c0 + e, mean[e], rstd[e], scale[e], shift[e]);
-      const double* sc = scratch + ((size_t)n * C + c0 + e) * 2;
+      bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, (size_t)n * astride + c0 + e, mean[e], rstd[e], scale[e], shift[e]);
+      const double* sc = scratch + ((size_t)n * sstride + c0 + e) * 2;
       mg[e] = (float)(sc[0] * inv_hw); mgx[e] = (float)(sc[1] * inv_hw);
     }
     constexpr int U = 4;
@@ -391,8 +388,8 @@ in_bwd_apply_kernel(const T* __restrict__ x, const double* __restrict__ stats,
       c_cached = c0;
 #pragma unroll
       for (int e = 0; e < W; ++e) {
-        bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, c0 + e, mean[e], rstd[e], scale[e], shift[e]);
-        const double* sc = scratch + ((size_t)n * C + c0 + e) * 2;
+        bwd_channel<AFFINE>(stats + ((size_t)n * C + c0 + e) * 2, inv_hw, gamma, beta, (size_t)n * astride + c0 + e, mean[e], rstd[e], scale[e], shift[e]);
+        const double* sc = scratch + ((size_t)n * sstride + c0 + e) * 2;
         mg[e] = (float)(sc[0] * inv_hw); mgx[e] = (float)(sc[1] * inv_hw);
       }
     }
@@ -442,7 +439,8 @@ int stats_impl(const T* x, int N, long long HW, int C, double* stats, cudaStream
 
 template <typename T>
 int apply_impl(const T* x, const double* stats, int N, long long HW, int C, int act, const T* res,
-               int S, const float* gammas, const float* betas, const float* w, T* y, cudaStream_t st) {
+               int S, const float* gammas, const float* betas, const float* w, const float* agamma, const float* abeta,
+               int astride, T* y, cudaStream_t st) {
   if (fast_ok<T>(C, HW)) {
     const long long nvec = HW * C / Vec<T>::W;
     static const int ctas_per_sm = [] { const char* e = getenv("MSG_IN_CTAS"); return e ? atoi(e) : 12; }();
@@ -456,7 +454,7 @@ int apply_impl(const T* x, const double* stats, int N, long long HW, int C, int 
     if (want > maxb) want = maxb;
     if (want < 1) want = 1;
     dim3 grid((unsigned)want, N);
-#define MSG_IN_APPLY(ACT, RES) in_apply_fast_kernel<T, ACT, RES><<<grid, TPB, 0, st>>>(x, stats, HW, C, res, S, gammas, betas, w, y)
+#define MSG_IN_APPLY(ACT, RES) in_apply_fast_kernel<T, ACT, RES><<<grid, TPB, 0, st>>>(x, stats, HW, C, res, S, gammas, betas, w, agamma, abeta, astride, y)
     if (res) {
       if (act == MSG_ACT_RELU) MSG_IN_APPLY(MSG_ACT_RELU, true);
       else if (act == MSG_ACT_LRELU) MSG_IN_APPLY(MSG_ACT_LRELU, true);
@@ -469,38 +467,39 @@ int apply_impl(const T* x, const double* stats, int N, long long HW, int C, int 
 #undef MSG_IN_APPLY
   } else {
     dim3 grid(blocks_per_image(N, HW * C), N);
-    in_apply_kernel<T, false><<<grid, TPB, 0, st>>>(x, stats, HW, C, act, res, S, gammas, betas, w, y);
+    in_apply_kernel<T, false><<<grid, TPB, 0, st>>>(x, stats, HW, C, act, res, S, gammas, betas, w, agamma, abeta, astride, y);
   }
   return check_launch("in_apply_kernel");
 }
 
 template <typename T>
 int bwd_reduce_impl(const T* x, const double* stats, const T* dy, int N, long long HW, int C, int act,
-                    const float* gamma, const float* beta, double* scratch, cudaStream_t st) {
-  cudaMemsetAsync(scratch, 0, (size_t)N * C * 2 * sizeof(double), st);
+                    const float* gamma, const float* beta, int astride, double* scratch, cudaStream_t st) {
+  if (astride == 0 || astride == C) cudaMemsetAsync(scratch, 0, (size_t)N * C * 2 * sizeof(double), st);
+  else cudaMemset2DAsync(scratch, (size_t)astride * 2 * sizeof(double), 0, (size_t)C * 2 * sizeof(double), N, st);
   if (fast_ok<T>(C, HW)) {
     dim3 grid(blocks_per_image(N, HW * C / Vec<T>::W), N);
-    if (gamma) in_bwd_reduce_kernel<T, true, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, scratch);
-    else in_bwd_reduce_kernel<T, true, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, scratch);
+    if (gamma) in_bwd_reduce_kernel<T, true, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, astride, scratch);
+    else in_bwd_reduce_kernel<T, true, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, 0, scratch);
   } else {
     dim3 grid(C, N);
-    if (gamma) in_bwd_reduce_kernel<T, false, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, scratch);
-    else in_bwd_reduce_kernel<T, false, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, scratch);
+    if (gamma) in_bwd_reduce_kernel<T, false, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, astride, scratch);
+    else in_bwd_reduce_kernel<T, false, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, 0, scratch);
   }
   return check_launch("in_bwd_reduce_kernel");
 }
 
 template <typename T>
 int bwd_apply_impl(const T* x, const double* stats, const T* dy, int N, long long HW, int C, int act,
-                   const float* gamma, const float* beta, const double* scratch, T* dx, cudaStream_t st) {
+                   const float* gamma, const float* beta, int astride, const double* scratch, T* dx, cudaStream_t st) {
   if (fast_ok<T>(C, HW)) {
     dim3 grid(blocks_per_image(N, HW * C / Vec<T>::W), N);
-    if (gamma) in_bwd_apply_kernel<T, true, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, scratch, dx);
-    else in_bwd_apply_kernel<T, true, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, scratch, dx);
+    if (gamma) in_bwd_apply_kernel<T, true, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, astride, scratch, dx);
+    else in_bwd_apply_kernel<T, true, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, 0, scratch, dx);
   } else {
     dim3 grid(blocks_per_image(N, HW * C), N);
-    if (gamma) in_bwd_apply_kernel<T, false, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, scratch, dx);
-    else in_bwd_apply_kernel<T, false, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, scratch, dx);
+    if (gamma) in_bwd_apply_kernel<T, false, true><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, gamma, beta, astride, scratch, dx);
+    else in_bwd_apply_kernel<T, false, false><<<grid, TPB, 0, st>>>(x, stats, dy, HW, C, act, nullptr, nullptr, 0, scratch, dx);
   }
   return check_launch("in_bwd_apply_kernel");
 }
@@ -508,8 +507,8 @@ int bwd_apply_impl(const T* x, const double* stats, const T* dy, int N, long lon
 template <typename T>
 int bwd_impl(const T* x, const double* stats, const T* dy, int N, long long HW, int C, int act,
              double* scratch, T* dx, cudaStream_t st) {
-  int rc = bwd_reduce_impl<T>(x, stats, dy, N, HW, C, act, nullptr, nullptr, scratch, st);
-  return rc ? rc : bwd_apply_impl<T>(x, stats, dy, N, HW, C, act, nullptr, nullptr, scratch, dx, st);
+  int rc = bwd_reduce_impl<T>(x, stats, dy, N, HW, C, act, nullptr, nullptr, 0, scratch, st);
+  return rc ? rc : bwd_apply_impl<T>(x, stats, dy, N, HW, C, act, nullptr, nullptr, 0, scratch, dx, st);
 }
 
 }  // namespace
@@ -525,17 +524,28 @@ extern "C" int msg_instnorm_stats(int dtype, const void* x, int N, long long HW,
   MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_stats: bad dtype");
 }
 
-extern "C" int msg_instnorm_apply(int dtype, const void* x, const double* stats, int N, long long HW,
-                                  int C, int act, const void* residual, int S, const float* gammas,
-                                  const float* betas, const float* w, void* y, void* stream) {
+extern "C" int msg_instnorm_apply_affine(int dtype, const void* x, const double* stats, int N, long long HW, int C, int act,
+                                         const void* residual, int S, const float* gammas, const float* betas, const float* w,
+                                         const float* gamma, const float* beta, int img_stride, void* y, void* stream) {
   MSG_REQUIRE(N > 0 && HW > 0 && C > 0, MSG_ERR_SHAPE, "instnorm_apply: bad shape");
   MSG_REQUIRE(act == MSG_ACT_NONE || act == MSG_ACT_RELU || act == MSG_ACT_LRELU, MSG_ERR_UNSUPPORTED, "instnorm_apply: bad act");
   MSG_REQUIRE(S == 0 || (gammas && betas && w), MSG_ERR_SHAPE, "instnorm_apply: S>0 needs gammas/betas/w");
+  MSG_REQUIRE((gamma == nullptr) == (beta == nullptr), MSG_ERR_SHAPE, "instnorm_apply: gamma and beta go together");
+  MSG_REQUIRE(gamma == nullptr || S == 0, MSG_ERR_SHAPE, "instnorm_apply: a style blend (S > 0) and an affine table exclude each other");
+  MSG_REQUIRE(img_stride == 0 || img_stride >= C, MSG_ERR_SHAPE, "instnorm_apply: img_stride must be 0 or >= C");
   if (dtype == MSG_F32)
-    return apply_impl<float>((const float*)x, stats, N, HW, C, act, (const float*)residual, S, gammas, betas, w, (float*)y, as_stream(stream));
+    return apply_impl<float>((const float*)x, stats, N, HW, C, act, (const float*)residual, S, gammas, betas, w, gamma, beta, img_stride,
+                             (float*)y, as_stream(stream));
   if (dtype == MSG_BF16)
-    return apply_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, N, HW, C, act, (const __nv_bfloat16*)residual, S, gammas, betas, w, (__nv_bfloat16*)y, as_stream(stream));
+    return apply_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, N, HW, C, act, (const __nv_bfloat16*)residual, S, gammas, betas, w,
+                                     gamma, beta, img_stride, (__nv_bfloat16*)y, as_stream(stream));
   MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_apply: bad dtype");
+}
+
+extern "C" int msg_instnorm_apply(int dtype, const void* x, const double* stats, int N, long long HW,
+                                  int C, int act, const void* residual, int S, const float* gammas,
+                                  const float* betas, const float* w, void* y, void* stream) {
+  return msg_instnorm_apply_affine(dtype, x, stats, N, HW, C, act, residual, S, gammas, betas, w, nullptr, nullptr, 0, y, stream);
 }
 
 extern "C" int msg_instnorm_bwd(int dtype, const void* x, const double* stats, const void* dy, int N,
@@ -549,31 +559,45 @@ extern "C" int msg_instnorm_bwd(int dtype, const void* x, const double* stats, c
   MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_bwd: bad dtype");
 }
 
-extern "C" int msg_instnorm_bwd_reduce(int dtype, const void* x, const double* stats, const void* dy, int N,
-                                       long long HW, int C, int act, const float* gamma, const float* beta,
-                                       double* sums, void* stream) {
+extern "C" int msg_instnorm_bwd_reduce_affine(int dtype, const void* x, const double* stats, const void* dy, int N, long long HW, int C,
+                                              int act, const float* gamma, const float* beta, int img_stride, double* sums,
+                                              void* stream) {
   MSG_REQUIRE(N > 0 && HW > 0 && C > 0, MSG_ERR_SHAPE, "instnorm_bwd_reduce: bad shape");
   MSG_REQUIRE(act == MSG_ACT_NONE || act == MSG_ACT_RELU || act == MSG_ACT_LRELU, MSG_ERR_UNSUPPORTED, "instnorm_bwd_reduce: bad act");
   MSG_REQUIRE((gamma == nullptr) == (beta == nullptr), MSG_ERR_SHAPE, "instnorm_bwd_reduce: gamma and beta go together");
+  MSG_REQUIRE(img_stride == 0 || (gamma != nullptr && img_stride >= C), MSG_ERR_SHAPE, "instnorm_bwd_reduce: img_stride must be 0 or >= C");
   if (dtype == MSG_F32)
-    return bwd_reduce_impl<float>((const float*)x, stats, (const float*)dy, N, HW, C, act, gamma, beta, sums, as_stream(stream));
+    return bwd_reduce_impl<float>((const float*)x, stats, (const float*)dy, N, HW, C, act, gamma, beta, img_stride, sums, as_stream(stream));
   if (dtype == MSG_BF16)
-    return bwd_reduce_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, (const __nv_bfloat16*)dy, N, HW, C, act, gamma, beta, sums,
-                                          as_stream(stream));
+    return bwd_reduce_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, (const __nv_bfloat16*)dy, N, HW, C, act, gamma, beta, img_stride,
+                                          sums, as_stream(stream));
   MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_bwd_reduce: bad dtype");
+}
+
+extern "C" int msg_instnorm_bwd_reduce(int dtype, const void* x, const double* stats, const void* dy, int N,
+                                       long long HW, int C, int act, const float* gamma, const float* beta,
+                                       double* sums, void* stream) {
+  return msg_instnorm_bwd_reduce_affine(dtype, x, stats, dy, N, HW, C, act, gamma, beta, 0, sums, stream);
+}
+
+extern "C" int msg_instnorm_bwd_apply_affine(int dtype, const void* x, const double* stats, const void* dy, int N, long long HW, int C,
+                                             int act, const float* gamma, const float* beta, int img_stride, const double* sums,
+                                             void* dx, void* stream) {
+  MSG_REQUIRE(N > 0 && HW > 0 && C > 0, MSG_ERR_SHAPE, "instnorm_bwd_apply: bad shape");
+  MSG_REQUIRE(act == MSG_ACT_NONE || act == MSG_ACT_RELU || act == MSG_ACT_LRELU, MSG_ERR_UNSUPPORTED, "instnorm_bwd_apply: bad act");
+  MSG_REQUIRE((gamma == nullptr) == (beta == nullptr), MSG_ERR_SHAPE, "instnorm_bwd_apply: gamma and beta go together");
+  MSG_REQUIRE(img_stride == 0 || (gamma != nullptr && img_stride >= C), MSG_ERR_SHAPE, "instnorm_bwd_apply: img_stride must be 0 or >= C");
+  if (dtype == MSG_F32)
+    return bwd_apply_impl<float>((const float*)x, stats, (const float*)dy, N, HW, C, act, gamma, beta, img_stride, sums, (float*)dx,
+                                 as_stream(stream));
+  if (dtype == MSG_BF16)
+    return bwd_apply_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, (const __nv_bfloat16*)dy, N, HW, C, act, gamma, beta, img_stride,
+                                         sums, (__nv_bfloat16*)dx, as_stream(stream));
+  MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_bwd_apply: bad dtype");
 }
 
 extern "C" int msg_instnorm_bwd_apply(int dtype, const void* x, const double* stats, const void* dy, int N,
                                       long long HW, int C, int act, const float* gamma, const float* beta,
                                       const double* sums, void* dx, void* stream) {
-  MSG_REQUIRE(N > 0 && HW > 0 && C > 0, MSG_ERR_SHAPE, "instnorm_bwd_apply: bad shape");
-  MSG_REQUIRE(act == MSG_ACT_NONE || act == MSG_ACT_RELU || act == MSG_ACT_LRELU, MSG_ERR_UNSUPPORTED, "instnorm_bwd_apply: bad act");
-  MSG_REQUIRE((gamma == nullptr) == (beta == nullptr), MSG_ERR_SHAPE, "instnorm_bwd_apply: gamma and beta go together");
-  if (dtype == MSG_F32)
-    return bwd_apply_impl<float>((const float*)x, stats, (const float*)dy, N, HW, C, act, gamma, beta, sums, (float*)dx,
-                                 as_stream(stream));
-  if (dtype == MSG_BF16)
-    return bwd_apply_impl<__nv_bfloat16>((const __nv_bfloat16*)x, stats, (const __nv_bfloat16*)dy, N, HW, C, act, gamma, beta, sums,
-                                         (__nv_bfloat16*)dx, as_stream(stream));
-  MSG_REQUIRE(false, MSG_ERR_UNSUPPORTED, "instnorm_bwd_apply: bad dtype");
+  return msg_instnorm_bwd_apply_affine(dtype, x, stats, dy, N, HW, C, act, gamma, beta, 0, sums, dx, stream);
 }

@@ -113,6 +113,9 @@ struct LaParams {
   const float* bqkv;
   const float* bproj;
   const double* in_stats;     // XF: raw plane sums [N][C][2] of the input tensor
+  const float* in_gamma;      // XF: optional affine of the input norm (common.cuh: in_affine), or null
+  const float* in_beta;
+  int in_img_stride;
   int in_act;
   unsigned long long* trace;  // MSG_LA_TRACE builds only: [role][event] = (tag, clock) pairs of CTA 0
 };
@@ -192,7 +195,9 @@ __device__ __forceinline__ void acc_pass(uint32_t taddr, F&& f, R&& released) {
   }
 }
 
-template <int C, bool XF>
+// AFF (with XF): the input norm has a per-image affine.  A template parameter so that the affine-free kernel keeps its register
+// allocation (C = 128 spills in its transform warps).
+template <int C, bool XF, bool AFF = false>
 __global__ void __launch_bounds__(32 * Cfg<C>::NWARPS, 1)
 la_stage_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapWqkv,
                 const __grid_constant__ CUtensorMap mapWproj, const __grid_constant__ CUtensorMap mapOut, const LaParams p) {
@@ -716,11 +721,9 @@ la_stage_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant_
       if (img != cur_img) {
         asm volatile("bar.sync 2, 128;" ::: "memory");
         for (int ci = xt; ci < C; ci += 128) {
-          const double* st = p.in_stats + ((size_t)img * C + ci) * 2;
-          float mean, rstd;
-          finalize_stats(st[0], st[1], inv_hw, mean, rstd);
-          xf_tab[ci] = rstd;
-          xf_tab[C + ci] = 0.f - mean * rstd;
+          float g = 1.f, b = 0.f, mean, rstd;
+          if constexpr (AFF) in_affine(p.in_gamma, p.in_beta, (size_t)img * p.in_img_stride + ci, g, b);
+          in_scale_shift(p.in_stats + ((size_t)img * C + ci) * 2, inv_hw, g, b, mean, rstd, xf_tab[ci], xf_tab[C + ci]);
         }
         asm volatile("bar.sync 2, 128;" ::: "memory");
         cur_img = img;
@@ -780,17 +783,17 @@ la_stage_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant_
 
 unsigned long long* g_trace = nullptr;
 
-template <int C, bool XF>
+template <int C, bool XF, bool AFF = false>
 int launch(const CUtensorMap& mX, const CUtensorMap& mQ, const CUtensorMap& mP, const CUtensorMap& mO, const LaParams& p, cudaStream_t st) {
   static DeviceOnce attr_set;
   if (attr_set.needed()) {
-    cudaError_t e = cudaFuncSetAttribute(la_stage_kernel<C, XF>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<C>::SMEM);
+    cudaError_t e = cudaFuncSetAttribute(la_stage_kernel<C, XF, AFF>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<C>::SMEM);
     MSG_REQUIRE(e == cudaSuccess, MSG_ERR_CUDA, "la_stage: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     attr_set.done();
   }
   int grid = sm_count();
   if (grid > p.total_tiles) grid = p.total_tiles;
-  la_stage_kernel<C, XF><<<grid, 32 * Cfg<C>::NWARPS, Cfg<C>::SMEM, st>>>(mX, mQ, mP, mO, p);
+  la_stage_kernel<C, XF, AFF><<<grid, 32 * Cfg<C>::NWARPS, Cfg<C>::SMEM, st>>>(mX, mQ, mP, mO, p);
   return check_launch("la_stage_kernel");
 }
 
@@ -806,8 +809,9 @@ bool la_stage_supported(int dtype, int N, int H, int W, int C, const void* x, co
   return get_encode() != nullptr;
 }
 
-int la_stage_fwd(const void* x, const double* in_stats, int in_act, const void* wqkv, const float* bqkv, const void* wproj,
-                 const float* bproj, int N, int H, int W, int C, void* out, cudaStream_t st) {
+int la_stage_fwd(const void* x, const double* in_stats, const float* in_gamma, const float* in_beta, int in_img_stride, int in_act,
+                 const void* wqkv, const float* bqkv, const void* wproj, const float* bproj, int N, int H, int W, int C, void* out,
+                 cudaStream_t st) {
   EncodeTiledFn enc = get_encode();
   MSG_REQUIRE(enc != nullptr, MSG_ERR_CUDA, "la_stage: cuTensorMapEncodeTiled unavailable");
   LaParams p;
@@ -816,6 +820,7 @@ int la_stage_fwd(const void* x, const double* in_stats, int in_act, const void* 
   p.tiles_per_img = (H / 4) * p.tiles_w;
   p.total_tiles = N * p.tiles_per_img;
   p.bqkv = bqkv; p.bproj = bproj; p.in_stats = in_stats; p.in_act = in_act;
+  p.in_gamma = in_gamma; p.in_beta = in_beta; p.in_img_stride = in_img_stride;
   p.trace = g_trace;
   CUtensorMap mX, mO, mQ, mP;
   for (int which = 0; which < 2; ++which) {
@@ -841,8 +846,13 @@ int la_stage_fwd(const void* x, const double* in_stats, int in_act, const void* 
     MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "la_stage: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
   }
   const bool xf = in_stats != nullptr;
-  if (C == 64) return xf ? launch<64, true>(mX, mQ, mP, mO, p, st) : launch<64, false>(mX, mQ, mP, mO, p, st);
-  return xf ? launch<128, true>(mX, mQ, mP, mO, p, st) : launch<128, false>(mX, mQ, mP, mO, p, st);
+  const bool aff = in_gamma != nullptr;
+  if (C == 64) {
+    if (!xf) return launch<64, false>(mX, mQ, mP, mO, p, st);
+    return aff ? launch<64, true, true>(mX, mQ, mP, mO, p, st) : launch<64, true>(mX, mQ, mP, mO, p, st);
+  }
+  if (!xf) return launch<128, false>(mX, mQ, mP, mO, p, st);
+  return aff ? launch<128, true, true>(mX, mQ, mP, mO, p, st) : launch<128, true>(mX, mQ, mP, mO, p, st);
 }
 
 }  // namespace msg
@@ -860,12 +870,20 @@ extern "C" int msg_la_stage_supported(int dtype, int N, int H, int W, int C, con
   return la_stage_supported(dtype, N, H, W, C, x, wqkv, wproj, out) ? 1 : 0;
 }
 
-extern "C" int msg_la_stage_fwd(int dtype, const void* x, const double* in_stats, int in_act, const void* wqkv, const float* bqkv,
-                                const void* wproj, const float* bproj, int N, int H, int W, int C, void* out, void* stream) {
+extern "C" int msg_la_stage_fwd_affine(int dtype, const void* x, const double* in_stats, const float* in_gamma, const float* in_beta,
+                                       int in_img_stride, int in_act, const void* wqkv, const float* bqkv, const void* wproj,
+                                       const float* bproj, int N, int H, int W, int C, void* out, void* stream) {
   MSG_REQUIRE(x && wqkv && bqkv && wproj && bproj && out, MSG_ERR_SHAPE, "la_stage: null pointer");
   MSG_REQUIRE(la_stage_supported(dtype, N, H, W, C, x, wqkv, wproj, out), MSG_ERR_UNSUPPORTED,
               "la_stage: needs bf16, C in {64, 128}, H and W multiples of 4, 16-byte aligned pointers (got C=%d, %dx%d)", C, H, W);
   MSG_REQUIRE(in_stats == nullptr || in_act == MSG_ACT_NONE || in_act == MSG_ACT_RELU, MSG_ERR_UNSUPPORTED,
               "la_stage: fused input norm supports ReLU / no activation");
-  return la_stage_fwd(x, in_stats, in_act, wqkv, bqkv, wproj, bproj, N, H, W, C, out, as_stream(stream));
+  MSG_REQUIRE((in_gamma == nullptr) == (in_beta == nullptr) && (in_gamma == nullptr || in_stats != nullptr) && in_img_stride >= 0,
+              MSG_ERR_SHAPE, "la_stage: an input affine needs gamma, beta and in_stats");
+  return la_stage_fwd(x, in_stats, in_gamma, in_beta, in_img_stride, in_act, wqkv, bqkv, wproj, bproj, N, H, W, C, out, as_stream(stream));
+}
+
+extern "C" int msg_la_stage_fwd(int dtype, const void* x, const double* in_stats, int in_act, const void* wqkv, const float* bqkv,
+                                const void* wproj, const float* bproj, int N, int H, int W, int C, void* out, void* stream) {
+  return msg_la_stage_fwd_affine(dtype, x, in_stats, nullptr, nullptr, 0, in_act, wqkv, bqkv, wproj, bproj, N, H, W, C, out, stream);
 }

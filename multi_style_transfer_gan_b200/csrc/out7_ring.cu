@@ -48,6 +48,9 @@ struct O7Params {
   const float* bias;                    // [3]
   const double* in_stats;               // [N][Cs_total][2] raw plane sums of f
   int Cs_total, cs_off;
+  const float* in_gamma;                // optional affine of f's norm (common.cuh: in_affine), or null
+  const float* in_beta;
+  int in_img_stride;
   float* y;                             // fp32 NCHW [N][3][H][W]
 };
 
@@ -136,7 +139,7 @@ out7_ring_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_constant
     SlabRing ring(bars.S);
     for (Walk pc = pieces; pc.next();) {
       if (pc.img != cur_img) {
-        load_scale_shift(p.in_stats, pc.img, p.Cs_total, p.cs_off, lchunk, inv_hw, sc, sh);
+        load_scale_shift(p.in_stats, p.in_gamma, p.in_beta, p.in_img_stride, pc.img, p.Cs_total, p.cs_off, lchunk, inv_hw, sc, sh);
         cur_img = pc.img;
       }
       const int r_lo = pc.r0 < 0 ? 0 : pc.r0, r_hi = pc.r1 > p.H ? p.H : pc.r1;
@@ -191,8 +194,9 @@ out7_ring_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_constant
 
 using namespace msg;
 
-extern "C" int msg_out7_ring(const msg_out7_ring_desc* d, const void* f, const double* in_stats, const void* residual,
-                             const void* w_stacks, const float* bias, float* y, void* stream) {
+extern "C" int msg_out7_ring_affine(const msg_out7_ring_desc* d, const void* f, const double* in_stats, const float* in_gamma,
+                                    const float* in_beta, int in_img_stride, const void* residual, const void* w_stacks, const float* bias,
+                                    float* y, void* stream) {
   cudaStream_t st = as_stream(stream);
   MSG_REQUIRE(d != nullptr && f && in_stats && residual && w_stacks && y, MSG_ERR_SHAPE, "out7_ring: null argument");
   MSG_REQUIRE(d->dtype == MSG_BF16, MSG_ERR_UNSUPPORTED, "out7_ring: bf16 only");
@@ -200,6 +204,7 @@ extern "C" int msg_out7_ring(const msg_out7_ring_desc* d, const void* f, const d
   MSG_REQUIRE((d->Cf_total & 7) == 0 && (d->cf_off & 7) == 0 && d->cf_off + 64 <= d->Cf_total, MSG_ERR_SHAPE, "out7_ring: f channel layout");
   MSG_REQUIRE((d->Cr_total & 7) == 0 && (d->cr_off & 7) == 0 && d->cr_off + 64 <= d->Cr_total, MSG_ERR_SHAPE, "out7_ring: residual channel layout");
   MSG_REQUIRE(d->cs_off >= 0 && d->cs_off + 64 <= d->Cs_total, MSG_ERR_SHAPE, "out7_ring: stats layout");
+  MSG_REQUIRE((in_gamma == nullptr) == (in_beta == nullptr) && in_img_stride >= 0, MSG_ERR_SHAPE, "out7_ring: gamma and beta go together");
   MSG_REQUIRE((((uintptr_t)f | (uintptr_t)residual | (uintptr_t)w_stacks) & 15) == 0, MSG_ERR_ALIGN, "out7_ring: operands must be 16-byte aligned");
   MSG_REQUIRE(get_encode() != nullptr, MSG_ERR_CUDA, "out7_ring: cuTensorMapEncodeTiled unavailable");
 
@@ -209,6 +214,7 @@ extern "C" int msg_out7_ring(const msg_out7_ring_desc* d, const void* f, const d
   p.total_rows = (long long)d->N * p.segs * d->H;
   MSG_REQUIRE(p.total_rows < (1LL << 40), MSG_ERR_SHAPE, "out7_ring: too many rows");
   p.bias = bias; p.in_stats = in_stats; p.Cs_total = d->Cs_total; p.cs_off = d->cs_off; p.y = y;
+  p.in_gamma = in_gamma; p.in_beta = in_beta; p.in_img_stride = in_img_stride;
 
   CUtensorMap mapF, mapR, mapB;
   CUresult r = encode_slab(&mapF, (const __nv_bfloat16*)f + d->cf_off, 64, d->Cf_total, d->W, d->H, d->N);
@@ -218,4 +224,9 @@ extern "C" int msg_out7_ring(const msg_out7_ring_desc* d, const void* f, const d
   r = encode_weights(&mapB, w_stacks, W_ROWS);
   MSG_REQUIRE(r == CUDA_SUCCESS, MSG_ERR_CUDA, "out7_ring: cuTensorMapEncodeTiled(w) failed with %d", (int)r);
   return launch<out7_ring_kernel>("out7_ring_kernel", o7_shape(), NTHREADS, p.total_rows, 8, p, mapF, mapR, mapB, st);
+}
+
+extern "C" int msg_out7_ring(const msg_out7_ring_desc* d, const void* f, const double* in_stats, const void* residual,
+                             const void* w_stacks, const float* bias, float* y, void* stream) {
+  return msg_out7_ring_affine(d, f, in_stats, nullptr, nullptr, 0, residual, w_stacks, bias, y, stream);
 }

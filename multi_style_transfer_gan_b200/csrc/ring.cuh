@@ -359,16 +359,15 @@ __device__ __forceinline__ void store_piece_bf16(uint8_t* stg, const float (&v)[
 // ---------------------------------------------------------------- transform warps
 // Thread t of the four transform warps owns the physical 16-byte chunk (t & 7) of the slab rows (t >> 3) + 16 i: because the
 // 128-byte swizzle only uses row & 7, the LOGICAL channel chunk is the same for all its rows and its 8 per-image scales / shifts
-// (x * rstd - mean * rstd) live in registers.
-__device__ __forceinline__ void load_scale_shift(const double* in_stats, int img, int Cs_total, int cs_off, int lchunk, double inv_hw,
-                                                 float (&sc)[8], float (&sh)[8]) {
+// (in_scale_shift: x * rstd * gamma + beta - mean * rstd * gamma, the affine optional) live in registers.
+__device__ __forceinline__ void load_scale_shift(const double* in_stats, const float* in_gamma, const float* in_beta, int in_img_stride,
+                                                 int img, int Cs_total, int cs_off, int lchunk, double inv_hw, float (&sc)[8], float (&sh)[8]) {
 #pragma unroll
   for (int e = 0; e < 8; ++e) {
-    const double* st = in_stats + ((size_t)img * Cs_total + cs_off + lchunk * 8 + e) * 2;
-    float mean, rstd;
-    finalize_stats(st[0], st[1], inv_hw, mean, rstd);
-    sc[e] = rstd;
-    sh[e] = 0.f - mean * rstd;
+    const int c = cs_off + lchunk * 8 + e;
+    float g, b, mean, rstd;
+    in_affine(in_gamma, in_beta, (size_t)img * in_img_stride + c, g, b);
+    in_scale_shift(in_stats + ((size_t)img * Cs_total + c) * 2, inv_hw, g, b, mean, rstd, sc[e], sh[e]);
   }
 }
 

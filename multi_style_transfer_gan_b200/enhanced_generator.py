@@ -9,6 +9,10 @@ extension) raises.
 Precision: ``model.set_precision("fp32" | "bf16")`` (default "fp32" = the parity mode, <=1e-4 vs the
 reference); inside ``torch.autocast("cuda")`` -- which is how the reference trains
 (enhanced_train.py:61,88) -- the bf16 tensor-core path is used automatically.
+
+Style-conditional generator (an extension, not in the reference): ``model.enable_style_affine(S)`` gives every
+InstanceNorm an [S, C] affine (conditional instance norm, Dumoulin et al.) and ``model(x, style=w)`` blends the S
+styles per image, gamma_n = sum_s w[n, s] gamma_s (beta alike), in one forward pass.
 """
 import math
 
@@ -69,13 +73,19 @@ class ConvTranspose2d(Conv2d):
 
 
 class InstanceNorm2d(_NoForward):
-    """affine=False, track_running_stats=False, eps=1e-5: no parameters, no state_dict entries."""
+    """affine=False, track_running_stats=False, eps=1e-5: no parameters, no state_dict entries -- until
+    EnhancedGenerator.enable_style_affine gives it weight / bias [S, C] (nn.InstanceNorm2d(affine=True) with a leading
+    style axis, initialised to 1 and 0)."""
 
     def __init__(self, num_features):
         super().__init__()
         self.num_features, self.eps = num_features, 1e-5
         self.weight = None
         self.bias = None
+
+    def _enable_style_affine(self, num_styles, device):
+        self.weight = nn.Parameter(torch.ones(num_styles, self.num_features, device=device))
+        self.bias = nn.Parameter(torch.zeros(num_styles, self.num_features, device=device))
 
 
 class ReLU(_NoForward):
@@ -154,87 +164,102 @@ def _check_input(x, what):
     _lib.require_device(x.device.index)
 
 
+# A (argument 4 of the functions below): the StyleAffine tables of a style-conditional forward, or None.  It is not a tensor
+# input: no gradient flows to the style mix; the backward turns the per-image affine gradients into those of the [S, C]
+# parameters itself (GeneratorEngine.style_affine_end_bwd).
 class _GeneratorFn(torch.autograd.Function):
     """Whole-generator op: one autograd node, manual backward over saved NHWC activations."""
 
     @staticmethod
-    def forward(ctx, model, dtype, keys, grad_on, x, *params):
+    def forward(ctx, model, dtype, keys, grad_on, A, x, *params):
         eng = model._engine
         P = dict(zip(keys, params))
-        need = grad_on and (ctx.needs_input_grad[4] or any(ctx.needs_input_grad[5:]))   # needs_input_grad ignores no_grad
+        need = grad_on and (ctx.needs_input_grad[5] or any(ctx.needs_input_grad[6:]))   # needs_input_grad ignores no_grad
         save = ("ckpt" if model._checkpointing else "full") if need else False
-        a, s_enc = eng.encode(P, x, dtype, save)
-        y, s_dec = eng.decode(P, a, dtype, save)
+        a, s_enc = eng.encode(P, x, dtype, save, A)
+        y, s_dec = eng.decode(P, a, dtype, save, A)
         if need:
-            ctx.model, ctx.dtype, ctx.keys, ctx.saved = model, dtype, keys, (s_enc, s_dec)
+            ctx.model, ctx.dtype, ctx.keys, ctx.saved, ctx.A = model, dtype, keys, (s_enc, s_dec), A
             ctx.save_for_backward(*params)
         return y
 
     @staticmethod
     def backward(ctx, dy):
-        eng, dtype, keys = ctx.model._engine, ctx.dtype, ctx.keys
+        eng, dtype, keys, A = ctx.model._engine, ctx.dtype, ctx.keys, ctx.A
         P = dict(zip(keys, ctx.saved_tensors))
         s_enc, s_dec = ctx.saved
         # the optimizer registered the views of its flat gradient buffer (EnhancedCycleGAN._build_optimizers): accumulate there
         # directly and hand autograd nothing to add
         sinks = getattr(ctx.model, "_grad_sinks", None)
-        use_sink = sinks is not None and all(ctx.needs_input_grad[5:]) and all(k in sinks for k in keys)
+        use_sink = sinks is not None and all(ctx.needs_input_grad[6:]) and all(k in sinks for k in keys)
         G = eng.grad_sink(sinks, dy.device) if use_sink else {}
         dy = dy.contiguous().float()
-        da = eng.decode_bwd(P, G, s_dec, dy, dtype)
-        dx = eng.encode_bwd(P, G, s_enc, da, dtype, need_dx=ctx.needs_input_grad[4])
-        ctx.saved = None
+        if A is not None:
+            eng.style_affine_begin_bwd(A)
+        da = eng.decode_bwd(P, G, s_dec, dy, dtype, A)
+        dx = eng.encode_bwd(P, G, s_enc, da, dtype, need_dx=ctx.needs_input_grad[5], A=A)
+        if A is not None:
+            eng.style_affine_end_bwd(G, A)
+        ctx.saved = ctx.A = None
         if use_sink:
             eng.grad_sink_done(G)
-            return (None, None, None, None, dx) + (None,) * len(keys)
-        grads = tuple(G.get(k) if ctx.needs_input_grad[5 + i] else None for i, k in enumerate(keys))
-        return (None, None, None, None, dx) + grads
+            return (None, None, None, None, None, dx) + (None,) * len(keys)
+        grads = tuple(G.get(k) if ctx.needs_input_grad[6 + i] else None for i, k in enumerate(keys))
+        return (None, None, None, None, None, dx) + grads
 
 
 class _EncoderFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, model, dtype, keys, grad_on, x, *params):
+    def forward(ctx, model, dtype, keys, grad_on, A, x, *params):
         eng = model._engine
         P = dict(zip(keys, params))
-        need = grad_on and (ctx.needs_input_grad[4] or any(ctx.needs_input_grad[5:]))   # needs_input_grad ignores no_grad
+        need = grad_on and (ctx.needs_input_grad[5] or any(ctx.needs_input_grad[6:]))   # needs_input_grad ignores no_grad
         save = ("ckpt" if model._checkpointing else "full") if need else False
-        a, s_enc = eng.encode(P, x, dtype, save)
+        a, s_enc = eng.encode(P, x, dtype, save, A)
         if need:
-            ctx.model, ctx.dtype, ctx.keys, ctx.saved = model, dtype, keys, s_enc
+            ctx.model, ctx.dtype, ctx.keys, ctx.saved, ctx.A = model, dtype, keys, s_enc, A
             ctx.save_for_backward(*params)
         return a.float()  # [N,h,w,4c] tokens-major, fp32 for the user's blocks
 
     @staticmethod
     def backward(ctx, da):
-        eng, dtype, keys = ctx.model._engine, ctx.dtype, ctx.keys
+        eng, dtype, keys, A = ctx.model._engine, ctx.dtype, ctx.keys, ctx.A
         P = dict(zip(keys, ctx.saved_tensors))
         G = {}
-        dx = eng.encode_bwd(P, G, ctx.saved, da.contiguous().to(dtype), dtype, need_dx=ctx.needs_input_grad[4])
-        ctx.saved = None
-        return (None, None, None, None, dx) + tuple(G.get(k) for k in keys)
+        if A is not None:
+            eng.style_affine_begin_bwd(A)
+        dx = eng.encode_bwd(P, G, ctx.saved, da.contiguous().to(dtype), dtype, need_dx=ctx.needs_input_grad[5], A=A)
+        if A is not None:
+            eng.style_affine_end_bwd(G, A)
+        ctx.saved = ctx.A = None
+        return (None, None, None, None, None, dx) + tuple(G.get(k) for k in keys)
 
 
 class _DecoderFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, model, dtype, keys, grad_on, a, *params):
+    def forward(ctx, model, dtype, keys, grad_on, A, a, *params):
         eng = model._engine
         P = dict(zip(keys, params))
-        need = grad_on and (ctx.needs_input_grad[4] or any(ctx.needs_input_grad[5:]))   # needs_input_grad ignores no_grad
+        need = grad_on and (ctx.needs_input_grad[5] or any(ctx.needs_input_grad[6:]))   # needs_input_grad ignores no_grad
         save = ("ckpt" if model._checkpointing else "full") if need else False
-        y, s_dec = eng.decode(P, a.contiguous().to(dtype), dtype, save)
+        y, s_dec = eng.decode(P, a.contiguous().to(dtype), dtype, save, A)
         if need:
-            ctx.model, ctx.dtype, ctx.keys, ctx.saved = model, dtype, keys, s_dec
+            ctx.model, ctx.dtype, ctx.keys, ctx.saved, ctx.A = model, dtype, keys, s_dec, A
             ctx.save_for_backward(*params)
         return y
 
     @staticmethod
     def backward(ctx, dy):
-        eng, dtype, keys = ctx.model._engine, ctx.dtype, ctx.keys
+        eng, dtype, keys, A = ctx.model._engine, ctx.dtype, ctx.keys, ctx.A
         P = dict(zip(keys, ctx.saved_tensors))
         G = {}
-        da = eng.decode_bwd(P, G, ctx.saved, dy.contiguous().float(), dtype)
-        ctx.saved = None
-        return (None, None, None, None, da.float()) + tuple(G.get(k) for k in keys)
+        if A is not None:
+            eng.style_affine_begin_bwd(A)
+        da = eng.decode_bwd(P, G, ctx.saved, dy.contiguous().float(), dtype, A)
+        if A is not None:
+            eng.style_affine_end_bwd(G, A)
+        ctx.saved = ctx.A = None
+        return (None, None, None, None, None, da.float()) + tuple(G.get(k) for k in keys)
 
 
 class EnhancedGenerator(nn.Module):
@@ -261,6 +286,7 @@ class EnhancedGenerator(nn.Module):
         self._engine = GeneratorEngine(c)
         self._checkpointing = False
         self.precision = "fp32"
+        self.num_styles = None
 
     def _init_weights(self, m):
         # enhanced_generator.py:152-161 (fan_out of a ConvTranspose2d weight is size(0)*k*k -- the
@@ -288,6 +314,47 @@ class EnhancedGenerator(nn.Module):
         self.precision = precision
         return self
 
+    def enable_style_affine(self, num_styles):
+        """Makes the model style-conditional (conditional instance norm): each of the 25 InstanceNorm holders gets a weight and
+        a bias Parameter [num_styles, C], initialised to 1 and 0 (no RNG draws), and ``forward`` then requires ``style``.
+        The 70 plain state_dict keys keep their order; a plain checkpoint loads with strict=False (the 50 affine keys are
+        then missing and keep their identity init).  Returns self."""
+        S = int(num_styles)
+        if S < 1:
+            raise ValueError(f"num_styles must be >= 1, got {num_styles}")
+        if self.num_styles is not None:
+            raise ValueError(f"the model is already style-conditional ({self.num_styles} styles)")
+        dev = self.initial[0].weight.device
+        for name, _, holders in self._engine.sites:
+            for h in holders:
+                self.get_submodule(h)._enable_style_affine(S, dev)
+        self.num_styles = S
+        self._engine.invalidate()
+        return self
+
+    def _style_mix(self, style, x):
+        """Validates ``style`` before any device work: [S] (one mix for the batch) or [B, S] (one per image), fp32, no grad.
+        Returns it as a tensor (None for a plain model)."""
+        S = self.num_styles
+        if S is None:
+            if style is not None:
+                raise ValueError("style= needs a style-conditional model: call enable_style_affine(num_styles) first")
+            return None
+        if style is None:
+            raise ValueError(f"this model is style-conditional ({S} styles): pass style= ([{S}] or [B, {S}] weights)")
+        if isinstance(style, torch.Tensor):
+            if style.requires_grad:
+                raise ValueError("style must not require grad: gradients w.r.t. the style weights are not computed")
+            if style.dtype != torch.float32:
+                raise ValueError(f"style must be float32, got {style.dtype}")
+            w = style
+        else:
+            w = torch.as_tensor(style, dtype=torch.float32)
+        B = x.shape[0] if isinstance(x, torch.Tensor) and x.dim() == 4 else None
+        if not ((w.dim() == 1 and w.shape[0] == S) or (w.dim() == 2 and tuple(w.shape) == (B, S))):
+            raise ValueError(f"style must be [{S}] or [{B}, {S}], got {tuple(w.shape)}")
+        return w
+
     def invalidate_packed_weights(self):
         """Call after mutating parameters through raw pointers (the fused Adam does)."""
         self._engine.invalidate()
@@ -304,7 +371,10 @@ class EnhancedGenerator(nn.Module):
     def _blocks_are_identity(self):
         return all(type(b) is StructuralTransformerBlock for b in self.transformer_blocks)
 
-    def forward(self, x):
+    def forward(self, x, style=None):
+        """style: the style mix of a conditional model (enable_style_affine), fp32 [S] or [B, S] on the host or the device,
+        used as given (no normalisation); a plain model takes none."""
+        w = self._style_mix(style, x)
         _check_input(x, "EnhancedGenerator")
         dtype = _resolve_dtype(self.precision)
         keys, params = self._kernel_params()
@@ -314,16 +384,20 @@ class EnhancedGenerator(nn.Module):
         # (passed as an argument, not stored on the module: forward stays re-entrant across threads, gan_login_gui.py:755-767)
         grad_on = torch.is_grad_enabled()
         with torch.cuda.device(x.device):      # kernels launch on the tensors' device, whatever the caller's current device is
+            A = None
+            if w is not None:                  # the per-image affine tables of all 13 norm sites: one launch per call
+                w = w.to(x.device).expand(x.shape[0], self.num_styles).contiguous()
+                A = self._engine.style_tables(dict(zip(keys, params)), w)
             if self._blocks_are_identity():
                 # style_encoder output is only consumed by the (identity) blocks: dead, skipped
-                return _GeneratorFn.apply(self, dtype, keys, grad_on, xin.contiguous(), *params)
-            a = _EncoderFn.apply(self, dtype, keys, grad_on, xin.contiguous(), *params)     # [B,h,w,4c]
+                return _GeneratorFn.apply(self, dtype, keys, grad_on, A, xin.contiguous(), *params)
+            a = _EncoderFn.apply(self, dtype, keys, grad_on, A, xin.contiguous(), *params)     # [B,h,w,4c]
             B, h, w, C = a.shape
             style = self.style_encoder[3](self.style_encoder[2](a.mean(dim=(1, 2))))  # :142-147, :216
             t = a.reshape(B, h * w, C)                                                # :218-219
             for block in self.transformer_blocks:
                 t = block(t, style, x)                                                # :222-223
-            return _DecoderFn.apply(self, dtype, keys, grad_on, t.reshape(B, h, w, C), *params)
+            return _DecoderFn.apply(self, dtype, keys, grad_on, A, t.reshape(B, h, w, C), *params)
 
     def load_state_dict(self, state_dict, strict=True, **kw):
         out = super().load_state_dict(state_dict, strict=strict, **kw)

@@ -47,6 +47,42 @@ class _StatsArena:
         return t
 
 
+def norm_sites(c):
+    """The 13 InstanceNorm apply sites of a generator of width c in forward order: (site, channels, affine holders).  The four
+    branch norms of a MultiScaleBlock are one apply over the concatenated branches, so their holders share one site, in branch
+    order."""
+    width = {"down1": 2 * c, "down2": 4 * c, "up1": 2 * c, "up2": c}
+    sites = [("initial.1", c, ("initial.1",))]
+    for s in STAGES:
+        C = width[s]
+        sites += [(f"{s}.1", C, (f"{s}.1",)),
+                  (f"{s}.4.branch", C, tuple(f"{s}.4.branch{i}.1" for i in range(1, 5))),
+                  (f"{s}.4.fusion.1", C, (f"{s}.4.fusion.1",))]
+    return sites
+
+
+class StyleAffine:
+    """Per-image InstanceNorm affines of one conditional forward: the mix w [N, S] and the tables gamma / beta [N, Ct] fp32 that
+    msg_style_affine built from it, one column range per norm site (`off`).  The backward of the same forward reads them again
+    (checkpointed recompute included) and collects the per-image affine gradients of all sites in one fp64 arena `sums`."""
+
+    def __init__(self, w, gamma, beta, off):
+        self.w, self.gamma, self.beta, self.off = w, gamma, beta, off
+        self.sums = None
+
+    def at(self, site):
+        """(gamma, beta, img_stride) of a site, the C-ABI's affine argument (include/msg_b200.h)"""
+        o = self.off[site]
+        return self.gamma.view(-1)[o:], self.beta.view(-1)[o:], self.gamma.shape[1]
+
+    def sums_at(self, site):
+        return self.sums[2 * self.off[site]:]
+
+
+def _site(A, name):
+    return None if A is None else A.at(name)
+
+
 class GradSink(dict):
     """Parameter gradients accumulated straight into caller-owned fp32 buffers -- the views of the optimizer's flat gradient
     buffer -- instead of fresh tensors that autograd then adds to .grad: per conv that was a zeros() for the packed gradient, a
@@ -124,6 +160,12 @@ class GeneratorEngine:
         self.fuse_in_norm = os.environ.get("MSG_FUSE_IN_NORM", "1") == "1"
         self.fuse_la = os.environ.get("MSG_FUSE_LA", "1") == "1"      # fused LocalAttention stage kernel (inference)
         self._arena_floats = 0          # packed-gradient floats of one backward (measured on the first one)
+        # style-conditional models (EnhancedGenerator.enable_style_affine): column ranges of the norm sites in the affine tables
+        self.sites = norm_sites(c)
+        self.site_off, self.Ct = {}, 0
+        for name, C, _ in self.sites:
+            self.site_off[name] = self.Ct
+            self.Ct += C
 
     def _versions(self, params, names):
         return tuple((params[n].data_ptr(), params[n]._version) for n in names)
@@ -177,8 +219,54 @@ class GeneratorEngine:
             b = _pad_dim(b, 0, self.edge_pad(dtype))
         return b.contiguous()
 
+    # ---- style affine --------------------------------------------------------------------------
+    def _holder_columns(self):
+        """(holder, first column, channels) of the 25 affine holders in table order"""
+        for name, C, holders in self.sites:
+            q = C // len(holders)
+            for i, h in enumerate(holders):
+                yield h, self.site_off[name] + i * q, q
+
+    def style_tables(self, P, w):
+        """w: fp32 [N, S] mix on the device -> StyleAffine (one msg_style_affine launch).  The holders' [S, C] parameters are
+        packed into [S, Ct] once per parameter version, like the weight packs."""
+        hs = [h for h, _, _ in self._holder_columns()]
+        tabs = []
+        for which in ("weight", "bias"):
+            names = [f"{h}.{which}" for h in hs]
+            tabs.append(self._slab_cached(P, ("style_affine", which), names,
+                                          lambda: torch.cat([P[k].detach() for k in names], 1).contiguous()))
+        g, b = ops.style_affine(w, *tabs)
+        return StyleAffine(w, g, b, self.site_off)
+
+    def style_affine_begin_bwd(self, A):
+        A.sums = torch.zeros(A.w.shape[0] * self.Ct * 2, device=A.w.device, dtype=torch.float64)
+
+    def style_affine_end_bwd(self, G, A):
+        """One msg_style_affine_bwd over the backward's sums arena -> the [S, C] gradients of the holders into G."""
+        S = A.w.shape[1]
+        dg = torch.zeros((S, self.Ct), device=A.w.device, dtype=torch.float32)
+        db = torch.zeros_like(dg)
+        ops.style_affine_bwd(A.sums, A.w, dg, db)
+        A.sums = None
+        for h, o, q in self._holder_columns():
+            for k, t in ((f"{h}.weight", dg[:, o:o + q]), (f"{h}.bias", db[:, o:o + q])):
+                if isinstance(G, GradSink):
+                    G.sinks[k].add_(t)
+                else:
+                    G[k] = t if k not in G else G[k] + t
+
+    def _in_bwd(self, x, st, dy, A, site):
+        """Backward of ReLU(IN(x)) at one norm site; conditional: reduce -> apply with the forward's per-image affine, the
+        reductions (d beta_n, d gamma_n) landing in the site's columns of the sums arena."""
+        if A is None:
+            return ops.instnorm_bwd(x, st, dy, ACT_RELU)
+        aff, sums = A.at(site), A.sums_at(site)
+        ops.instnorm_bwd_reduce_affine(x, st, dy, aff, sums, ACT_RELU)
+        return ops.instnorm_bwd_apply_affine(x, st, dy, sums, aff, ACT_RELU)
+
     # ---- forward ---------------------------------------------------------------------------------
-    def _stage_fwd(self, P, s, a_in, dtype, keep=True, arena=None, defer_apply=False):
+    def _stage_fwd(self, P, s, a_in, dtype, keep=True, arena=None, defer_apply=False, A=None):
         """keep=False (inference): intermediates are dropped as soon as their consumer has been
         launched, so the caching allocator recycles them within the stage."""
         g = self.geom
@@ -195,7 +283,7 @@ class GeneratorEngine:
             yi, sti = a_in
             wn = f"{s}.0.weight"
             wsl = self._slab_cached(P, (s, "down_ring_w"), [wn], lambda: slab.down_ring_weights(P[wn].detach()))
-            y0 = slab.down_ring(yi, sti, wsl, self._bias(P, f"{s}.0"), C, stats=st0)
+            y0 = slab.down_ring(yi, sti, wsl, self._bias(P, f"{s}.0"), C, stats=st0, in_affine=_site(A, "initial.1"))
         elif (self.convT_ring and g[f"{s}.0"].kind == "convT" and dtype == torch.bfloat16 and self.inwidth[s] in (64, 128) and C % 64 == 0):
             # transposed conv as a row ring of TMEM accumulators (csrc/convt_ring.cu): one launch per horizontal output phase, every
             # input row loaded once per launch, the four vertical taps of a horizontal tap as one N = 256 MMA.  128 -> 64 at 256^2:
@@ -222,16 +310,18 @@ class GeneratorEngine:
             # inference, C in {64, 128}: the whole LocalAttention stage -- IN + ReLU of y0 on the landed tile, qkv 1x1, window
             # attention with S / P in tensor memory, proj 1x1 -- is ONE tcgen05 launch; qkv and the attention output never
             # exist in HBM (csrc/la_stage.cu)
-            a1 = ops.la_stage_fwd(y0, wq, self._bias(P, f"{s}.3.qkv"), wp, self._bias(P, f"{s}.3.proj"), in_stats=st0, in_act=ACT_RELU)
+            a1 = ops.la_stage_fwd(y0, wq, self._bias(P, f"{s}.3.qkv"), wp, self._bias(P, f"{s}.3.proj"), in_stats=st0, in_act=ACT_RELU,
+                                  in_affine=_site(A, f"{s}.1"))
             del y0
-            return self._msb_fwd(P, s, a1, None, dtype, keep, arena, g, C, defer_apply)
+            return self._msb_fwd(P, s, a1, None, dtype, keep, arena, g, C, defer_apply, A)
         if not keep and self.fuse_in_norm and g[f"{s}.3.qkv"].fused_in_norm_ok(y0, wq):
             # inference: ReLU(IN(y0)) has ONE consumer, the 1x1 qkv conv (LocalAttention has no residual), so the
             # conv normalises its A tiles in shared memory and the normalised tensor never exists in HBM
             a0 = None
-            qkv = g[f"{s}.3.qkv"].forward(y0, wq, self._bias(P, f"{s}.3.qkv"), in_stats=st0, in_act=ACT_RELU)
+            qkv = g[f"{s}.3.qkv"].forward(y0, wq, self._bias(P, f"{s}.3.qkv"), in_stats=st0, in_act=ACT_RELU,
+                                          in_affine=_site(A, f"{s}.1"))
         else:
-            a0 = ops.instnorm_apply(y0, st0, ACT_RELU, out=None if keep else y0)
+            a0 = ops.instnorm_apply(y0, st0, ACT_RELU, out=None if keep else y0, affine=_site(A, f"{s}.1"))
             qkv = g[f"{s}.3.qkv"].forward(a0, wq, self._bias(P, f"{s}.3.qkv"))
         att = ops.local_attn_fwd(qkv)
         if not keep:
@@ -239,10 +329,10 @@ class GeneratorEngine:
         a1 = g[f"{s}.3.proj"].forward(att, wp, self._bias(P, f"{s}.3.proj"))
         if not keep:
             del att
-            return self._msb_fwd(P, s, a1, None, dtype, keep, arena, g, C, defer_apply)
-        return self._msb_fwd(P, s, a1, dict(a_in=a_in, y0=y0, st0=st0, a0=a0, qkv=qkv, att=att), dtype, keep, arena, g, C)
+            return self._msb_fwd(P, s, a1, None, dtype, keep, arena, g, C, defer_apply, A)
+        return self._msb_fwd(P, s, a1, dict(a_in=a_in, y0=y0, st0=st0, a0=a0, qkv=qkv, att=att), dtype, keep, arena, g, C, A=A)
 
-    def _msb_fwd(self, P, s, a1, saved, dtype, keep, arena, g, C, defer_apply=False):
+    def _msb_fwd(self, P, s, a1, saved, dtype, keep, arena, g, C, defer_apply=False, A=None):
         """MultiScaleBlock of stage s on a1 (enhanced_generator.py:78-84)."""
         dev = a1.device
         b = torch.empty_like(a1)
@@ -274,21 +364,21 @@ class GeneratorEngine:
         wf = self._packed(P, n, "fwd", dtype)
         if not keep and self.fuse_in_norm and g[n].fused_in_norm_ok(b, wf):
             bn = None       # ReLU(IN(branches)) is consumed only by the 1x1 fusion conv: normalised on the fly
-            f = g[n].forward(b, wf, self._bias(P, n), stats=stf, in_stats=stb, in_act=ACT_RELU)
+            f = g[n].forward(b, wf, self._bias(P, n), stats=stf, in_stats=stb, in_act=ACT_RELU, in_affine=_site(A, f"{s}.4.branch"))
         else:
-            bn = ops.instnorm_apply(b, stb, ACT_RELU, out=None if keep else b)
+            bn = ops.instnorm_apply(b, stb, ACT_RELU, out=None if keep else b, affine=_site(A, f"{s}.4.branch"))
             f = g[n].forward(bn, wf, self._bias(P, n), stats=stf)
         if defer_apply and not keep:
             # the stage's last IN + ReLU + residual is applied by its consumer on the landed row slabs (csrc/out7_ring.cu)
             return (f, stf, a1), None
-        a2 = ops.instnorm_apply(f, stf, ACT_RELU, residual=a1, out=None if keep else f)
+        a2 = ops.instnorm_apply(f, stf, ACT_RELU, residual=a1, out=None if keep else f, affine=_site(A, f"{s}.4.fusion.1"))
         if not keep:
             return a2, None
         saved.update(a1=a1, b=b, stb=stb, bn=bn, f=f, stf=stf)
         return a2, saved
 
-    def encode(self, P, x, dtype, save):
-        """x: fp32 NCHW image -> (a [N,H/4,W/4,4c] NHWC, saved)."""
+    def encode(self, P, x, dtype, save, A=None):
+        """x: fp32 NCHW image -> (a [N,H/4,W/4,4c] NHWC, saved).  A: the StyleAffine of a conditional model, else None."""
         N, Cx, H, W = x.shape
         if Cx != 3:
             raise RuntimeError(f"EnhancedGenerator expects 3 input channels, got {Cx}")
@@ -309,16 +399,16 @@ class GeneratorEngine:
         if not save and self.down_ring and dtype == torch.bfloat16 and self.c == 64 and self.use_slab and H % 2 == 0 and W % 2 == 0:
             a = (yi, sti)           # applied by down1's first conv (csrc/down_ring.cu)
         else:
-            a = ops.instnorm_apply(yi, sti, ACT_RELU, out=None if save else yi)
+            a = ops.instnorm_apply(yi, sti, ACT_RELU, out=None if save else yi, affine=_site(A, "initial.1"))
         saved = {"x0": x0, "yi": yi, "sti": sti} if save else None
         for s in ("down1", "down2"):
             a_in = a
-            a, sv = self._stage_fwd(P, s, a_in, dtype, keep=(save == "full"), arena=arena)
+            a, sv = self._stage_fwd(P, s, a_in, dtype, keep=(save == "full"), arena=arena, A=A)
             if save:
                 saved[s] = sv if save == "full" else {"a_in": a_in}
         return a, saved
 
-    def decode(self, P, a, dtype, save):
+    def decode(self, P, a, dtype, save, A=None):
         """a: [N,H/4,W/4,4c] NHWC -> (y fp32 NCHW in [-1,1], saved)."""
         saved = {} if save else None
         arena = _StatsArena(a.shape[0], 3 * (self.width["up1"] + self.width["up2"]), a.device)
@@ -327,7 +417,7 @@ class GeneratorEngine:
         fuse_out = (not save and self.out7_ring and dtype == torch.bfloat16 and self.c == 64 and self.use_slab)
         for s in ("up1", "up2"):
             a_in = a
-            a, sv = self._stage_fwd(P, s, a_in, dtype, keep=(save == "full"), arena=arena, defer_apply=(fuse_out and s == "up2"))
+            a, sv = self._stage_fwd(P, s, a_in, dtype, keep=(save == "full"), arena=arena, defer_apply=(fuse_out and s == "up2"), A=A)
             if save:
                 saved[s] = sv if save == "full" else {"a_in": a_in}
         if isinstance(a, tuple):
@@ -335,7 +425,7 @@ class GeneratorEngine:
             N, H, W, _ = f.shape
             y = torch.empty((N, 3, H, W), device=f.device, dtype=torch.float32)
             wsl = self._slab_cached(P, ("output", "ring_w"), ["output.0.weight"], lambda: slab.out7_ring_weights(P["output.0.weight"].detach()))
-            slab.out7_ring(f, stf, a1, wsl, P["output.0.bias"].detach().contiguous(), nchw_out=y)
+            slab.out7_ring(f, stf, a1, wsl, P["output.0.bias"].detach().contiguous(), nchw_out=y, in_affine=_site(A, "up2.4.fusion.1"))
             return y, saved
         N, H, W, _ = a.shape
         y = torch.empty((N, 3, H, W), device=a.device, dtype=torch.float32)
@@ -404,13 +494,13 @@ class GeneratorEngine:
         return g.dgrad(dy, self._packed(P, name, "dgrad", dtype), in_hw or x.shape[1:3], out=dx_out,
                        accumulate=accumulate, dy_c_off=dy_c_off)
 
-    def _stage_bwd(self, P, G, s, sv, da2, dtype):
+    def _stage_bwd(self, P, G, s, sv, da2, dtype, A=None):
         if "y0" not in sv:  # checkpointed: recompute the stage from its input (enhanced_generator.py:186-208)
-            _, sv = self._stage_fwd(P, s, sv["a_in"], dtype, keep=True)
+            _, sv = self._stage_fwd(P, s, sv["a_in"], dtype, keep=True, A=A)
         C = self.width[s]
-        df = ops.instnorm_bwd(sv["f"], sv["stf"], da2, ACT_RELU)
+        df = self._in_bwd(sv["f"], sv["stf"], da2, A, f"{s}.4.fusion.1")
         dbn = self._conv_bwd(P, G, f"{s}.4.fusion.0", sv["bn"], df, dtype)
-        db = ops.instnorm_bwd(sv["b"], sv["stb"], dbn, ACT_RELU)
+        db = self._in_bwd(sv["b"], sv["stb"], dbn, A, f"{s}.4.branch")
         if self.use_slab and dtype == torch.bfloat16 and C in self._msb_dprog and db.shape[2] % 8 == 0:
             # data gradient of the four branches: one row-slab launch (N = C per tap) + the residual add
             wn = [f"{s}.4.branch{i}.0.weight" for i in range(1, 5)]
@@ -427,7 +517,7 @@ class GeneratorEngine:
         datt = self._conv_bwd(P, G, f"{s}.3.proj", sv["att"], da1, dtype)
         dqkv = ops.local_attn_bwd(sv["qkv"], datt)
         da0 = self._conv_bwd(P, G, f"{s}.3.qkv", sv["a0"], dqkv, dtype)
-        dy0 = ops.instnorm_bwd(sv["y0"], sv["st0"], da0, ACT_RELU)
+        dy0 = self._in_bwd(sv["y0"], sv["st0"], da0, A, f"{s}.1")
         return self._conv_bwd(P, G, f"{s}.0", sv["a_in"], dy0, dtype)
 
     def grad_sink(self, sinks, device):
@@ -437,18 +527,19 @@ class GeneratorEngine:
     def grad_sink_done(self, G):
         self._arena_floats = max(self._arena_floats, G.used)
 
-    def decode_bwd(self, P, G, saved, dy, dtype):
-        """dy: fp32 NCHW grad of the image.  Returns d(a) at the decoder input (NHWC)."""
+    def decode_bwd(self, P, G, saved, dy, dtype, A=None):
+        """dy: fp32 NCHW grad of the image.  Returns d(a) at the decoder input (NHWC).  A: the forward's StyleAffine, its sums
+        arena allocated (style_affine_begin_bwd)."""
         dz = ops.tanh_bwd_nchw(saved["y"], dy, dtype, self.edge_pad(dtype))
         da = self._conv_bwd(P, G, "output.0", saved["a_last"], dz, dtype)
         for s in ("up2", "up1"):
-            da = self._stage_bwd(P, G, s, saved[s], da, dtype)
+            da = self._stage_bwd(P, G, s, saved[s], da, dtype, A)
         return da
 
-    def encode_bwd(self, P, G, saved, da, dtype, need_dx):
+    def encode_bwd(self, P, G, saved, da, dtype, need_dx, A=None):
         for s in ("down2", "down1"):
-            da = self._stage_bwd(P, G, s, saved[s], da, dtype)
-        dyi = ops.instnorm_bwd(saved["yi"], saved["sti"], da, ACT_RELU)
+            da = self._stage_bwd(P, G, s, saved[s], da, dtype, A)
+        dyi = self._in_bwd(saved["yi"], saved["sti"], da, A, "initial.1")
         dx0 = self._conv_bwd(P, G, "initial.0", saved["x0"], dyi, dtype, need_dx=need_dx)
         if not need_dx:
             return None

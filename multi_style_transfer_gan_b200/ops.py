@@ -52,8 +52,21 @@ def _dev(t):
     _lib.require_device(idx)
 
 
-def conv_raw(desc, x, w, bias, y, stats=None, in_stats=None):
-    _lib.call("msg_conv2d", ctypes.byref(desc), _p(x), _p(w), _p(bias), _p(y), _p(stats), _p(in_stats), _stream())
+def _aff(affine):
+    """(gamma, beta, img_stride) of an optional InstanceNorm affine -> C-ABI arguments (include/msg_b200.h); gamma / beta are
+    fp32 device tensors whose first element is that of image 0, channel 0 of the site."""
+    if affine is None:
+        return None, None, 0
+    g, b, stride = affine
+    return _p(g), _p(b), int(stride)
+
+
+def conv_raw(desc, x, w, bias, y, stats=None, in_stats=None, in_affine=None):
+    if in_affine is None:
+        _lib.call("msg_conv2d", ctypes.byref(desc), _p(x), _p(w), _p(bias), _p(y), _p(stats), _p(in_stats), _stream())
+    else:
+        _lib.call("msg_conv2d_affine", ctypes.byref(desc), _p(x), _p(w), _p(bias), _p(y), _p(stats), _p(in_stats), *_aff(in_affine),
+                  _stream())
 
 
 def make_desc(dt, N, Hi, Wi, Ci_total, ci_off, Cin, Ho, Wo, Co_total, co_off, Cout, Hg, Wg, KH, KW,
@@ -139,9 +152,10 @@ class ConvGeom:
 
     # ---- launches
     def forward(self, x, wp, bias, out=None, co_off=0, stats=None, act=ACT_NONE, in_stats=None,
-                in_act=ACT_NONE, ci_off=0, nchw_out=None, extra_flags=0):
+                in_act=ACT_NONE, ci_off=0, nchw_out=None, extra_flags=0, in_affine=None):
         """x: [N,Hi,Wi,Ci_total].  Writes channels [co_off, co_off+Cout) of `out` [N,Ho,Wo,Co_total]
-        (allocated if None).  nchw_out: fp32 [N,Cout,Ho,Wo] tensor to write instead (final image)."""
+        (allocated if None).  nchw_out: fp32 [N,Cout,Ho,Wo] tensor to write instead (final image).
+        in_affine: (gamma, beta, img_stride) of the fused input norm (TMA kernel only, see fused_in_norm_ok)."""
         _dev(x)
         N, Hi, Wi, Ci_total = x.shape
         Ho, Wo = self.out_hw(Hi, Wi)
@@ -162,14 +176,14 @@ class ConvGeom:
             d = make_desc(dt, N, Hi, Wi, Ci_total, ci_off, self.Cin, Ho, Wo, Co_total, co_off, self.Cout,
                           Ho, Wo, self.k, self.k, self.stride, self.pad, self.pad, self.dil, 1, 0, 0, act,
                           flags, in_act)
-            conv_raw(d, x, wp, bias, y, stats, in_stats)
+            conv_raw(d, x, wp, bias, y, stats, in_stats, in_affine)
         else:
             per_phase = self.Cout * 4 * self.Cin
             for ph in range(2):
                 for pw in range(2):
                     d = make_desc(dt, N, Hi, Wi, Ci_total, ci_off, self.Cin, Ho, Wo, Co_total, co_off,
                                   self.Cout, Hi, Wi, 2, 2, 1, 1 - ph, 1 - pw, 1, 2, ph, pw, act, flags, in_act)
-                    conv_raw(d, x, wp[(ph * 2 + pw) * per_phase:], bias, y, stats, in_stats)
+                    conv_raw(d, x, wp[(ph * 2 + pw) * per_phase:], bias, y, stats, in_stats, in_affine)
         return nchw_out if nchw_out is not None else out
 
     def dgrad(self, dy, wpd, in_hw, out=None, co_off=0, accumulate=False, dy_c_off=0):
@@ -254,14 +268,19 @@ def instnorm_stats(x, stats=None):
     return stats
 
 
-def instnorm_apply(x, stats, act=ACT_RELU, residual=None, out=None, gammas=None, betas=None, w=None):
+def instnorm_apply(x, stats, act=ACT_RELU, residual=None, out=None, gammas=None, betas=None, w=None, affine=None):
+    """affine: (gamma, beta, img_stride) table (include/msg_b200.h) instead of the blend of gammas / betas by w."""
     _dev(x)
     N, H, W, C = x.shape
     if out is None:
         out = torch.empty_like(x)
     S = 0 if gammas is None else gammas.shape[0]
-    _lib.call("msg_instnorm_apply", _dt(x), _p(x), _p(stats), N, H * W, C, act, _p(residual), S,
-              _p(gammas), _p(betas), _p(w), _p(out), _stream())
+    if affine is None:
+        _lib.call("msg_instnorm_apply", _dt(x), _p(x), _p(stats), N, H * W, C, act, _p(residual), S,
+                  _p(gammas), _p(betas), _p(w), _p(out), _stream())
+    else:
+        _lib.call("msg_instnorm_apply_affine", _dt(x), _p(x), _p(stats), N, H * W, C, act, _p(residual), S,
+                  _p(gammas), _p(betas), _p(w), *_aff(affine), _p(out), _stream())
     return out
 
 
@@ -310,6 +329,44 @@ def instnorm_bwd_apply(x, stats, dy, sums, act=ACT_RELU, gamma=None, beta=None, 
     return out
 
 
+def instnorm_bwd_reduce_affine(x, stats, dy, affine, sums, act=ACT_RELU):
+    """instnorm_bwd_reduce with a per-image affine (gamma, beta, img_stride): writes the (sum g, sum g * xhat) = (d beta_n,
+    d gamma_n) of its C channels into `sums`, a flat fp64 view whose rows are img_stride channels apart (the layout of the
+    affine tables)."""
+    _dev(x)
+    N, H, W, C = x.shape
+    _lib.call("msg_instnorm_bwd_reduce_affine", _dt(x), _p(x), _p(stats), _p(dy), N, H * W, C, act, *_aff(affine), _p(sums),
+              _stream())
+    return sums
+
+
+def instnorm_bwd_apply_affine(x, stats, dy, sums, affine, act=ACT_RELU, out=None):
+    _dev(x)
+    N, H, W, C = x.shape
+    if out is None:
+        out = torch.empty_like(x)
+    _lib.call("msg_instnorm_bwd_apply_affine", _dt(x), _p(x), _p(stats), _p(dy), N, H * W, C, act, *_aff(affine), _p(sums),
+              _p(out), _stream())
+    return out
+
+
+def style_affine(w, gammas, betas):
+    """Per-image affine tables gamma / beta [N, Ct] = w [N, S] @ gammas / betas [S, Ct] (msg_style_affine: fmaf chain over s)."""
+    _dev(w)
+    N, S = w.shape
+    Ct = gammas.shape[1]
+    g = torch.empty((N, Ct), device=w.device, dtype=torch.float32)
+    b = torch.empty_like(g)
+    _lib.call("msg_style_affine", _p(w), N, S, _p(gammas), _p(betas), Ct, _p(g), _p(b), _stream())
+    return g, b
+
+
+def style_affine_bwd(sums, w, dgammas, dbetas):
+    """dgammas / dbetas [S, Ct] += the gradients of style_affine's tables from one sums arena [N, Ct, 2] fp64."""
+    N, S = w.shape
+    _lib.call("msg_style_affine_bwd", _p(sums), _p(w), N, S, dgammas.shape[1], _p(dgammas), _p(dbetas), _stream())
+
+
 # ---- LocalAttention core -------------------------------------------------------------------------
 def local_attn_fwd(qkv, ws=4):
     _dev(qkv)
@@ -335,7 +392,7 @@ def la_stage_supported(x, wqkv, wproj):
     return _lib.load().msg_la_stage_supported(_dt(x), N, H, W, C, _p(x), _p(wqkv), _p(wproj), _p(x)) == 1
 
 
-def la_stage_fwd(x, wqkv, bqkv, wproj, bproj, in_stats=None, in_act=ACT_NONE, out=None):
+def la_stage_fwd(x, wqkv, bqkv, wproj, bproj, in_stats=None, in_act=ACT_NONE, out=None, in_affine=None):
     """LocalAttention.forward (enhanced_generator.py:13-47) in one launch: [IN + act of the producer] -> qkv 1x1 ->
     4x4-window channel attention -> proj 1x1.  x: [N,H,W,C] bf16 (raw conv output with `in_stats`, else normalised);
     wqkv / wproj: packed bf16 1x1 weights ([3C][C], [C][C]); biases fp32."""
@@ -343,8 +400,12 @@ def la_stage_fwd(x, wqkv, bqkv, wproj, bproj, in_stats=None, in_act=ACT_NONE, ou
     N, H, W, C = x.shape
     if out is None:
         out = torch.empty_like(x)
-    _lib.call("msg_la_stage_fwd", _dt(x), _p(x), _p(in_stats), in_act, _p(wqkv), _p(bqkv), _p(wproj), _p(bproj), N, H, W, C,
-              _p(out), _stream())
+    if in_affine is None:
+        _lib.call("msg_la_stage_fwd", _dt(x), _p(x), _p(in_stats), in_act, _p(wqkv), _p(bqkv), _p(wproj), _p(bproj), N, H, W, C,
+                  _p(out), _stream())
+    else:
+        _lib.call("msg_la_stage_fwd_affine", _dt(x), _p(x), _p(in_stats), *_aff(in_affine), in_act, _p(wqkv), _p(bqkv), _p(wproj),
+                  _p(bproj), N, H, W, C, _p(out), _stream())
     return out
 
 

@@ -610,9 +610,9 @@ def out7_ring_weights(w, dtype=torch.bfloat16):
     return out.reshape(7 * 128, 64).to(dtype).contiguous()
 
 
-def out7_ring(f, in_stats, residual, w_stacks, bias, nchw_out=None):
+def out7_ring(f, in_stats, residual, w_stacks, bias, nchw_out=None, in_affine=None):
     """y = tanh(conv7x7(residual + ReLU(IN(f))) + bias): f, residual [N,H,W,64] bf16, in_stats fp64 [N,64,2] (raw plane sums of f)
-    -> fp32 [N,3,H,W]."""
+    -> fp32 [N,3,H,W].  in_affine: optional (gamma, beta, img_stride) of the IN (ops.instnorm_apply)."""
     ops._dev(f)
     N, H, W, Cf = f.shape
     if f.dtype != torch.bfloat16 or residual.dtype != torch.bfloat16 or residual.shape[:3] != f.shape[:3]:
@@ -624,8 +624,12 @@ def out7_ring(f, in_stats, residual, w_stacks, bias, nchw_out=None):
     d = _lib.Out7RingDesc()
     d.dtype, d.N, d.H, d.W = _lib.BF16, N, H, W
     d.Cf_total, d.cf_off, d.Cr_total, d.cr_off, d.Cs_total, d.cs_off = Cf, 0, residual.shape[3], 0, in_stats.shape[1], 0
-    _lib.call("msg_out7_ring", ctypes.byref(d), ops._p(f), ops._p(in_stats), ops._p(residual), ops._p(w_stacks), ops._p(bias),
-              ops._p(nchw_out), ops._stream())
+    if in_affine is None:
+        _lib.call("msg_out7_ring", ctypes.byref(d), ops._p(f), ops._p(in_stats), ops._p(residual), ops._p(w_stacks), ops._p(bias),
+                  ops._p(nchw_out), ops._stream())
+    else:
+        _lib.call("msg_out7_ring_affine", ctypes.byref(d), ops._p(f), ops._p(in_stats), *ops._aff(in_affine), ops._p(residual),
+                  ops._p(w_stacks), ops._p(bias), ops._p(nchw_out), ops._stream())
     return nchw_out
 
 
@@ -674,8 +678,9 @@ def down_ring_weights(w, dtype=torch.bfloat16):
     return torch.cat(out, 0).to(dtype).contiguous()
 
 
-def down_ring(x, in_stats, w_stacks, bias, Cout, out=None, co_off=0, stats=None, ci_off=0):
-    """Conv2d(64, Cout, 4, 2, 1) of ReLU(IN(x)) (in_stats: fp64 [N,C,2] raw plane sums of x; None: x is used as it is):
+def down_ring(x, in_stats, w_stacks, bias, Cout, out=None, co_off=0, stats=None, ci_off=0, in_affine=None):
+    """Conv2d(64, Cout, 4, 2, 1) of ReLU(IN(x)) (in_stats: fp64 [N,C,2] raw plane sums of x; None: x is used as it is; in_affine:
+    optional (gamma, beta, img_stride) of the IN):
     x [N,H,W,>=64] bf16 -> out [N,H/2,W/2,Co_total] bf16 (Cout channels at co_off), IN statistics accumulated into stats."""
     ops._dev(x)
     N, H, W, Ci_total = x.shape
@@ -689,7 +694,11 @@ def down_ring(x, in_stats, w_stacks, bias, Cout, out=None, co_off=0, stats=None,
     d.Ci_total, d.ci_off, d.Co_total, d.co_off = Ci_total, ci_off, out.shape[3], co_off
     d.Cs_total, d.cs_off = (in_stats.shape[1], 0) if in_stats is not None else (0, 0)
     d.flags = _lib.CONV_STATS if stats is not None else 0
-    _lib.call("msg_down_ring", ctypes.byref(d), ops._p(x), ops._p(in_stats), ops._p(w_stacks), ops._p(bias), ops._p(out), ops._p(stats),
-              ops._stream())
+    if in_affine is None:
+        _lib.call("msg_down_ring", ctypes.byref(d), ops._p(x), ops._p(in_stats), ops._p(w_stacks), ops._p(bias), ops._p(out),
+                  ops._p(stats), ops._stream())
+    else:
+        _lib.call("msg_down_ring_affine", ctypes.byref(d), ops._p(x), ops._p(in_stats), *ops._aff(in_affine), ops._p(w_stacks),
+                  ops._p(bias), ops._p(out), ops._p(stats), ops._stream())
     _lib.launches += Cout // 64 - 1                 # one kernel per 64 output channels
     return out

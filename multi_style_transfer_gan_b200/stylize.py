@@ -77,9 +77,10 @@ class MultiStyleStylizer:
         self.use_graph = bool(use_graph)
         self._graphs = {}
 
-    def _forward_chunk(self, xi, weights, w_x, gain, clip, dst, maps=None, normalize=False):
+    def _forward_chunk(self, xi, weights, w_x, gain, clip, dst, maps=None, normalize=False, style=None):
         """All styles of one micro-batch + the blend into dst, enqueued on the current stream (and the style streams).
-        maps: the micro-batch's weight maps [Bm, K, h, w] on the device (per-pixel blend) instead of `weights`."""
+        maps: the micro-batch's weight maps [Bm, K, h, w] on the device (per-pixel blend) instead of `weights`.
+        style: the micro-batch's style mix ([S] or [Bi, S] on the device) for conditional generators."""
         cur = torch.cuda.current_stream(self.device)
         capturing = torch.cuda.is_current_stream_capturing()
         if self.style_streams:
@@ -91,64 +92,71 @@ class MultiStyleStylizer:
             for g, st in zip(self.generators, self._streams):
                 st.wait_event(ready)
                 with torch.cuda.stream(st):
-                    y = g(xi)
+                    y = g(xi) if style is None else g(xi, style=style)
                     ev_s = torch.cuda.Event()
                     ev_s.record(st)
                 if not capturing:                 # (inside a capture the graph's private pool orders reuse itself)
                     xi.record_stream(st)
+                    if style is not None:
+                        style.record_stream(st)
                     y.record_stream(cur)
                 ys.append(y)
                 done.append(ev_s)
             for ev_s in done:
                 cur.wait_event(ev_s)
         else:
-            ys = [g(xi) for g in self.generators]
+            ys = [g(xi) if style is None else g(xi, style=style) for g in self.generators]
         if maps is None:
             ops.blend_outputs(ys, weights, x=xi if w_x != 0.0 else None, w_x=w_x, gain=gain, clip=clip, out=dst)
         else:
             ops.blend_maps(ys, maps, x=xi if maps.shape[1] > len(ys) else None, gain=gain, clip=clip, normalize=normalize,
                            out=dst)
 
-    def _replay(self, xi, weights, w_x, gain, clip, dst, pver=None, maps=None, normalize=False):
+    def _replay(self, xi, weights, w_x, gain, clip, dst, pver=None, maps=None, normalize=False, style=None):
         """CUDA-graph path: the ~210 launches of a micro-batch (S forwards + blend) are captured once per
         (shape, blend parameters) and replayed, so the host cost of a micro-batch is one graph launch.  Weights are
         read through the per-generator pack caches at capture time: `invalidate_graphs()` after changing them.
         Weight maps are a graph input like the images: the key holds their shape and `normalize`, each replay copies the
-        micro-batch's maps into the entry's static buffer."""
+        micro-batch's maps into the entry's static buffer.  So is the style mix of conditional generators: moving a style
+        slider replays the same graph."""
         key = (tuple(xi.shape), tuple(float(w) for w in weights) if maps is None else ("maps", tuple(maps.shape), bool(normalize)),
                float(w_x), float(gain), clip, dst.dtype,
-               pver if pver is not None else tuple(g.param_version() for g in self.generators))
+               pver if pver is not None else tuple(g.param_version() for g in self.generators),
+               None if style is None else ("style", tuple(style.shape)))
         ent = self._graphs.get(key)
         if ent is None:
             sx = torch.empty_like(xi)
             sd = torch.empty_like(dst)
             sx.copy_(xi)
             sm = None if maps is None else maps.clone()
+            ss = None if style is None else style.clone()
             for _ in range(2):                    # warm-up outside capture: weight packs, function attributes, allocator
-                self._forward_chunk(sx, weights, w_x, gain, clip, sd, sm, normalize)
+                self._forward_chunk(sx, weights, w_x, gain, clip, sd, sm, normalize, ss)
             torch.cuda.current_stream(self.device).synchronize()
             gr = torch.cuda.CUDAGraph()
             l0 = _lib.launches
             try:
                 with torch.cuda.graph(gr):
-                    self._forward_chunk(sx, weights, w_x, gain, clip, sd, sm, normalize)
+                    self._forward_chunk(sx, weights, w_x, gain, clip, sd, sm, normalize, ss)
             except Exception as e:                # capture refused (e.g. a user-supplied transformer block that syncs):
                 import warnings                   # same kernels, launched one by one
                 warnings.warn(f"MultiStyleStylizer: CUDA-graph capture failed ({e!r}); continuing without graphs")
                 self.use_graph = False
                 torch.cuda.synchronize(self.device)
-                self._forward_chunk(xi, weights, w_x, gain, clip, dst, maps, normalize)
+                self._forward_chunk(xi, weights, w_x, gain, clip, dst, maps, normalize, style)
                 return
             while len(self._graphs) >= 8:         # stale keys (old parameter versions, other shapes): drop the oldest
                 self._graphs.pop(next(iter(self._graphs)))
             # the captured launches address the packed weights of each generator's cache (allocated during the warm-up, outside
             # the graph's pool): the entry keeps them alive, so invalidate_packed_weights() cannot free memory a graph reads
             keep = [list(g._engine._cache.values()) for g in self.generators]
-            ent = self._graphs[key] = (gr, sx, sd, _lib.launches - l0, keep, sm)
-        gr, sx, sd, n_launches, _, sm = ent
+            ent = self._graphs[key] = (gr, sx, sd, _lib.launches - l0, keep, sm, ss)
+        gr, sx, sd, n_launches, _, sm, ss = ent
         sx.copy_(xi)
         if sm is not None:
             sm.copy_(maps)
+        if ss is not None:
+            ss.copy_(style)
         gr.replay()
         _lib.launches += n_launches               # kernels inside the replayed graph (the launch counter is per C-ABI call)
         dst.copy_(sd)
@@ -158,7 +166,7 @@ class MultiStyleStylizer:
 
     @torch.no_grad()
     def __call__(self, x, weights=None, w_x=0.0, gain=1.0, clip=None, out_uint8=False, out=None, *, weight_maps=None,
-                 feather_sigma=0.0, normalize_maps=False):
+                 feather_sigma=0.0, normalize_maps=False, style=None):
         """x: float32 [B,3,H,W] in [-1,1], or uint8 [B,H,W,3] (PIL layout: ToTensor + Normalize(0.5, 0.5) then run on the
         device, batch_process_images.py:287-291 -- a quarter of the host-to-device bytes), on the device or on the host
         (pinned for overlap).
@@ -169,19 +177,28 @@ class MultiStyleStylizer:
         with map S weighting the input image, h <= H, w <= W), sampled bilinearly at every pixel (ops.blend_maps;
         enhanced_local_style.py:126-176, 232-236).  A [B, S, 1, 1] tensor gives each image its own global mix.
         feather_sigma > 0 blurs each map plane with a Gaussian first (ops.gaussian_blur); normalize_maps divides the
-        sampled weights of each pixel by their sum."""
+        sampled weights of each pixel by their sum.
+        style (style-conditional generators, EnhancedGenerator.enable_style_affine, all with the same number of styles K):
+        the mix fp32 [K] or [B, K] every generator runs with (sliced per micro-batch like the weight maps)."""
         S = len(self.generators)
         hw = (tuple(x.shape[1:3]) if x.dtype == torch.uint8 else tuple(x.shape[2:4])) if x.dim() == 4 else (0, 0)
         check_blend_args(S, x.shape[0], *hw, weights, w_x, weight_maps, float(feather_sigma))
+        num_styles = {getattr(g, "num_styles", None) for g in self.generators}
+        if len(num_styles) != 1:
+            raise ValueError("the generators must all be plain, or all style-conditional with the same number of styles")
+        if style is not None or num_styles != {None}:
+            style = self.generators[0]._style_mix(style, x)
         with torch.cuda.device(self.device):
+            if style is not None:
+                style = style.to(self.device).contiguous()
             maps = None
             if weight_maps is not None:            # moved and feathered once per call, sliced per micro-batch
                 maps = weight_maps.to(self.device, torch.float32).contiguous()
                 if feather_sigma > 0:
                     maps = ops.gaussian_blur(maps, feather_sigma)
-            return self._run(x, weights, w_x, gain, clip, out_uint8, out, maps, bool(normalize_maps))
+            return self._run(x, weights, w_x, gain, clip, out_uint8, out, maps, bool(normalize_maps), style)
 
-    def _run(self, x, weights, w_x, gain, clip, out_uint8, out, maps=None, normalize=False):
+    def _run(self, x, weights, w_x, gain, clip, out_uint8, out, maps=None, normalize=False, style=None):
         B = x.shape[0]
         mb = self.micro_batch
         host_in = not x.is_cuda
@@ -225,10 +242,11 @@ class MultiStyleStylizer:
             if dst is None:
                 dst = torch.empty((hi - lo,) + tuple(out.shape[1:]), device=self.device, dtype=out.dtype)
             mi = None if maps is None else (maps if maps.shape[0] == 1 else maps[lo:hi])
+            si = None if style is None else (style if style.dim() == 1 else style[lo:hi])
             if self.use_graph:
-                self._replay(xi, weights, w_x, gain, clip, dst, pver, mi, normalize)
+                self._replay(xi, weights, w_x, gain, clip, dst, pver, mi, normalize, si)
             else:
-                self._forward_chunk(xi, weights, w_x, gain, clip, dst, mi, normalize)
+                self._forward_chunk(xi, weights, w_x, gain, clip, dst, mi, normalize, si)
             if host_out:
                 out[lo:hi].copy_(dst, non_blocking=True)
         if host_out:
